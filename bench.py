@@ -2,6 +2,7 @@
 """bench.py -- drone-steps/sec of the batched quadrotor-swarm step on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
+    python bench.py --steps K --dump-outputs DIR                   # + what the last timed step returned, as DIR/*.npy
     python bench.py --impl reference [--gpus N] ...                 # CPU arm: the oracle port on all host cores
     torchrun --nproc-per-node N ... bench.py --gpus N ...           # one rank per GPU, weak scaling
 
@@ -14,10 +15,11 @@ step of every env = one launch of the fused step kernel.
 Every workload is measured IN STEADY STATE: the episode clocks are staggered uniformly over [0, ep_len) and the batch is
 pre-rolled for more than one episode before anything is timed, so every timed step contains ~N/ep_len auto-resets (with
 scenario resampling) and the real mix of floor contact / collisions of a random-action rollout; the number of episodes that
-ended inside the timed window is reported (`resets_in_window`).  The timed region is a sequence of K-step blocks (K =
---steps), each bracketed by its own CUDA-event pair on the launching stream, repeated until >= 0.5 s of device time have
-been measured; the reported time is the MEDIAN block (max over ranks), so the figure does not depend on K.  NCCL is
-initialised and warmed up before the warm-up steps.
+ended inside the timed window is reported (`resets_in_window`).  The timed region is exactly K = --steps steps after W =
+--warmup untimed ones, split into up to 10 blocks of back-to-back steps, each bracketed by its own CUDA-event pair on the
+launching stream; the reported time per step is that of the MEDIAN block (max over ranks).  The number of steps a workload
+runs is fixed by the arguments, not by the clock, so with the same arguments every run computes the same outputs
+(--dump-outputs).  NCCL is initialised and warmed up before the warm-up steps.
 
 Per-step working set at 65536 envs (260 MB) exceeds the 126 MB L2 -> back-to-back steps, no flush.  The small BASELINE
 points (configs[1] 4096x8, configs[2] 4096x8 obstacles, configs[3] 1024x32) are measured with per-step events and an L2
@@ -27,7 +29,6 @@ Prints ONE JSON line (rank 0).
 """
 import argparse
 import json
-import math
 import os
 import subprocess
 import sys
@@ -41,7 +42,8 @@ ENVS_PER_GPU = 65536
 ENVS_CFG2 = 4096
 ENVS_CFG4 = 1024
 AGENTS = 8
-MIN_TIMED_S = 0.5
+TIMED_BLOCKS = 10           # the --steps timed steps are split into this many event-bracketed blocks (median reported)
+DUMP_ROWS = 131072          # --dump-outputs: at most this many drones (seeded sample), 29 MB at obs 54
 # Algorithmic HBM bytes per drone-step (SURVEY.md 8d, restated in DESIGN.md "Roofline"):
 # state 120 B read + 120 B written, goal 12 R, tick/flags 4 R+W, action 16 R, obs 4*D W, reward 4 + done 1 W
 ALGO_BYTES = {"cfg2": 497.0, "cfg3": 453.0, "cfg4": 501.0, "mix": 497.0 + 16.0 + 12.0}
@@ -66,6 +68,19 @@ def committed_traffic_per_launch():
             return float(json.load(f)["dram_bytes_per_launch"])
     except Exception:
         return None
+
+
+def dump_outputs(out_dir, tensors):
+    """(obs, rew, done) of one step -> out_dir/{obs,rew,done}.npy, float32.  With more than DUMP_ROWS drones all three keep the
+    same rows, drawn once from a fixed seed, so two builds run with the same arguments can be compared array for array."""
+    import numpy as np
+    obs, rew, done = (t.float().cpu().numpy() for t in tensors)
+    if obs.shape[0] > DUMP_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(obs.shape[0], DUMP_ROWS, replace=False))
+        obs, rew, done = obs[rows], rew[rows], done[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("obs", obs), ("rew", rew), ("done", done)):
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 class ClockSampler:
@@ -173,8 +188,11 @@ def run_reference(args, rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=2000, help="timed steps of every workload")
     ap.add_argument("--warmup", type=int, default=20)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write obs / rew / done of the last timed step of the headline workload (rank 0) as DIR/<name>.npy, float32; "
+                         f"more than {DUMP_ROWS} drones -> the same seeded sample of rows in all three")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--envs-per-gpu", type=int, default=ENVS_PER_GPU, help="override for size sweeps (not the bench line)")
     ap.add_argument("--skip-cpu", action="store_true")
@@ -184,6 +202,8 @@ def main():
                     help="another workload as the timed one (profiling aid; the bench line is cfg2)")
     ap.add_argument("--no-steady", action="store_true", help="profiling aid: skip the staggering + pre-roll (round-1 behaviour)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -251,20 +271,16 @@ def main():
             sim.episode_stats(reset=True)
         return sim, pool, cfg, pre
 
-    def timed_blocks(sim, pool, K, flush=None, min_s=MIN_TIMED_S, max_blocks=4000):
-        """Blocks of K back-to-back steps, one CUDA-event pair per block on the launching stream, until >= min_s of device time.
-        flush: a buffer larger than L2 rewritten before every step (then K = 1 per event pair).  Returns a dict of timings."""
+    def timed_steps(sim, pool, flush=None):
+        """--warmup untimed steps, then exactly --steps timed ones in up to TIMED_BLOCKS blocks of back-to-back steps, one
+        CUDA-event pair per block on the launching stream (an event between every two steps would cost ~2 us each).
+        flush: a buffer larger than L2 rewritten before every step (then one step per block, the flush outside the events).
+        ms_per_step is the median over blocks of block time / steps.  Returns a dict of timings and the (obs, rew, done)
+        tensors of the last timed step (they alias the simulator's buffers)."""
         for i in range(args.warmup):
             sim.step(pool[i % POOL])
-        # size the run from one untimed probe block
-        p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        p0.record(stream)
-        for i in range(K):
-            sim.step(pool[i % POOL])
-        p1.record(stream)
-        torch.cuda.synchronize(dev)
-        probe_ms = max(p0.elapsed_time(p1), 1e-3)
-        nblk = int(min(max_blocks, max(3, math.ceil(min_s * 1e3 / probe_ms))))
+        nblk = args.steps if flush is not None else min(args.steps, TIMED_BLOCKS)
+        bounds = [args.steps * b // nblk for b in range(nblk + 1)]
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(nblk)]
         ep0 = sim.episode_stats()["episodes"]
         l0 = sim.launch_count
@@ -272,21 +288,20 @@ def main():
         for i in range(3):                        # the barrier idles the GPU: a few untimed steps before the first event
             sim.step(pool[i % POOL])
         t_wall = time.perf_counter()
-        j = 0
         for b in range(nblk):
             if flush is not None:
                 flush.fill_(float(b))
             ev[b][0].record(stream)
-            for i in range(K):
-                sim.step(pool[j % POOL]); j += 1
+            for j in range(bounds[b], bounds[b + 1]):
+                last = sim.step(pool[j % POOL])
             ev[b][1].record(stream)
         barrier()
         wall = time.perf_counter() - t_wall
-        ms = sorted(a.elapsed_time(b) for a, b in ev)
-        med = ms[len(ms) // 2]
-        return {"ms_per_step": med / K, "block_ms_median": med, "block_ms_min": ms[0], "block_ms_max": ms[-1], "blocks": nblk,
-                "steps_per_block": K, "timed_s": sum(ms) * 1e-3, "wall_s": wall,
-                "resets_in_window": int(sim.episode_stats()["episodes"] - ep0), "launches": int(sim.launch_count - l0 - 3)}
+        blk_ms = [a.elapsed_time(e) for a, e in ev]
+        per = sorted(t / (bounds[b + 1] - bounds[b]) for b, t in enumerate(blk_ms))
+        return {"ms_per_step": per[len(per) // 2], "step_ms_min": per[0], "step_ms_max": per[-1], "steps": args.steps,
+                "blocks": nblk, "timed_s": sum(blk_ms) * 1e-3, "wall_s": wall,
+                "resets_in_window": int(sim.episode_stats()["episodes"] - ep0), "launches": int(sim.launch_count - l0 - 3)}, last
 
     def reduce_max(x):
         if world == 1:
@@ -304,16 +319,16 @@ def main():
 
     peak, peak_src = measured_hbm_peak()
 
-    def point(workload, n_envs, K, flush=None, algo=None, label=None):
+    def point(workload, n_envs, flush=None, algo=None, label=None):
         """One secondary workload -> its JSON sub-object (max over ranks)."""
         sim, pool, cfg, pre = make(workload, n_envs)
-        r = timed_blocks(sim, pool, K, flush=flush)
+        r, _ = timed_steps(sim, pool, flush=flush)
         ms = reduce_max(r["ms_per_step"])
         resets = reduce_sum(r["resets_in_window"])
         nd_ = n_envs * cfg.num_agents
         sub = cfg.fork.substeps if cfg.env_mode == "fork" else 1
         out = {"workload": label, "envs_per_gpu": n_envs, "agents": cfg.num_agents, "obs_dim": sim.D, "ms_per_step": ms,
-               "value": world * nd_ * sub / (ms * 1e-3), "unit": "drone-steps/s", "blocks": r["blocks"], "steps_per_block": r["steps_per_block"],
+               "value": world * nd_ * sub / (ms * 1e-3), "unit": "drone-steps/s", "steps": r["steps"], "blocks": r["blocks"],
                "timed_s": r["timed_s"], "pre_roll_steps": pre, "resets_in_window": int(resets),
                "l2": "flushed before every timed step (256 MiB write), per-step CUDA events" if flush is not None else "working set > L2, back-to-back steps"}
         if algo is not None:
@@ -330,7 +345,10 @@ def main():
         sampler.start()            # nvidia-smi takes ~1 s to deliver its first sample: start it before the pre-roll
     sim, act_pool, cfg, pre_roll = make(args.workload, n_envs)
     nd = n_envs * cfg.num_agents
-    head = timed_blocks(sim, act_pool, args.steps)
+    head, last = timed_steps(sim, act_pool)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)     # before anything else steps this simulator
+    del last
     clocks = None
     if rank == 0:
         if head["wall_s"] < 3.0:      # keep the GPU under the same load a little longer so that nvidia-smi samples it
@@ -350,7 +368,7 @@ def main():
     out_t = (torch.empty((nd, sim.D), dtype=torch.float32, pin_memory=True),
              torch.empty((nd,), dtype=torch.float32, pin_memory=True), torch.empty((nd,), dtype=torch.uint8, pin_memory=True))
     out = tuple(t.numpy() for t in out_t)
-    e2e_steps = max(50, min(args.steps, 300))
+    e2e_steps = args.steps
     for i in range(3):
         sim.step_host(host_acts[i % POOL], out)
     barrier()
@@ -373,26 +391,26 @@ def main():
     extra = {}
     if not args.skip_small:
         flush_buf = torch.empty(256 * 1024 * 1024 // 4, dtype=torch.float32, device=dev)
-        extra["cfg2_4096"] = point("cfg2", ENVS_CFG2, 1, flush=flush_buf, algo=ALGO_BYTES["cfg2"],
+        extra["cfg2_4096"] = point("cfg2", ENVS_CFG2, flush=flush_buf, algo=ALGO_BYTES["cfg2"],
                                    label="configs[1]: 4096 envs x 8 quads per GPU, static_same_goal, obs 54")
-        extra["cfg3_4096"] = point("cfg3", ENVS_CFG2, 1, flush=flush_buf, algo=ALGO_BYTES["cfg3"],
+        extra["cfg3_4096"] = point("cfg3", ENVS_CFG2, flush=flush_buf, algo=ALGO_BYTES["cfg3"],
                                    label="configs[2]: 4096 envs x 8 quads per GPU, 12 obstacles, SDF obs, downwash, obs 40")
-        extra["cfg4_k32_1024"] = point("cfg4", ENVS_CFG4, 1, flush=flush_buf, algo=ALGO_BYTES["cfg4"],
+        extra["cfg4_k32_1024"] = point("cfg4", ENVS_CFG4, flush=flush_buf, algo=ALGO_BYTES["cfg4"],
                                        label="configs[3]: 1024 envs x 32 quads per GPU, obs 54")
         del flush_buf
-        extra["cfg3_obstacles"] = point("cfg3", n_envs, args.steps, algo=ALGO_BYTES["cfg3"],
+        extra["cfg3_obstacles"] = point("cfg3", n_envs, algo=ALGO_BYTES["cfg3"],
                                         label="configs[2] at the sweep size: 65536 envs x 8 quads per GPU, 12 obstacles, SDF obs, downwash, obs 40")
-        extra["cfg4_k32_16384"] = point("cfg4", n_envs // 4, args.steps, algo=ALGO_BYTES["cfg4"],
+        extra["cfg4_k32_16384"] = point("cfg4", n_envs // 4, algo=ALGO_BYTES["cfg4"],
                                         label="configs[3] at the sweep size: 16384 envs x 32 quads per GPU (the same 524288 drones), obs 54")
-        extra["mix_scenarios"] = point("mix", n_envs, args.steps, algo=ALGO_BYTES["mix"],
+        extra["mix_scenarios"] = point("mix", n_envs, algo=ALGO_BYTES["mix"],
                                        label="upstream training recipe quads_mode=mix: 65536 envs x 8 quads per GPU, one of 9 formation scenarios per "
                                              "episode (goals moving every step in 3 of them), obs 54; +16 B goal written, +12 B scenario row read per drone-step")
-        extra["fork_k4"] = point("fork", n_envs, min(args.steps, 100),
+        extra["fork_k4"] = point("fork", n_envs,
                                  label="fork env of sb_train.py: 65536 envs x 4 chasers per GPU, dynamic_repulsive, one call = 8 control steps "
                                        "(value counts control steps; ms_per_step is per call)")
         # configs[4] as written: 65536 envs TOTAL, sharded over the ranks (strong scaling)
         if world > 1:
-            s = point("cfg2", ENVS_PER_GPU // world, args.steps, algo=ALGO_BYTES["cfg2"],
+            s = point("cfg2", ENVS_PER_GPU // world, algo=ALGO_BYTES["cfg2"],
                       label=f"configs[4] strong scaling: 65536 envs x 8 quads in total = {ENVS_PER_GPU // world} envs per GPU")
         else:
             s = {"workload": "configs[4] strong scaling: 65536 envs x 8 quads in total (1 GPU: the headline run)", "envs_per_gpu": n_envs,
@@ -489,12 +507,13 @@ def main():
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": WORKLOAD, "envs_per_gpu": n_envs, "agents": cfg.num_agents, "obs_dim": d_head,
                        "act_dim": 4, "l2": "inputs larger than L2 (260 MB touched per step vs 126 MB L2), no flush",
-                       "timing": f"median of {head['blocks']} blocks of {args.steps} back-to-back steps, one CUDA-event pair per block on the "
-                                 f"launching stream ({head['timed_s']:.2f} s of device time), max over ranks; barrier + synchronize on both sides",
+                       "timing": f"{args.steps} back-to-back steps in {head['blocks']} blocks, one CUDA-event pair per block on the "
+                                 f"launching stream ({head['timed_s']:.2f} s of device time), median block, max over ranks; "
+                                 f"barrier + synchronize on both sides",
                        "steady_state": f"episode clocks staggered uniformly, {pre_roll} pre-roll steps (> 1 episode) before the warm-up",
                        "parallelism": f"env-sharded x{world}, no collective in the step"},
-            "timed_window": {"blocks": head["blocks"], "steps_per_block": args.steps, "block_ms_median": head["block_ms_median"],
-                             "block_ms_min": head["block_ms_min"], "block_ms_max": head["block_ms_max"], "timed_s": head["timed_s"],
+            "timed_window": {"steps": head["steps"], "blocks": head["blocks"], "step_ms_median": head["ms_per_step"],
+                             "step_ms_min": head["step_ms_min"], "step_ms_max": head["step_ms_max"], "timed_s": head["timed_s"],
                              "resets_in_window": int(head_resets), "pre_roll_steps": pre_roll},
             "clocks": clocks,
             "e2e": {"value": e2e_value, "unit": "drone-steps/s", "h2d_bytes_per_step": nd * 4 * 4,

@@ -112,37 +112,6 @@ def test_mix_vec_env_infos_name_the_scenario_of_the_episode():
                                          "dynamic_diff_goal", "dynamic_formations", "swap_goals", "swarm_vs_swarm"}
 
 
-def test_from_reference_cfg_with_the_real_dataclass():
-    """`QuadSimConfig.from_reference_cfg` fed with the reference's own `QuadrotorEnvConfig` (swarm_rl/global_cfg.py), incl.
-    the overrides `sb_train.py:110-138` applies.  Skipped where the reference checkout is absent (the GPU box)."""
-    import os
-    import sys
-    ref = os.environ.get("QS_REFERENCE_ROOT", "/root/reference")
-    if not os.path.isdir(os.path.join(ref, "swarm_rl")):
-        pytest.skip("reference checkout not present")
-    sys.path.insert(0, ref)
-    try:
-        from swarm_rl.global_cfg import QuadrotorEnvConfig
-    finally:
-        sys.path.remove(ref)
-    rcfg = QuadrotorEnvConfig()
-    cfg = QuadSimConfig.from_reference_cfg(rcfg, num_envs=rcfg.num_envs)
-    assert (cfg.env_mode, cfg.num_envs, cfg.num_agents, cfg.quads_mode) == ("fork", 13, 4, "dynamic_repulsive")
-    assert cfg.obs_dim == 6 + 2 * 3 and cfg.act_dim == 2 and cfg.ep_len == 3000
-    assert tuple(cfg.room_dims) == (15.0, 15.0, 3.0) and cfg.fork.capture_radius == 3.0
-    c = cfg.to_c()
-    assert c.fork.cam_num == 3 and abs(c.fork.cam_focal_length - 0.035) < 1e-12 and c.fork.cam_pixel_noise == 3.0
-    # the author's current sweep
-    rcfg.neighbor_obs_type = "ndist_nsangle"
-    rcfg.obs_repr = "cdist_cdistdot_dist_distdot_sangle_angledot"
-    rcfg.pixel_noise_cam = 0
-    rcfg.num_envs = 12
-    cfg = QuadSimConfig.from_reference_cfg(rcfg, num_envs=rcfg.num_envs)
-    assert cfg.obs_dim == 7 + 3 * 3 and cfg.to_c().fork.cam_pixel_noise == 0.0 and cfg.to_c().neighbor_obs_type == 6
-    obs_space, act_space = make_spaces(cfg)
-    assert obs_space.shape == (16,) and act_space.shape == (2,)
-
-
 def test_episode_extra_stats_keys_with_obstacles():
     """The obstacle env adds the obstacle counters and names the scenario the episode actually ran (mix -> o_random | o_static_same_goal)."""
     cfg = QuadSimConfig(num_envs=2, num_agents=4, quads_mode="mix", use_obstacles=True, use_downwash=True, neighbor_visible_num=2,
