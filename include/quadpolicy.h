@@ -16,9 +16,10 @@
  *                            QuadNeighborhoodEncoderDeepsets.forward            quad_multi_model.py:16-41
  *
  * Architecture built: self encoder S -> 256 -> 256, deep-sets neighbour encoder ('mean_embed') W -> 256 -> 256 averaged over V neighbours,
- * feed-forward 512 -> 512, all tanh; heads 512 -> A (actor) and 512 -> 1 (critic).  bf16 operands, fp32 accumulation
- * (tcgen05 tensor cores); biases, heads and outputs fp32.  Sampling and log-probabilities stay with the caller (state-independent
- * log-std diagonal Gaussian, ActorCriticPolicyCustom.py:312).
+ * optional obstacle encoder O -> 256 -> 256, feed-forward [self | neighbour | obstacle] (512 or 768) -> 512, all tanh; heads 512 -> A (actor) and 512 -> 1 (critic).
+ * bf16 operands, fp32 accumulation (tcgen05 tensor cores); biases, heads and outputs fp32.  Sampling and log-probabilities stay with the
+ * caller (state-independent log-std diagonal Gaussian, ActorCriticPolicyCustom.py:312).  Not built: the 'attention' and 'mlp' neighbour
+ * encoders, widths other than 256.
  *
  * All pointers are CUDA device addresses unless stated; `stream` is a cudaStream_t passed as void*.  Calls return 0 or a negative
  * qp_status; qp_last_error() gives a message.  A handle is bound to one device and is not thread-safe.
@@ -33,7 +34,9 @@
 extern "C" {
 #endif
 
-#define QP_API_VERSION 1
+/* Version 2 appended obst_dim to qp_config and the obst_* fields to qp_tower_weights.  qp_create still accepts a version-1 config (the first six
+ * fields): such a handle has no obstacle encoder and never reads the obst_* fields of qp_tower_weights. */
+#define QP_API_VERSION 2
 
 typedef enum { QP_OK = 0, QP_ERR_NULL = -1, QP_ERR_BAD_CONFIG = -2, QP_ERR_CUDA = -3 } qp_status;
 
@@ -44,6 +47,7 @@ typedef struct {
     int32_t num_nbr;     /* V: neighbour rows in the observation, 0 = no neighbour encoder */
     int32_t hidden;      /* rnn_size: 256 (the only width built) */
     int32_t act_dim;     /* A <= 8 */
+    int32_t obst_dim;    /* O: obstacle observation columns (9 = the SDF patch), 0 = no obstacle encoder; O <= 24 (since version 2) */
 } qp_config;
 
 /* one tower's parameters: device pointers to fp32 arrays in nn.Linear layout (weight [out, in] row-major, bias [out]) */
@@ -52,8 +56,11 @@ typedef struct {
     const float *self_w2, *self_b2; /* [256, 256], [256] */
     const float *nbr_w1, *nbr_b1;   /* [256, W], [256]   (ignored when num_nbr == 0) */
     const float *nbr_w2, *nbr_b2;   /* [256, 256], [256] */
-    const float *ff_w, *ff_b;       /* [512, 512], [512]; input = [self encoder | neighbour encoder] */
+    const float *ff_w, *ff_b;       /* [512, 512] ([512, 768] when obst_dim > 0), [512]; input = [self | neighbour | obstacle encoder];
+                                       without neighbours (num_nbr == 0) the neighbour block must be zeros */
     const float *head_w, *head_b;   /* actor: [A, 512], [A]; critic: [1, 512], [1] */
+    const float *obst_w1, *obst_b1; /* [256, O], [256]   (since version 2; read only when obst_dim > 0) */
+    const float *obst_w2, *obst_b2; /* [256, 256], [256] */
 } qp_tower_weights;
 
 typedef struct qp_policy qp_policy;
@@ -68,8 +75,8 @@ int64_t qp_launch_count(const qp_policy *p);
  * stay valid (and unchanged) until the stream has passed this call; a later qp_forward on the same stream sees the new weights. */
 int qp_set_weights(qp_policy *p, int tower, const qp_tower_weights *w, void *stream);
 
-/* obs: [n, obs_stride] fp32 (self block first, then V neighbour rows of W values, as Appendix B of SURVEY.md);
- * mean: [n, A]; value: [n].  One kernel launch, nothing touches the host. */
+/* obs: [n, obs_stride] fp32 (self block first, then V neighbour rows of W values, then the O obstacle columns, as Appendix B of SURVEY.md),
+ * obs_stride >= S + V * W + O; mean: [n, A]; value: [n].  One kernel launch, nothing touches the host. */
 int qp_forward(qp_policy *p, const float *obs, int n, int obs_stride, float *mean, float *value, void *stream);
 
 /* GAE over a rollout held on the device: rewards / values [T, n] fp32, dones [T, n] bytes (dones[t] = the transition produced by step t

@@ -26,13 +26,18 @@
 //   bytes), in the order the kernel consumes them.  The first layers share one 128 x 32 observation tile per stream, K laid out
 //   [self (24) | neighbour (8)]: the self encoder's image has zeros in the neighbour slots and the neighbour encoder's in the self slots,
 //   so the self part is written once per tile and each neighbour pass rewrites one 16-byte chunk per row.
+//   Obstacle encoder (the OB instantiation, qp_config.obst_dim > 0; quad_multi_model.py's obstacle MLP, O -> 256 -> 256): runs after the self
+//   encoder on stream 1's x tile, whose self slots then hold the O obstacle columns; the feed-forward (K = 768) has one accumulator, ACC0.
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <stdint.h>
 
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 #include <string>
+#include <type_traits>
 
 #include "../../include/quadpolicy.h"
 
@@ -52,13 +57,20 @@ constexpr int EPI_WARPS = 8, EPI_THREADS = 32 * EPI_WARPS, THREADS = EPI_THREADS
 constexpr int RES_BYTES = 2 * CHUNK1 + 8 * CHUNK;                    // neighbour-encoder weights: 147456 = 9 chunks
 constexpr int RES_CHUNKS = RES_BYTES / CHUNK;
 constexpr int STREAM_BYTES = 2 * CHUNK1 + 8 * CHUNK + 32 * CHUNK;    // streamed per tile: self L1, self L2, feed-forward
-constexpr int TOWER_IMG_BYTES = RES_BYTES + STREAM_BYTES;            // 819200
+constexpr int STREAM_CHUNKS = STREAM_BYTES / CHUNK;                  // 41
+// obstacle encoder (compile-time variant): its inputs take the self slots of stream 1's x tile, so O <= SELF_PAD; streamed per tile on top:
+// obstacle L1, obstacle L2, the feed-forward's third K block (4 quarters x 4 chunks)
+constexpr int MAX_OBST = SELF_PAD;
+constexpr int OBST_BYTES = 2 * CHUNK1 + 8 * CHUNK + 16 * CHUNK;
+constexpr int OBST_CHUNKS = OBST_BYTES / CHUNK;                      // 25
+constexpr size_t tower_img_bytes(int obst_dim) { return (size_t)(RES_BYTES + STREAM_BYTES + (obst_dim > 0 ? OBST_BYTES : 0)); }   // 819200 / 1228800
 
 // fp32 side parameters of one tower
 struct TowerParams {
     float bias[4 * H + FF];                 // b_self1, b_self2, b_nbr1, b_nbr2, b_ff
     float head_wt[FF * MAX_ACT];            // [512][8]: transposed nn.Linear.weight, zero-padded
     float head_b[MAX_ACT];
+    float obst_bias[2 * H];                 // b_obst1, b_obst2 (read through L1: shared memory has no room left)
 };
 constexpr int B_SELF1 = 0, B_SELF2 = H, B_NBR1 = 2 * H, B_NBR2 = 3 * H, B_FF = 4 * H, N_BIAS = 4 * H + FF;
 
@@ -70,6 +82,11 @@ struct Args {
     int stagger;                            // clocks between the start of neighbouring blocks (0 = off)
     long long *trace;                       // debug (qp_debug_trace): clock64 stamps of block 0's second tile, tower 0; null = off
 };
+// arguments of the obstacle variant: a type of its own, so that the plain kernel's parameter block (copied to its stack) stays as it is
+struct ArgsOb : Args {
+    int O;                                  // obstacle columns, at S + V * W
+};
+template <bool OB> using KernelArgs = typename std::conditional<OB, ArgsOb, Args>::type;
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -277,7 +294,9 @@ static_assert(sizeof(Smem) <= 232448, "shared-memory map exceeds the 227 KB a bl
 // element (row, k) of an x tile: K-chunk (8 elements, 16 B) major, then 8-row groups of 128 B: LBO = 2048, SBO = 128
 __device__ __forceinline__ uint32_t xoff(int row, int kchunk) { return (uint32_t)(kchunk * 2048 + (row >> 3) * 128 + (row & 7) * 16); }
 
-__global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Args a)
+// OB: with the obstacle encoder (a compile-time variant, so that the plain kernel keeps its register allocation and code layout)
+template <bool OB>
+__global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const KernelArgs<OB> a)
 {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     Smem &sm = *reinterpret_cast<Smem *>(smem_raw);
@@ -307,6 +326,9 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Args a
         while (clock64() < until) __nanosleep(256);
     }
     constexpr uint32_t ACC0 = 0, ACC1 = 128, R10 = 256, R11 = 384;      // TMEM columns: stream accumulators, stream activation regions
+    // Feed-forward input [self | neighbour mean | obstacle]: R10 | R11 | -- without obstacles (the quarters ping-pong between ACC0 and ACC1);
+    // R10 | ACC1 | R11 with them: the three 256-wide activations leave one accumulator, ACC0, for all four quarters
+    constexpr uint32_t R_MEAN = OB ? ACC1 : R11;
     const int S = a.S, W = a.W, V = a.V, A = a.A;
     const int n_tiles = (a.n + TILE_M - 1) / TILE_M;
     // phase bookkeeping, advanced identically by every role: items issued per stream, tiles, ring chunks
@@ -323,10 +345,10 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Args a
         if (warp == 9) {
             for (int tower = 0; tower < 2; ++tower) {
                 // the whole tower image, in consumption order, once per tile: [neighbour encoder (9 chunks, skipped without neighbours) |
-                // self L1 | self L2 x 8 | feed-forward x 32]
+                // self L1 | self L2 x 8 | (OB: obstacle L1 | obstacle L2 x 8) | feed-forward x 32 (OB: x 48)]
                 if (lane == 0) {
                     const uint8_t *img = a.wimg[tower] + (V > 0 ? 0 : RES_BYTES);
-                    const int n_loads = (V > 0 ? RES_CHUNKS : 0) + 41;
+                    const int n_loads = (V > 0 ? RES_CHUNKS : 0) + STREAM_CHUNKS + (OB ? OBST_CHUNKS : 0);
                     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
                         for (int i = 0; i < n_loads; ++i) {
                             const uint32_t slot = n_chunk % STAGES;
@@ -432,16 +454,51 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Args a
                             N_ITEM_INC(s);
                             if (tr) { if (lane == 0) a.trace[tm] = clock64(); tm += 1; }
                         }
-                        // ---- feed-forward: four quarters of 128 outputs, K = 512: chunks 0-3 read R10 (self encoder), chunks 4-7 R11 (neighbour
-                        //      mean, written by the epilogue warps while the first half of quarter 0 runs)
+                        if constexpr (OB) {
+                            // ---- obstacle encoder layer 1: halves on the two accumulators, A = x tile of stream 1 (the obstacle inputs sit in its self
+                            //      slots; the neighbour images have zeros there, this image zeros in the neighbour slots)
+                            {
+                                const uint32_t slot = ring_take();
+                                for (int s = 0; s < 2; ++s) {
+                                    wait_prev(s);
+                                    issue_l1_ss(tmem + (s ? ACC1 : ACC0), xb1, ring0 + slot * (uint32_t)CHUNK + (uint32_t)s * CHUNK1);
+                                    commit_one(&sm.acc_full[s]);
+                                    N_ITEM_INC(s);
+                                    if (tr) { if (lane == 0) a.trace[tm] = clock64(); tm += 1; }
+                                }
+                                ring_release(slot);
+                            }
+                            // ---- obstacle encoder layer 2: A = R11 (hidden), output back into R11 -- the epilogue writes it once BOTH halves have
+                            //      completed (in-place: every MMA of this layer reads all of R11)
+                            wait_prev(0);
+                            wait_prev(1);
+                            for (int s = 0; s < 2; ++s) {
+#pragma unroll
+                                for (int c = 0; c < 4; ++c) {
+                                    const uint32_t slot = ring_take();
+                                    if (c == 0) issue_chunk_ts<true>(tmem + (s ? ACC1 : ACC0), tmem + R11, ring0 + slot * (uint32_t)CHUNK);
+                                    else issue_chunk_ts<false>(tmem + (s ? ACC1 : ACC0), tmem + R11 + (uint32_t)c * 32u, ring0 + slot * (uint32_t)CHUNK);
+                                    held[c] = slot;
+                                    n_chunk += 1;
+                                }
+#pragma unroll
+                                for (int c = 0; c < 4; ++c) commit_one(&sm.empty[held[c]]);
+                                commit_one(&sm.acc_full[s]);
+                                N_ITEM_INC(s);
+                                if (tr) { if (lane == 0) a.trace[tm] = clock64(); tm += 1; }
+                            }
+                        }
+                        // ---- feed-forward: four quarters of 128 outputs, K = 512 (OB: 768): chunks 0-3 read R10 (self encoder), chunks 4-7 R_MEAN
+                        //      (neighbour mean, written by the epilogue warps while the first half of quarter 0 runs), OB: chunks 8-11 R11 (obstacle)
+                        constexpr int FF_CHUNKS = OB ? 12 : 8;
                         for (int qtr = 0; qtr < 4; ++qtr) {
-                            const int s = qtr & 1;
+                            const int s = OB ? 0 : (qtr & 1);
                             wait_prev(s);
                             if (qtr == 0) wait_prev(1);
 #pragma unroll
-                            for (int c = 0; c < 8; ++c) {
+                            for (int c = 0; c < FF_CHUNKS; ++c) {
                                 const uint32_t slot = ring_take();
-                                const uint32_t acol = tmem + (c < 4 ? R10 + (uint32_t)c * 32u : R11 + (uint32_t)(c - 4) * 32u);
+                                const uint32_t acol = tmem + (c < 4 ? R10 + (uint32_t)c * 32u : c < 8 ? R_MEAN + (uint32_t)(c - 4) * 32u : R11 + (uint32_t)(c - 8) * 32u);
                                 if (c == 4 && qtr == 0) { mbar_wait(&sm.mean_ready, (n_tile - 1u) & 1u); tc_fence_after(); }
                                 if (c == 0) issue_chunk_ts<true>(tmem + (s ? ACC1 : ACC0), acol, ring0 + slot * (uint32_t)CHUNK);
                                 else issue_chunk_ts<false>(tmem + (s ? ACC1 : ACC0), acol, ring0 + slot * (uint32_t)CHUNK);
@@ -493,13 +550,14 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Args a
                 N_ITEM_INC(s);
                 if (tr) a.trace[te++] = clock64();
             };
-            // accumulator -> + bias -> tanh -> packed bf16 -> activation region `dst` (columns of layer half h, this thread's 64)
-            auto epi_to_tmem = [&](uint32_t acc, int bias0, int h, uint32_t dst) {
+            // accumulator -> + bias -> tanh -> packed bf16 -> activation region `dst` (columns of layer half h, this thread's 64); `bias`: the
+            // layer's 256 biases (shared memory, or global for the obstacle encoder)
+            auto epi_to_tmem = [&](uint32_t acc, const float *bias, int h, uint32_t dst) {
 #pragma unroll
                 for (int b = 0; b < 4; ++b) {                            // 16 columns at a time (register budget: the 128 running sums stay live)
                     uint32_t v[16], u[8];
                     tmem_ld16(lane_addr + acc + (uint32_t)(q * 64 + b * 16), v);
-                    const float4 *bp = reinterpret_cast<const float4 *>(sm.bias + bias0 + h * 128 + q * 64 + b * 16);
+                    const float4 *bp = reinterpret_cast<const float4 *>(bias + h * 128 + q * 64 + b * 16);
 #pragma unroll
                     for (int i = 0; i < 4; ++i) {
                         const float4 bb = bp[i];
@@ -532,11 +590,22 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Args a
                         for (int i = 0; i < 8; ++i) f[i] = (live && kc * 8 + i < S) ? __ldg(orow + kc * 8 + i) : 0.f;
                         const uint4 u = make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
                         *reinterpret_cast<uint4 *>(sm.xbuf[0] + xoff(row_l, kc)) = u;
-                        *reinterpret_cast<uint4 *>(sm.xbuf[1] + xoff(row_l, kc)) = u;
+                        if constexpr (!OB) *reinterpret_cast<uint4 *>(sm.xbuf[1] + xoff(row_l, kc)) = u;
                     }
                 } else {
                     if (V > 0) *reinterpret_cast<uint4 *>(sm.xbuf[0] + xoff(row_l, 3)) = nbr_chunk(0);
                     if (V > 1) *reinterpret_cast<uint4 *>(sm.xbuf[1] + xoff(row_l, 3)) = nbr_chunk(1);
+                    if constexpr (OB) {                                  // the obstacle inputs (columns S + V W ..) in the self slots of stream 1's tile
+                        const float *orow_o = orow + S + V * W;
+#pragma unroll 1
+                        for (int kc = 0; kc < 3; ++kc) {                 // one chunk at a time: 24 loads in flight beside the 128 running sums spill
+                            float f[8];
+#pragma unroll
+                            for (int i = 0; i < 8; ++i) f[i] = (live && kc * 8 + i < a.O) ? __ldg(orow_o + kc * 8 + i) : 0.f;
+                            *reinterpret_cast<uint4 *>(sm.xbuf[1] + xoff(row_l, kc)) =
+                                make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
+                        }
+                    }
                 }
                 fence_proxy_async();
                 __syncwarp();
@@ -546,14 +615,14 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Args a
                 for (int j0 = 0; j0 < V; j0 += 2) {
                     const int nact = (V - j0) < 2 ? (V - j0) : 2;
                     const float keep = j0 == 0 ? 0.f : 1.f;              // the first pair of passes starts the running sum
-                    for (int s = 0; s < nact; ++s) { wait_acc(s); epi_to_tmem(s ? ACC1 : ACC0, B_NBR1, 0, s ? R11 : R10); item_done(s); }
+                    for (int s = 0; s < nact; ++s) { wait_acc(s); epi_to_tmem(s ? ACC1 : ACC0, sm.bias + B_NBR1, 0, s ? R11 : R10); item_done(s); }
                     for (int s = 0; s < nact; ++s) {
                         wait_acc(s);                                     // both layer-1 MMAs of this pass have read the x tile
                         if (q == s && j0 + s + 2 < V) {
                             *reinterpret_cast<uint4 *>(sm.xbuf[s] + xoff(row_l, 3)) = nbr_chunk(j0 + s + 2);
                             fence_proxy_async();
                         }
-                        epi_to_tmem(s ? ACC1 : ACC0, B_NBR1, 1, s ? R11 : R10);
+                        epi_to_tmem(s ? ACC1 : ACC0, sm.bias + B_NBR1, 1, s ? R11 : R10);
                         item_done(s);
                     }
 #pragma unroll
@@ -580,11 +649,23 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Args a
                         }
                 }
                 // ---- self encoder layer 1 (halves on the two accumulators) -> hidden in R11 (stream 1's last MMAs have completed)
-                for (int s = 0; s < 2; ++s) { wait_acc(s); epi_to_tmem(s ? ACC1 : ACC0, B_SELF1, s, R11); item_done(s); }
+                for (int s = 0; s < 2; ++s) { wait_acc(s); epi_to_tmem(s ? ACC1 : ACC0, sm.bias + B_SELF1, s, R11); item_done(s); }
                 // ---- self encoder layer 2 -> R10
-                for (int s = 0; s < 2; ++s) { wait_acc(s); epi_to_tmem(s ? ACC1 : ACC0, B_SELF2, s, R10); item_done(s); }
-                // ---- neighbour mean -> R11 (no neighbours: zeros, like an absent encoder half).  Both layer-2 MMAs, R11's last readers,
-                //      have completed (their accumulators were waited for above); the feed-forward reads R11 from its 5th K chunk on
+                for (int s = 0; s < 2; ++s) { wait_acc(s); epi_to_tmem(s ? ACC1 : ACC0, sm.bias + B_SELF2, s, R10); item_done(s); }
+                if constexpr (OB) {
+                    // ---- obstacle encoder layer 1 -> hidden in R11 (the self encoder's layer-2 MMAs, R11's last readers, have completed)
+                    for (int s = 0; s < 2; ++s) { wait_acc(s); epi_to_tmem(s ? ACC1 : ACC0, P->obst_bias, s, R11); item_done(s); }
+                    // ---- obstacle encoder layer 2 -> R11 in place: both halves' MMAs must have completed before either half is written
+                    wait_acc(0);
+                    wait_acc(1);
+                    for (int s = 0; s < 2; ++s) { epi_to_tmem(s ? ACC1 : ACC0, P->obst_bias + H, s, R11); item_done(s); }
+                    // the neighbour mean goes to ACC1: every epilogue warp has finished reading it (a row's two column halves are in two warps)
+                    tc_fence_before();
+                    asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS) : "memory");
+                    tc_fence_after();
+                }
+                // ---- neighbour mean -> R_MEAN (no neighbours: zeros, like an absent encoder half).  Its last readers (R11: the self encoder's
+                //      layer-2 MMAs; OB, ACC1: the epilogue above) are done; the feed-forward reads it from its 5th K chunk on
                 {
                     const float inv = V > 0 ? 1.0f / (float)V : 0.f;
 #pragma unroll
@@ -594,7 +675,7 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Args a
                             uint32_t u[16];
 #pragma unroll
                             for (int i = 0; i < 16; ++i) u[i] = pack_bf16(nsum[h * 64 + b * 32 + 2 * i] * inv, nsum[h * 64 + b * 32 + 2 * i + 1] * inv);
-                            tmem_st16(lane_addr + R11 + (uint32_t)(h * 64 + q * 32 + b * 16), u);
+                            tmem_st16(lane_addr + R_MEAN + (uint32_t)(h * 64 + q * 32 + b * 16), u);
                         }
                     tmem_st_wait();
                     tc_fence_before();
@@ -606,7 +687,7 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Args a
 #pragma unroll
                 for (int o = 0; o < MAX_ACT; ++o) head[o] = 0.f;
                 for (int qtr = 0; qtr < 4; ++qtr) {
-                    const int s = qtr & 1;
+                    const int s = OB ? 0 : (qtr & 1);
                     wait_acc(s);
 #pragma unroll
                     for (int b = 0; b < 2; ++b) {
@@ -1019,31 +1100,38 @@ int qp_create(const qp_config *cfg, int device, qp_policy **out)
 {
     if (!cfg || !out) return qp_fail(nullptr, QP_ERR_NULL, "qp_create: null argument");
     *out = nullptr;
-    if (cfg->api_version != QP_API_VERSION) return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create: api_version mismatch");
-    if (cfg->hidden != H) return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create: only hidden = 256 is built");
-    if (cfg->self_dim < 1 || cfg->self_dim > SELF_PAD || cfg->nbr_dim < 0 || cfg->nbr_dim > NBR_PAD || cfg->num_nbr < 0)
+    if (cfg->api_version != 1 && cfg->api_version != QP_API_VERSION) return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create: api_version mismatch");
+    qp_config c;                                                         // a version-1 struct ends before obst_dim
+    memset(&c, 0, sizeof(c));
+    memcpy(&c, cfg, cfg->api_version == 1 ? offsetof(qp_config, obst_dim) : sizeof(qp_config));
+    if (c.hidden != H) return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create: only hidden = 256 is built");
+    if (c.self_dim < 1 || c.self_dim > SELF_PAD || c.nbr_dim < 0 || c.nbr_dim > NBR_PAD || c.num_nbr < 0)
         return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create: self_dim must be in [1, 24], nbr_dim in [0, 8]");
-    if (cfg->act_dim < 1 || cfg->act_dim > MAX_ACT) return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create: act_dim out of [1, 8]");
+    if (c.act_dim < 1 || c.act_dim > MAX_ACT) return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create: act_dim out of [1, 8]");
+    if (c.obst_dim < 0 || c.obst_dim > MAX_OBST) return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create: obst_dim out of [0, 24]");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || device < 0 || device >= ndev) return qp_fail(nullptr, QP_ERR_CUDA, "qp_create: no such CUDA device");
     int prev = 0;
     cudaGetDevice(&prev);
     cudaSetDevice(device);
     qp_policy *p = new qp_policy();
-    p->cfg = *cfg; p->device = device; p->launches = 0; p->trace = nullptr; p->max_grid = 0;
+    p->cfg = c; p->device = device; p->launches = 0; p->trace = nullptr; p->max_grid = 0;
     if (const char *g = getenv("QP_MAX_GRID")) p->max_grid = atoi(g);
     p->stagger = STAGGER_CLK;
     if (const char *g = getenv("QP_STAGGER")) p->stagger = atoi(g);
     p->wimg[0] = p->wimg[1] = nullptr; p->params[0] = p->params[1] = nullptr;
     cudaDeviceGetAttribute(&p->sms, cudaDevAttrMultiProcessorCount, device);
     cudaError_t r = cudaSuccess;
+    const size_t img_bytes = tower_img_bytes(c.obst_dim);
     for (int t = 0; t < 2 && r == cudaSuccess; ++t) {
-        r = cudaMalloc(&p->wimg[t], (size_t)TOWER_IMG_BYTES);
-        if (r == cudaSuccess) r = cudaMemset(p->wimg[t], 0, (size_t)TOWER_IMG_BYTES);
+        r = cudaMalloc(&p->wimg[t], img_bytes);
+        if (r == cudaSuccess) r = cudaMemset(p->wimg[t], 0, img_bytes);
         if (r == cudaSuccess) r = cudaMalloc(&p->params[t], sizeof(TowerParams));
         if (r == cudaSuccess) r = cudaMemset(p->params[t], 0, sizeof(TowerParams));
     }
-    if (r == cudaSuccess) r = cudaFuncSetAttribute(policy_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
+    if (r == cudaSuccess)
+        r = c.obst_dim > 0 ? cudaFuncSetAttribute(policy_forward_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem))
+                           : cudaFuncSetAttribute(policy_forward_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
     cudaSetDevice(prev);
     if (r != cudaSuccess) {
         for (int t = 0; t < 2; ++t) { cudaFree(p->wimg[t]); cudaFree(p->params[t]); }
@@ -1072,8 +1160,10 @@ int qp_set_weights(qp_policy *p, int tower, const qp_tower_weights *w, void *str
 {
     if (!p || !w) return qp_fail(p, QP_ERR_NULL, "qp_set_weights: null argument");
     if (tower < 0 || tower > 1) return qp_fail(p, QP_ERR_BAD_CONFIG, "qp_set_weights: tower must be 0 (actor) or 1 (critic)");
+    const int S = p->cfg.self_dim, O = p->cfg.obst_dim;
+    if (O > 0 && (!w->obst_w1 || !w->obst_b1 || !w->obst_w2 || !w->obst_b2))       // a handle without obstacles never reads these fields
+        return qp_fail(p, QP_ERR_NULL, "qp_set_weights: null obstacle-encoder pointer (obst_dim > 0)");
     cudaStream_t s = (cudaStream_t)stream;
-    const int S = p->cfg.self_dim;
     const int n_out = tower == 0 ? p->cfg.act_dim : 1;
     uint8_t *img = p->wimg[tower];
     // one (N = 128) x kc image
@@ -1087,15 +1177,22 @@ int qp_set_weights(qp_policy *p, int tower, const qp_tower_weights *w, void *str
         for (int h = 0; h < 2; ++h)
             for (int c = 0; c < 4; ++c) pack(w->nbr_w2, H, H, NH * h, 64 * c, 64, 0, 0, img + 2 * CHUNK1 + (size_t)(h * 4 + c) * CHUNK);
     }
-    // streamed block, in consumption order: self L1 halves, self L2 (half, chunk), feed-forward (quarter, chunk)
+    // streamed block, in consumption order: self L1 halves, self L2 (half, chunk), [obstacle L1 halves, obstacle L2 (half, chunk),]
+    // feed-forward (quarter, chunk)
     uint8_t *st = img + RES_BYTES;
-    for (int h = 0; h < 2; ++h) pack(w->self_w1, H, S, NH * h, 0, 32, SELF_PAD, S, st + (size_t)h * CHUNK1);
-    st += 2 * CHUNK1;
-    for (int h = 0; h < 2; ++h)
-        for (int c = 0; c < 4; ++c) pack(w->self_w2, H, H, NH * h, 64 * c, 64, 0, 0, st + (size_t)(h * 4 + c) * CHUNK);
-    st += 8 * CHUNK;
+    auto pack_encoder = [&](const float *w1, int in_dim, const float *w2) {
+        // layer 1 reads K slots 0 .. in_dim - 1 of its x tile; the neighbour slots (24..31) meet zeros
+        for (int h = 0; h < 2; ++h) pack(w1, H, in_dim, NH * h, 0, 32, SELF_PAD, in_dim, st + (size_t)h * CHUNK1);
+        st += 2 * CHUNK1;
+        for (int h = 0; h < 2; ++h)
+            for (int c = 0; c < 4; ++c) pack(w2, H, H, NH * h, 64 * c, 64, 0, 0, st + (size_t)(h * 4 + c) * CHUNK);
+        st += 8 * CHUNK;
+    };
+    pack_encoder(w->self_w1, S, w->self_w2);
+    if (O > 0) pack_encoder(w->obst_w1, O, w->obst_w2);
+    const int ff_chunks = O > 0 ? 12 : 8, ff_in = 64 * ff_chunks;         // K = [self | neighbour (| obstacle)]
     for (int qtr = 0; qtr < 4; ++qtr)
-        for (int c = 0; c < 8; ++c) pack(w->ff_w, FF, FF, NH * qtr, 64 * c, 64, 0, 0, st + (size_t)(qtr * 8 + c) * CHUNK);
+        for (int c = 0; c < ff_chunks; ++c) pack(w->ff_w, FF, ff_in, NH * qtr, 64 * c, 64, 0, 0, st + (size_t)(qtr * ff_chunks + c) * CHUNK);
     TowerParams *P = p->params[tower];
     const cudaMemcpyKind dd = cudaMemcpyDeviceToDevice;
     QP_CUDA(p, cudaMemcpyAsync(P->bias + B_SELF1, w->self_b1, H * sizeof(float), dd, s));
@@ -1105,6 +1202,10 @@ int qp_set_weights(qp_policy *p, int tower, const qp_tower_weights *w, void *str
         QP_CUDA(p, cudaMemcpyAsync(P->bias + B_NBR2, w->nbr_b2, H * sizeof(float), dd, s));
     }
     QP_CUDA(p, cudaMemcpyAsync(P->bias + B_FF, w->ff_b, FF * sizeof(float), dd, s));
+    if (O > 0) {
+        QP_CUDA(p, cudaMemcpyAsync(P->obst_bias, w->obst_b1, H * sizeof(float), dd, s));
+        QP_CUDA(p, cudaMemcpyAsync(P->obst_bias + H, w->obst_b2, H * sizeof(float), dd, s));
+    }
     pack_head_kernel<<<(FF * MAX_ACT + 255) / 256, 256, 0, s>>>(w->head_w, n_out, P->head_wt);
     QP_CUDA(p, cudaMemsetAsync(P->head_b, 0, sizeof(P->head_b), s));
     QP_CUDA(p, cudaMemcpyAsync(P->head_b, w->head_b, (size_t)n_out * sizeof(float), dd, s));
@@ -1227,16 +1328,18 @@ int qp_bias_tanh_mean_backward(const void *grad_mean, const void *y, int n, int 
 int qp_forward(qp_policy *p, const float *obs, int n, int obs_stride, float *mean, float *value, void *stream)
 {
     if (!p || !obs || !mean || !value) return qp_fail(p, QP_ERR_NULL, "qp_forward: null argument");
-    if (n < 1 || obs_stride < p->cfg.self_dim + p->cfg.nbr_dim * p->cfg.num_nbr) return qp_fail(p, QP_ERR_BAD_CONFIG, "qp_forward: bad n / obs_stride");
-    Args a;
+    if (n < 1 || obs_stride < p->cfg.self_dim + p->cfg.nbr_dim * p->cfg.num_nbr + p->cfg.obst_dim)
+        return qp_fail(p, QP_ERR_BAD_CONFIG, "qp_forward: bad n / obs_stride (obs_stride must be >= S + V * W + O)");
+    ArgsOb a;
     a.obs = obs; a.n = n; a.stride = obs_stride; a.S = p->cfg.self_dim; a.W = p->cfg.nbr_dim; a.V = p->cfg.num_nbr; a.A = p->cfg.act_dim;
     for (int t = 0; t < 2; ++t) { a.wimg[t] = p->wimg[t]; a.params[t] = p->params[t]; }
-    a.mean = mean; a.value = value; a.trace = p->trace;
+    a.mean = mean; a.value = value; a.trace = p->trace; a.O = p->cfg.obst_dim;
     a.stagger = (n >= 8 * p->sms * TILE_M) ? p->stagger : 0;            // only worth it when every block has several tiles
     const int tiles = (n + TILE_M - 1) / TILE_M;
     int grid = tiles < p->sms ? tiles : p->sms;
     if (p->max_grid > 0 && grid > p->max_grid) grid = p->max_grid;
-    policy_forward_kernel<<<grid, THREADS, sizeof(Smem), (cudaStream_t)stream>>>(a);
+    if (a.O > 0) policy_forward_kernel<true><<<grid, THREADS, sizeof(Smem), (cudaStream_t)stream>>>(a);
+    else policy_forward_kernel<false><<<grid, THREADS, sizeof(Smem), (cudaStream_t)stream>>>(static_cast<const Args &>(a));
     p->launches += 1;
     QP_CUDA(p, cudaGetLastError());
     return QP_OK;

@@ -14,20 +14,26 @@ import torch
 from . import _capi
 
 
+QP_API_VERSION = 2
+
+
 class QpConfigC(C.Structure):
-    _fields_ = [(n, C.c_int32) for n in ("api_version", "self_dim", "nbr_dim", "num_nbr", "hidden", "act_dim")]
+    _fields_ = [(n, C.c_int32) for n in ("api_version", "self_dim", "nbr_dim", "num_nbr", "hidden", "act_dim", "obst_dim")]
 
 
 class QpTowerWeightsC(C.Structure):
-    FIELDS = ("self_w1", "self_b1", "self_w2", "self_b2", "nbr_w1", "nbr_b1", "nbr_w2", "nbr_b2", "ff_w", "ff_b", "head_w", "head_b")
+    FIELDS = ("self_w1", "self_b1", "self_w2", "self_b2", "nbr_w1", "nbr_b1", "nbr_w2", "nbr_b2", "ff_w", "ff_b", "head_w", "head_b",
+              "obst_w1", "obst_b1", "obst_w2", "obst_b2")
     _fields_ = [(n, C.c_void_p) for n in FIELDS]
 
 
 def supported(policy) -> bool:
-    """The architecture the kernel is built for: deep-sets ('mean_embed') or no neighbour encoder, no obstacle encoder, hidden 256."""
+    """The architecture the kernel is built for: deep-sets ('mean_embed') or no neighbour encoder, optionally the obstacle encoder
+    (9 SDF inputs), hidden 256."""
     enc = policy.actor
-    return (enc.kind in ("mean_embed", "none") and enc.O == 0 and enc.self_encoder[0].out_features == 256
-            and enc.S <= 24 and enc.W <= 8 and policy.action_net.out_features <= 8 and (enc.kind == "none" or enc.neighbor[0].out_features == 256))
+    return (enc.kind in ("mean_embed", "none") and enc.O in (0, 9) and enc.self_encoder[0].out_features == 256
+            and enc.S <= 24 and enc.W <= 8 and policy.action_net.out_features <= 8 and (enc.kind == "none" or enc.neighbor[0].out_features == 256)
+            and (enc.O == 0 or enc.obstacle[0].out_features == 256))
     # 'attention' (the fork's default, quad_multi_model.py:42-102) and 'mlp' stay on the torch path
 
 
@@ -140,16 +146,16 @@ def bias_tanh_mean_backward(grad_mean: torch.Tensor, y: torch.Tensor, V: int):
 class FusedPolicy:
     def __init__(self, policy, device):
         if not supported(policy):
-            raise ValueError("the fused policy kernel is built for hidden 256, deep-sets / no neighbour encoder, no obstacle encoder, S <= 24, W <= 8")
+            raise ValueError("the fused policy kernel is built for hidden 256, deep-sets / no neighbour encoder, optional obstacle encoder, S <= 24, W <= 8")
         self.policy = policy
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise RuntimeError("FusedPolicy runs on CUDA devices only (no CPU path)")
         enc = policy.actor
-        self.S, self.W, self.V = enc.S, enc.W, (enc.V if enc.kind == "mean_embed" else 0)
+        self.S, self.W, self.V, self.O = enc.S, enc.W, (enc.V if enc.kind == "mean_embed" else 0), enc.O
         self.A = policy.action_net.out_features
         self._lib = _capi.lib()
-        cfg = QpConfigC(1, self.S, self.W, self.V, 256, self.A)
+        cfg = QpConfigC(QP_API_VERSION, self.S, self.W, self.V, 256, self.A, self.O)
         if self._lib.qp_config_size() != C.sizeof(QpConfigC):
             raise RuntimeError("qp_config layout mismatch")
         h = C.c_void_p()
@@ -191,7 +197,9 @@ class FusedPolicy:
             if self.V > 0:
                 t.update({"nbr_w1": enc.neighbor[0].weight, "nbr_b1": enc.neighbor[0].bias,
                           "nbr_w2": enc.neighbor[2].weight, "nbr_b2": enc.neighbor[2].bias})
-            ff_in = enc.feed_forward[0].in_features
+            if self.O > 0:
+                t.update({"obst_w1": enc.obstacle[0].weight, "obst_b1": enc.obstacle[0].bias,
+                          "obst_w2": enc.obstacle[2].weight, "obst_b2": enc.obstacle[2].bias})
             w = QpTowerWeightsC()
             for name in QpTowerWeightsC.FIELDS:
                 v = t.get(name)
@@ -199,8 +207,8 @@ class FusedPolicy:
                     setattr(w, name, None)
                     continue
                 v = v.detach().to(device=self.device, dtype=torch.float32).contiguous()
-                if name == "ff_w" and ff_in == 256:      # no neighbour encoder: the neighbour half of the feed-forward input is absent
-                    v = torch.cat([v, torch.zeros_like(v)], dim=1).contiguous()
+                if name == "ff_w" and self.V == 0:       # no neighbour encoder: its block of the feed-forward input, [self | neighbour | obstacle], is zeros
+                    v = torch.cat([v[:, :256], torch.zeros_like(v[:, :256]), v[:, 256:]], dim=1).contiguous()
                 self._keep.append(v)
                 setattr(w, name, v.data_ptr())
             with torch.cuda.device(self.device):
