@@ -86,7 +86,9 @@ int qp_gae(const float *rewards, const float *values, const uint8_t *dones, cons
 
 /* The elementwise half of a dense tanh layer in the PPO update (ActorCriticPolicyCustom.evaluate_actions -> QuadMultiEncoder.forward under
  * autograd): y = tanh(z + bias) and, in one pass, its backward grad_z = grad_y * (1 - y^2) with grad_bias = column sums of grad_z.
- * z, y, grad_* are [n, h] row-major, bf16 (is_bf16 != 0, the autocast path) or fp32; bias / grad_bias are fp32 [h]; h even, <= 2048. */
+ * z, y, grad_* are [n, h] row-major, bf16 (is_bf16 != 0, the autocast path) or fp32; bias / grad_bias are fp32 [h]; h even, <= 2048.
+ * The [n, h] pointers must be aligned to one element pair (8 bytes fp32, 4 bytes bf16), else QP_ERR_BAD_CONFIG; with h % 8 == 0 and
+ * 16-byte alignment the calls take the faster 8-column form. */
 int qp_bias_tanh(const void *z, const float *bias, int n, int h, int is_bf16, void *y, void *stream);
 int qp_bias_tanh_backward(const void *grad_y, const void *y, int n, int h, int is_bf16, void *grad_z, float *grad_bias, void *stream);
 

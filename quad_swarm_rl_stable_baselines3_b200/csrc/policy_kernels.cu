@@ -1224,6 +1224,10 @@ int qp_gae(const float *rewards, const float *values, const uint8_t *dones, cons
     return QP_OK;
 }
 
+// the pair kernels (bias_tanh_kernel, bias_tanh_bwd_kernel) load and store float2 / __nv_bfloat162: every [n, h] operand must be aligned
+// to one element pair, which "h even" alone does not give (a contiguous view at an odd element offset)
+static bool pair_aligned(int is_bf16, size_t addr_bits) { return (addr_bits & (is_bf16 ? 3 : 7)) == 0; }
+
 static int bias_tanh_grid(int n)
 {
     int dev = 0, sms = 148;
@@ -1237,6 +1241,8 @@ int qp_bias_tanh(const void *z, const float *bias, int n, int h, int is_bf16, vo
 {
     if (!z || !bias || !y) return qp_fail(nullptr, QP_ERR_NULL, "qp_bias_tanh: null argument");
     if (n < 1 || h < 2 || (h & 1) || h > 2048) return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_bias_tanh: h must be even and <= 2048, n >= 1");
+    if (!pair_aligned(is_bf16, (size_t)z | (size_t)y))
+        return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_bias_tanh: pointers must be aligned to one element pair (8 bytes fp32, 4 bytes bf16)");
     cudaStream_t s = (cudaStream_t)stream;
     if ((h & 7) == 0 && (((size_t)z | (size_t)y | (size_t)bias) & 15) == 0) {
         const int G = h / 8, RL = G >= 256 ? 1 : 256 / G, rows = (n + RL - 1) / RL, grid = bias_tanh_grid(rows);
@@ -1253,6 +1259,8 @@ int qp_bias_tanh_backward(const void *grad_y, const void *y, int n, int h, int i
 {
     if (!grad_y || !y || !grad_z || !grad_bias) return qp_fail(nullptr, QP_ERR_NULL, "qp_bias_tanh_backward: null argument");
     if (n < 1 || h < 2 || (h & 1) || h > 2048) return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_bias_tanh_backward: h must be even and <= 2048, n >= 1");
+    if (!pair_aligned(is_bf16, (size_t)grad_y | (size_t)y | (size_t)grad_z))
+        return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_bias_tanh_backward: pointers must be aligned to one element pair (8 bytes fp32, 4 bytes bf16)");
     cudaStream_t s = (cudaStream_t)stream;
     cudaError_t r = cudaMemsetAsync(grad_bias, 0, (size_t)h * sizeof(float), s);
     if (r == cudaSuccess) {
@@ -1296,7 +1304,7 @@ int qp_bias_tanh_mean(const void *z, const float *bias, int n, int V, int h, int
 {
     if (!z || !bias || !y || !mean) return qp_fail(nullptr, QP_ERR_NULL, "qp_bias_tanh_mean: null argument");
     if (n < 1 || V < 1 || h < 8 || (h & 7) || h > 2048 || ((((size_t)z | (size_t)y | (size_t)mean | (size_t)bias) & 15) != 0))
-        return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_bias_tanh_mean: h must be a multiple of 8 (<= 2048), pointers 16-byte aligned");
+        return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_bias_tanh_mean: n >= 1, V >= 1, h a multiple of 8 (<= 2048), pointers 16-byte aligned");
     const int G = h / 8, RL = G >= 256 ? 1 : 256 / G, grid = bias_tanh_grid((n + RL - 1) / RL);
     cudaStream_t s = (cudaStream_t)stream;
     if (is_bf16) bias_tanh_mean_kernel<<<grid, G * RL, 0, s>>>((const __nv_bfloat16 *)z, bias, n, V, h, RL, (__nv_bfloat16 *)y, (__nv_bfloat16 *)mean);
@@ -1310,7 +1318,7 @@ int qp_bias_tanh_mean_backward(const void *grad_mean, const void *y, int n, int 
 {
     if (!grad_mean || !y || !grad_z || !grad_bias) return qp_fail(nullptr, QP_ERR_NULL, "qp_bias_tanh_mean_backward: null argument");
     if (n < 1 || V < 1 || h < 8 || (h & 7) || h > 2048 || ((((size_t)grad_mean | (size_t)y | (size_t)grad_z) & 15) != 0))
-        return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_bias_tanh_mean_backward: h must be a multiple of 8 (<= 2048), pointers 16-byte aligned");
+        return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_bias_tanh_mean_backward: n >= 1, V >= 1, h a multiple of 8 (<= 2048), pointers 16-byte aligned");
     const int G = h / 8, RL = G >= 256 ? 1 : 256 / G;
     int grid = bias_tanh_grid((n + RL - 1) / RL);
     if (grid > 592) grid = 592;

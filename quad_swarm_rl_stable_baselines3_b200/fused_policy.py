@@ -38,10 +38,20 @@ def supported(policy) -> bool:
 
 
 def gae(rewards: torch.Tensor, values: torch.Tensor, dones: torch.Tensor, last_values: torch.Tensor, gamma: float, lam: float):
-    """`ppo.compute_gae` in one CUDA launch (`qp_gae`): rewards / values [T, n] float32, dones [T, n] bool, last_values [n]."""
+    """`ppo.compute_gae` in one CUDA launch (`qp_gae`): rewards / values [T, n] float32, dones [T, n] bool or uint8, last_values [n];
+    ValueError on any other dtype or shape."""
     if rewards.device.type != "cuda":
         raise RuntimeError("fused_policy.gae runs on CUDA tensors only (no CPU path)")
+    if rewards.dim() != 2:
+        raise ValueError("gae: rewards must be [T, n]")
     T, n = rewards.shape
+    # the kernel reads the [T, n] arrays as float32 and one byte per done flag: another dtype would be reinterpreted, not converted
+    for name, t, dtypes in (("rewards", rewards, (torch.float32,)), ("values", values, (torch.float32,)), ("dones", dones, (torch.bool, torch.uint8))):
+        if t.dtype not in dtypes or tuple(t.shape) != (T, n) or t.device != rewards.device:
+            raise ValueError(f"gae: {name} must be {' / '.join(str(d) for d in dtypes)} [{T}, {n}] on {rewards.device}, "
+                             f"got {t.dtype} {list(t.shape)} on {t.device}")
+    if tuple(last_values.shape) != (n,) or last_values.device != rewards.device:
+        raise ValueError(f"gae: last_values must be [{n}] on {rewards.device}, got {list(last_values.shape)} on {last_values.device}")
     rewards, values, last_values = rewards.contiguous(), values.contiguous(), last_values.contiguous().float()
     d8 = dones.contiguous().view(torch.uint8)
     adv, ret = torch.empty_like(rewards), torch.empty_like(rewards)
@@ -113,10 +123,17 @@ def bias_tanh_backward_first(grad_y: torch.Tensor, y: torch.Tensor, x: torch.Ten
     return gw, gb
 
 
+def _groups(rows: int, V: int) -> int:
+    """Groups of V consecutive rows; a remainder would be left unwritten in the outputs."""
+    if V < 1 or rows % V != 0:
+        raise ValueError(f"bias_tanh_mean: {rows} rows are not whole groups of V = {V}")
+    return rows // V
+
+
 def bias_tanh_mean(z: torch.Tensor, bias: torch.Tensor, V: int):
     """(y, mean): y = tanh(z + bias) on [n * V, h], mean [n, h] over each group of V rows (`qp_bias_tanh_mean`)."""
     _bt_check(z)
-    n = z.shape[0] // V
+    n = _groups(z.shape[0], V)
     b = bias.detach().to(device=z.device, dtype=torch.float32).contiguous()
     y, m = torch.empty_like(z), torch.empty((n, z.shape[1]), dtype=z.dtype, device=z.device)
     lib = _capi.lib()
@@ -130,13 +147,16 @@ def bias_tanh_mean(z: torch.Tensor, bias: torch.Tensor, V: int):
 
 def bias_tanh_mean_backward(grad_mean: torch.Tensor, y: torch.Tensor, V: int):
     _bt_check(y)
+    n = _groups(y.shape[0], V)
+    if tuple(grad_mean.shape) != (n, y.shape[1]):
+        raise ValueError(f"bias_tanh_mean_backward: grad_mean must be [{n}, {y.shape[1]}], got {list(grad_mean.shape)}")
     if grad_mean.dtype != y.dtype or not grad_mean.is_contiguous():
         grad_mean = grad_mean.to(y.dtype).contiguous()
     gz = torch.empty_like(y)
     gb = torch.empty(y.shape[1], dtype=torch.float32, device=y.device)
     lib = _capi.lib()
     with torch.cuda.device(y.device):
-        rc = lib.qp_bias_tanh_mean_backward(grad_mean.data_ptr(), y.data_ptr(), y.shape[0] // V, V, y.shape[1], int(y.dtype == torch.bfloat16),
+        rc = lib.qp_bias_tanh_mean_backward(grad_mean.data_ptr(), y.data_ptr(), n, V, y.shape[1], int(y.dtype == torch.bfloat16),
                                             gz.data_ptr(), gb.data_ptr(), C.c_void_p(torch.cuda.current_stream(y.device).cuda_stream))
     if rc != 0:
         raise RuntimeError(f"qp_bias_tanh_mean_backward failed ({rc}): {lib.qp_last_error(None).decode()}")
