@@ -156,8 +156,10 @@ def test_reset_parity(name):
     assert (st["tick"] == 0).all() and (st["step_ctr"] == 1).all()
 
 
-def run_parity(name, cfg, sim, oracles, kind, steps, hook=None, check_records=True):
-    """Every step: copy the GPU state into the oracle, step both with the same actions, compare everything."""
+def run_parity(name, cfg, sim, oracles, kind, steps, hook=None, check_records=True, record_envs=None):
+    """Every step: copy the GPU state into the oracle, step both with the same actions, compare everything.
+    `record_envs`, if given, is called after each step and returns a bool mask [N]: the envs whose just-finished episode record
+    is compared (default: every env that finished)."""
     K, N = cfg.num_agents, cfg.num_envs
     rs = np.random.RandomState(11)
     worst = dict(pos=0.0, vel=0.0, rot=0.0, omega=0.0, obs=0.0, rew=0.0)
@@ -250,7 +252,10 @@ def run_parity(name, cfg, sim, oracles, kind, steps, hook=None, check_records=Tr
         if done.any() and check_records:
             # per-episode records (infos[i]['episode_extra_stats']) of the envs that just finished
             env_rec, agent_rec = sim.episode_records_host()
-            for e in np.flatnonzero(done.reshape(N, K)[:, 0] & env_ok):
+            sel = done.reshape(N, K)[:, 0] & env_ok
+            if record_envs is not None:
+                sel = sel & record_envs()
+            for e in np.flatnonzero(sel):
                 ref_env, ref_agent = oracles[e].record()
                 same = np.array_equal(env_rec[e, 1:19], ref_env[1:19])
                 cnt["record_mismatch"] = cnt.get("record_mismatch", 0) + int(not same)
