@@ -54,7 +54,7 @@ rounds = int(os.environ.get("AB_ROUNDS", "3"))
 res = {l: [] for l in libs}
 for r in range(rounds):
     for l in libs:
-        path, *extra = l.split(":")            # "lib.so:QS_PERSIST=1:QS_BLOCK=64" sets environment knobs for that variant
+        path, *extra = l.split(":")            # "lib.so:QS_HOT=0:QS_BLOCK=64" sets environment knobs for that variant
         env = dict(os.environ, QS_LIB_PATH=os.path.abspath(path), **dict(kv.split("=", 1) for kv in extra))
         p = subprocess.run([sys.executable, "-c", CHILD, case], env=env, capture_output=True, text=True)
         line = [x for x in p.stdout.splitlines() if x.startswith("RESULT")]

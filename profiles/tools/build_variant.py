@@ -18,8 +18,8 @@ flags = [f for f in _capi.NVCC_FLAGS if f != "-shared"] + [f"-D{d}" for d in def
 r = subprocess.run(["nvcc"] + flags + [f"-DQS_KG={KG}", "-c", os.path.join(_capi.CSRC, "kernels_kg.cu"), "-o", obj], capture_output=True, text=True)
 lines = r.stderr.split("\n")
 for i, l in enumerate(lines):
-    if "Function properties" in l and f"step_kernelILi{KG}ELb0E" in l:
-        print(l.split(f"step_kernelILi{KG}ELb0E")[1][:6], lines[i + 1].strip(), "|", lines[i + 2].strip().replace("ptxas info    : ", ""))
+    if "Function properties" in l and f"11step_kernelILi{KG}E" in l:
+        print(l.split(f"11step_kernelILi{KG}E")[1][:6], lines[i + 1].strip(), "|", lines[i + 2].strip().replace("ptxas info    : ", ""))
 if r.returncode:
     sys.stderr.write(r.stderr)
     sys.exit(1)

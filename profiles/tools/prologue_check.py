@@ -12,10 +12,10 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 # (object, substring of the mangled name): the hot variants that ship
-KERNELS = [("kernels_kg8.o", "step_kernelILi8ELb0ELi0E"), ("kernels_kg8.o", "step_kernelILi8ELb0ELi1E"),
-           ("kernels_kg8.o", "step_kernelILi8ELb0ELi2E"), ("kernels_kg8.o", "step_kernelILi8ELb0ELi3E"),
-           ("kernels_kg8.o", "step_kernelILi8ELb0ELi4E"), ("kernels_kg8.o", "step_kernelILi8ELb0ELi6E"),
-           ("kernels_kg32.o", "step_kernelILi32ELb0ELi0E"), ("kernels_kg4.o", "fork_step_kernelILi4E")]
+KERNELS = [("kernels_kg8.o", "step_kernelILi8ELi0E"), ("kernels_kg8.o", "step_kernelILi8ELi1E"),
+           ("kernels_kg8.o", "step_kernelILi8ELi2E"), ("kernels_kg8.o", "step_kernelILi8ELi3E"),
+           ("kernels_kg8.o", "step_kernelILi8ELi4E"), ("kernels_kg8.o", "step_kernelILi8ELi6E"),
+           ("kernels_kg32.o", "step_kernelILi32ELi0E"), ("kernels_kg4.o", "fork_step_kernelILi4E")]
 WINDOW = 200          # instructions from the first state load that count as prologue
 
 

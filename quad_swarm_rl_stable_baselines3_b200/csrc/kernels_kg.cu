@@ -19,7 +19,7 @@ constexpr int KG = QS_KG;
 // (+1 KB per block of driver reservation) and leave the rest of the unified array to L1.  The step kernels stream their state
 // (no L1 reuse) but spill a few registers at the 128-register cap; with the maximum carve-out L1 shrinks to ~28 KB, the 16
 // resident warps' stack frames do not fit and every spill reload becomes an L2 round trip (profiles/README.md, v5: 89.3 ->
-// 86.3 us).  `block` == 0 (persistent form, whose prefetch buffers need all of it): maximum carve-out.
+// 86.3 us).  `block` == 0 (the reset kernels): maximum carve-out.
 // The attributes belong to the kernel instantiation on a device, not to a handle: several handles (train env + eval env, as
 // sb_train.py runs them) share them, so both the dynamic shared-memory limit and the carve-out are only ever RAISED -- a later,
 // smaller handle must not pull the limit below what an earlier one launches with (cudaErrorInvalidValue on its next step).
@@ -71,41 +71,23 @@ void set_attr(size_t bytes, void (*kernel)(Args...), int block = 0)
         case 4: { constexpr int FEAT = 4; CALL; } break;  \
         default: { constexpr int FEAT = 6; CALL; } break; \
     }
-// the persistent form exists for the feature sets without formation scenarios
-#define QS_FEAT_SWITCH_PERSIST(FEATv, CALL)               \
-    switch (FEATv) {                                      \
-        case 0: { constexpr int FEAT = 0; CALL; } break;  \
-        case 1: { constexpr int FEAT = 1; CALL; } break;  \
-        case 2: { constexpr int FEAT = 2; CALL; } break;  \
-        default: { constexpr int FEAT = 3; CALL; } break; \
-    }
-
-void prepare(int feat, size_t smem_plain, size_t smem_persist, int block, int *persist_blocks_per_sm, bool fork)
+void prepare(int feat, size_t smem, int block, bool fork)
 {
-    *persist_blocks_per_sm = 0;
     if (fork) {
-        set_attr(smem_plain, fork_step_kernel<KG>, block);
-        set_attr(smem_plain, fork_reset_kernel<KG>);
+        set_attr(smem, fork_step_kernel<KG>, block);
+        set_attr(smem, fork_reset_kernel<KG>);
         return;
     }
-    QS_FEAT_SWITCH(feat, set_attr(smem_plain, step_kernel<KG, false, FEAT>, block));
-    set_attr(smem_plain, reset_kernel<KG, false, false>);
-    set_attr(smem_plain, reset_kernel<KG, true, false>);
-    set_attr(smem_plain, reset_kernel<KG, false, true>);
-    if (feat < 4 && smem_persist > 0 && smem_persist <= 227 * 1024) {
-        QS_FEAT_SWITCH_PERSIST(feat, set_attr(smem_persist, step_kernel<KG, true, FEAT>);
-                       cudaOccupancyMaxActiveBlocksPerMultiprocessor(persist_blocks_per_sm, step_kernel<KG, true, FEAT>, block, smem_persist));
-    }
+    QS_FEAT_SWITCH(feat, set_attr(smem, step_kernel<KG, FEAT>, block));
+    set_attr(smem, reset_kernel<KG, false, false>);
+    set_attr(smem, reset_kernel<KG, true, false>);
+    set_attr(smem, reset_kernel<KG, false, true>);
 }
 
-void step(bool persist, int feat, LaunchShape s, cudaStream_t st, const DevConst &c, const DevPtrs &P, const float4 *actions, float *obs,
+void step(int feat, LaunchShape s, cudaStream_t st, const DevConst &c, const DevPtrs &P, const float4 *actions, float *obs,
           float *rew, uint8_t *done, float *term_obs, uint8_t *reset_success)
 {
-    if (persist && feat < 4) {
-        QS_FEAT_SWITCH_PERSIST(feat, (step_kernel<KG, true, FEAT><<<s.grid, s.block, s.smem, st>>>(c, P, actions, obs, rew, done, term_obs, reset_success)));
-    } else {
-        QS_FEAT_SWITCH(feat, (step_kernel<KG, false, FEAT><<<s.grid, s.block, s.smem, st>>>(c, P, actions, obs, rew, done, term_obs, reset_success)));
-    }
+    QS_FEAT_SWITCH(feat, (step_kernel<KG, FEAT><<<s.grid, s.block, s.smem, st>>>(c, P, actions, obs, rew, done, term_obs, reset_success)));
 }
 
 void reset(int feat, LaunchShape s, cudaStream_t st, const DevConst &c, const DevPtrs &P, const uint8_t *mask, float *obs)

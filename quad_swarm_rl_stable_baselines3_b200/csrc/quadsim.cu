@@ -129,9 +129,6 @@ struct qs_env {
     int block;              // threads per block
     int grid;
     size_t smem_bytes;
-    bool persist;           // upstream step kernel as a persistent, TMA-prefetched warp-tile loop (large batches)
-    int grid_persist;
-    size_t smem_persist;
     void *slab;             // one allocation for all device state
     size_t slab_bytes;
     // pinned host staging + device io buffers for the *_host entry points
@@ -141,7 +138,7 @@ struct qs_env {
     // the kernel of the next
     cudaStream_t cs[2]; cudaEvent_t ev_in, ev_out[2]; bool pipe_ready;
     long long launches;
-    // reset-first scheduling of the plain upstream step kernel (DevPtrs::hot_*): three rotating buffers in the slab
+    // reset-first scheduling of the upstream step kernel (DevPtrs::hot_*): three rotating buffers in the slab
     int *hot_list[3], *hot_cnt[3], *hot_flag[3];
     int hot_cap, hot_blocks; unsigned hot_phase; bool hot;
     uint32_t rng_step;      // Philox counter word 1: +1 per step / reset call (+ fork.substeps per fork step); the same for every env of the handle
@@ -403,9 +400,8 @@ int qs_create(const qs_config *cfg, int device, qs_env **out)
     // staged per warp-tile behind the tiles: the obstacle centres, or (formation scenarios, never with obstacles) the scenario rows
     const size_t obst_floats = cfg->use_obstacles ? (size_t)warps * (32 / e->KG) * cfg->num_obstacles * 2
                                                   : (scen_feat ? (size_t)warps * (32 / e->KG) * QS_SC_COUNT : 0);
-    // QS_PARK: 3 float4 per thread (goal, distance ring, window sums) parked in shared memory while the dynamics run
-    // (QS_EARLY_RNG: 4 float4 per thread -- the step's 16 pre-generated normals -- in the same per-thread scratch slots)
-    const size_t park_floats = e->fork ? 0 : (QS_EARLY_RNG ? (size_t)19 * e->block : (QS_PARK ? (size_t)12 * e->block : 0));
+    // per-thread scratch slots of the step kernel: 4 float4 (the step's 16 pre-generated normals) + 3 ints (per-env scalars)
+    const size_t park_floats = e->fork ? 0 : (size_t)19 * e->block;
     e->smem_bytes = (((tiles_floats + obst_floats + 3) & ~(size_t)3) + park_floats) * sizeof(float);
     if (e->smem_bytes > 200 * 1024) { delete e; return fail(nullptr, QS_ERR_BAD_CONFIG, "qs_create: observation tile does not fit in shared memory"); }
 
@@ -461,21 +457,7 @@ int qs_create(const qs_config *cfg, int device, qs_env **out)
     init_identity_kernel<<<(int)((nd + 127) / 128), 128>>>(e->dp, (int)nd);
     r = cudaDeviceSynchronize();
     if (r != cudaSuccess) { cudaFree(e->slab); delete e; return fail(nullptr, QS_ERR_CUDA, std::string("qs_create: state init: ") + cudaGetErrorString(r)); }
-    e->persist = false; e->grid_persist = 0; e->smem_persist = 0;
-    {
-        const size_t pf_floats = (tiles_floats + obst_floats + 3) & ~(size_t)3;
-        if (!e->fork) e->smem_persist = pf_floats * sizeof(float) + (size_t)warps * PF_SLOTS * 32 * sizeof(float4) + (size_t)warps * sizeof(uint64_t) +
-                                       (size_t)warps * 3 * (32 / e->KG) * sizeof(int);     // prefetch buffers, mbarriers, per-env scalars
-        int per_sm = 0;
-        launchers(e->KG).prepare(e->feat, e->smem_bytes, e->smem_persist, e->block, &per_sm, e->fork);
-        // Measured (profiles/README.md): the persistent form does not pay on this kernel (79.0 us plain vs 86.9 us persistent at
-        // 65536 envs): its prefetch buffers need the maximum carve-out, which leaves L1 too small for the spilled registers.  It is
-        // opt-in (QS_PERSIST=1) and kept bitwise-tested against the plain form.
-        const char *pe = getenv("QS_PERSIST");
-        const bool want = pe ? atoi(pe) != 0 : false;
-        if (!e->fork && per_sm > 0 && want) { e->persist = true; e->grid_persist = (e->grid < per_sm * sms) ? e->grid : per_sm * sms; }
-        if (const char *pb = getenv("QS_PERSIST_BLOCKS")) { int v = atoi(pb); if (v >= 1 && v < e->grid_persist) e->grid_persist = v; }   // tests: force looping
-    }
+    launchers(e->KG).prepare(e->feat, e->smem_bytes, e->block, e->fork);
     r = cudaGetLastError();
     if (r != cudaSuccess) { cudaFree(e->slab); delete e; return fail(nullptr, QS_ERR_CUDA, std::string("qs_create: ") + cudaGetErrorString(r)); }
     *out = e;
@@ -547,9 +529,6 @@ static void launch_step_range(qs_env *e, int e0, int n, cudaStream_t s, const fl
         F.evader += e0; F.flags += e0;
         launchers(e->KG).fork_step({ grid, e->block, e->smem_bytes }, s, c, e->fc, P, F, (const float2 *)actions, obs, rew, done, terminal_obs,
                                    reset_success);
-    } else if (e->persist) {
-        launchers(e->KG).step(true, e->feat, { grid < e->grid_persist ? grid : e->grid_persist, e->block, e->smem_persist }, s, c, P,
-                              (const float4 *)actions, obs, rew, done, terminal_obs, reset_success);
     } else {
         int g2 = grid;
         if (e->hot && e0 == 0 && n == e->cfg.num_envs) {                // full-range launches only: tile ids are relative to the launch
@@ -561,7 +540,7 @@ static void launch_step_range(qs_env *e, int e0, int n, cudaStream_t s, const fl
             P.hot_cap = e->hot_cap; P.hot_blocks = e->hot_blocks;
             g2 += e->hot_blocks;
         }
-        launchers(e->KG).step(false, e->feat, { g2, e->block, e->smem_bytes }, s, c, P, (const float4 *)actions, obs, rew, done, terminal_obs,
+        launchers(e->KG).step(e->feat, { g2, e->block, e->smem_bytes }, s, c, P, (const float4 *)actions, obs, rew, done, terminal_obs,
                               reset_success);
     }
     e->launches += 1;

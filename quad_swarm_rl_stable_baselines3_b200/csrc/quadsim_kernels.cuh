@@ -35,24 +35,6 @@
 #ifndef QS_STEP_MAXTHREADS
 #define QS_STEP_MAXTHREADS 128
 #endif
-#ifndef QS_PARK
-#define QS_PARK 0               // 1: goal / distance ring / window sums travel global -> shared by LDGSTS (no registers while the dynamics run).
-#endif                          //    Measured slower (cfg2 79.3 -> 85.1 us, profiles/README.md round 2): off.
-#ifndef QS_EARLY_RNG
-#define QS_EARLY_RNG 1          // the step's regular draws (OU + sensor noise) are generated in the shadow of the prologue loads
-#endif
-#ifndef QS_PREFETCH
-#define QS_PREFETCH -1          // with QS_EARLY_RNG: 1 = prefetch the warp's state rows into L2, draw, then load (L2 hits); 2 = prefetch into
-#endif                          // L1; 0 = load first, then draw; -1 = per variant as measured (profiles/README.md round 2: formation scenarios 1, others 0)
-#ifndef QS_EARLY_STORE
-#define QS_EARLY_STORE 1        // motor-lag and OU planes are written back right after the dynamics (12 registers dead for the rest of the step)
-#endif
-#ifndef QS_QUAT_ROUNDTRIP
-#define QS_QUAT_ROUNDTRIP 0     // 1: evaluate the zero-noise R -> quaternion -> R round trip of the sensor model literally
-#endif
-#ifndef QS_BODY_RODRIGUES
-#define QS_BODY_RODRIGUES 1     // rotate by exp([w_body]x) on the right instead of exp([R w_body]x) on the left (same matrix)
-#endif
 #define QS_PI_F 3.14159265358979323846f
 
 namespace qs {
@@ -95,7 +77,7 @@ struct DevPtrs {
     float4 *scen;              // [N, QS_SC_COUNT / 4] formation-scenario rows (formation scenarios only, else null)
     int *ep_rec;               // [N, QS_ER_COUNT] record of the last finished episode per env (QS_ER_*)
     float4 *ep_agent;          // [N*K] per-drone part of that record
-    // reset-first scheduling (step kernel, plain form): warp-tiles whose envs finish their episode in THIS step were listed by the
+    // reset-first scheduling (step kernel): warp-tiles whose envs finish their episode in THIS step were listed by the
     // previous step and are processed by the first `hot_blocks` blocks of the grid, so that the long auto-reset path overlaps the
     // rest of the grid instead of extending its tail.  Three buffers rotate: consumed now / produced now / count cleared now.
     int *hot_list_cur, *hot_cnt_cur, *hot_flag_cur;   // flags: one int per warp-tile (set = a hot block owns this tile in this step)
@@ -203,29 +185,12 @@ struct Drone {
     uint32_t colmask;
 };
 
-template <bool WITH_GOAL = true>
 __device__ __forceinline__ void load_drone(const DevPtrs &P, int gi, Drone &q)
 {
     // streamed once per step: keep them out of L1, which then holds the few spilled registers of the kernel
     float4 a = __ldcs(P.plane[PL_POS_VX] + gi), b = __ldcs(P.plane[PL_V_W] + gi), c = __ldcs(P.plane[PL_W_R0] + gi), d = __ldcs(P.plane[PL_R1] + gi),
            e = __ldcs(P.plane[PL_R2_FLAGS] + gi), f = __ldcs(P.plane[PL_ROT_DAMP] + gi), g = __ldcs(P.plane[PL_CMDS_DAMP] + gi),
-           h = __ldcs(P.plane[PL_OU] + gi), k = WITH_GOAL ? __ldcs(P.plane[PL_GOAL] + gi) : make_float4(0.f, 0.f, 0.f, 0.f);
-    q.p[0] = a.x; q.p[1] = a.y; q.p[2] = a.z; q.v[0] = a.w; q.v[1] = b.x; q.v[2] = b.y;
-    q.w[0] = b.z; q.w[1] = b.w; q.w[2] = c.x;
-    q.R[0] = c.y; q.R[1] = c.z; q.R[2] = c.w; q.R[3] = d.x; q.R[4] = d.y; q.R[5] = d.z; q.R[6] = d.w; q.R[7] = e.x; q.R[8] = e.y;
-    q.flags = __float_as_int(e.z); q.colmask = __float_as_uint(e.w);
-    q.rd[0] = f.x; q.rd[1] = f.y; q.rd[2] = f.z; q.rd[3] = f.w;
-    q.cd[0] = g.x; q.cd[1] = g.y; q.cd[2] = g.z; q.cd[3] = g.w;
-    q.ou[0] = h.x; q.ou[1] = h.y; q.ou[2] = h.z; q.ou[3] = h.w;
-    q.goal[0] = k.x; q.goal[1] = k.y; q.goal[2] = k.z;
-}
-
-// same unpacking out of a warp's prefetch buffer (slot s holds rows of plane s)
-__device__ __forceinline__ void load_drone_smem(const float4 *pf, int row, Drone &q)
-{
-    float4 a = pf[PL_POS_VX * 32 + row], b = pf[PL_V_W * 32 + row], c = pf[PL_W_R0 * 32 + row], d = pf[PL_R1 * 32 + row],
-           e = pf[PL_R2_FLAGS * 32 + row], f = pf[PL_ROT_DAMP * 32 + row], g = pf[PL_CMDS_DAMP * 32 + row],
-           h = pf[PL_OU * 32 + row], k = pf[PL_GOAL * 32 + row];
+           h = __ldcs(P.plane[PL_OU] + gi), k = __ldcs(P.plane[PL_GOAL] + gi);
     q.p[0] = a.x; q.p[1] = a.y; q.p[2] = a.z; q.v[0] = a.w; q.v[1] = b.x; q.v[2] = b.y;
     q.w[0] = b.z; q.w[1] = b.w; q.w[2] = c.x;
     q.R[0] = c.y; q.R[1] = c.z; q.R[2] = c.w; q.R[3] = d.x; q.R[4] = d.y; q.R[5] = d.z; q.R[6] = d.w; q.R[7] = e.x; q.R[8] = e.y;
@@ -310,13 +275,7 @@ __device__ __forceinline__ void dynamics_substep(const DevConst &c, const Rng &g
     }
     // Rodrigues rotation about the world-frame angular velocity (:544-551): R <- exp([R w]x dt) R.  Since exp([R w]x) = R exp([w]x) R^T
     // this is R exp([w]x dt) -- the same matrix, built from the body-frame rate directly (no R w product, |R w| = |w|)
-#if QS_BODY_RODRIGUES
     float wx = q.w[0], wy = q.w[1], wz = q.w[2];
-#else
-    float wx = q.R[0] * q.w[0] + q.R[1] * q.w[1] + q.R[2] * q.w[2];
-    float wy = q.R[3] * q.w[0] + q.R[4] * q.w[1] + q.R[5] * q.w[2];
-    float wz = q.R[6] * q.w[0] + q.R[7] * q.w[1] + q.R[8] * q.w[2];
-#endif
     float wn = norm3f(wx, wy, wz);
     if (wn != 0.0f) {
         float inv = 1.0f / wn, kx = wx * inv, ky = wy * inv, kz = wz * inv;
@@ -333,21 +292,12 @@ __device__ __forceinline__ void dynamics_substep(const DevConst &c, const Rng &g
         float d10 = sn * kz + oc * kx * ky, d11 = 1.f + oc * (ky * ky - 1.f), d12 = -sn * kx + oc * ky * kz;
         float d20 = -sn * ky + oc * kx * kz, d21 = sn * kx + oc * ky * kz, d22 = 1.f + oc * (kz * kz - 1.f);
         float n[9];
-#if QS_BODY_RODRIGUES
 #pragma unroll
         for (int i = 0; i < 3; ++i) {                                  // R dR
             n[3 * i] = q.R[3 * i] * d00 + q.R[3 * i + 1] * d10 + q.R[3 * i + 2] * d20;
             n[3 * i + 1] = q.R[3 * i] * d01 + q.R[3 * i + 1] * d11 + q.R[3 * i + 2] * d21;
             n[3 * i + 2] = q.R[3 * i] * d02 + q.R[3 * i + 1] * d12 + q.R[3 * i + 2] * d22;
         }
-#else
-#pragma unroll
-        for (int j = 0; j < 3; ++j) {
-            n[j] = d00 * q.R[j] + d01 * q.R[3 + j] + d02 * q.R[6 + j];
-            n[3 + j] = d10 * q.R[j] + d11 * q.R[3 + j] + d12 * q.R[6 + j];
-            n[6 + j] = d20 * q.R[j] + d21 * q.R[3 + j] + d22 * q.R[6 + j];
-        }
-#endif
 #pragma unroll
         for (int j = 0; j < 9; ++j) q.R[j] = n[j];
     }
@@ -443,32 +393,12 @@ __device__ __forceinline__ void self_obs(const DevConst &c, const SensorNoise &s
         p0 += c.s_pos * n.x; p1 += c.s_pos * n.y; p2 += c.s_pos * n.z;
         v0 += c.s_vel * n.w; v1 += c.s_vel * m.x; v2 += c.s_vel * m.y;
         w0 += c.s_gyro * m.z; w1 += c.s_gyro * m.w; w2 += c.s_gyro * l.x;
-#if !QS_QUAT_ROUNDTRIP
         // R -> quaternion -> R round trip with zero rotation noise (sensor_noise.py:34-63, 205-210; quad_utils.py:162-168): the identity
         // on rotation matrices.  In the float64 reference it returns R to 1e-16; evaluated literally in fp32 it only adds round-off
         // (~3e-7) on top of R, so the observation carries R itself (closer to the reference than the literal form, and ~50
         // instructions + 2 SFU operations less per drone-step)
 #pragma unroll
         for (int a = 0; a < 9; ++a) o[6 + a] = q.R[a];
-#else
-        // R -> quaternion -> R round trip (sensor_noise.py:34-63, 205-210; quad_utils.py:162-168), zero rotation noise
-        const float *R = q.R;
-        float tr = R[0] + R[4] + R[8], qw, qx, qy, qz, S;
-        // one sqrt + one reciprocal shared by the four rot2quat branches (sensor_noise.py:34-63)
-        const bool b0 = tr > 0.f, b1 = !b0 && (R[0] > R[4] && R[0] > R[8]), b2 = !b0 && !b1 && (R[4] > R[8]);
-        const float arg = b0 ? tr : (b1 ? R[0] - R[4] - R[8] : (b2 ? R[4] - R[0] - R[8] : R[8] - R[0] - R[4]));
-        S = sqrtf(arg + 1.0f) * 2.f;
-        const float iS = 1.0f / S, big = 0.25f * S;
-        const float a76 = (R[7] - R[5]) * iS, a26 = (R[2] - R[6]) * iS, a31 = (R[3] - R[1]) * iS;
-        const float s13 = (R[1] + R[3]) * iS, s26 = (R[2] + R[6]) * iS, s57 = (R[5] + R[7]) * iS;
-        qw = b0 ? big : (b1 ? a76 : (b2 ? a26 : a31));
-        qx = b0 ? a76 : (b1 ? big : (b2 ? s13 : s26));
-        qy = b0 ? a26 : (b1 ? s13 : (b2 ? big : s57));
-        qz = b0 ? a31 : (b1 ? s26 : (b2 ? s57 : big));
-        o[6] = 1.0f - 2.f * qy * qy - 2.f * qz * qz; o[7] = 2.f * qx * qy - 2.f * qz * qw; o[8] = 2.f * qx * qz + 2.f * qy * qw;
-        o[9] = 2.f * qx * qy + 2.f * qz * qw; o[10] = 1.0f - 2.f * qx * qx - 2.f * qz * qz; o[11] = 2.f * qy * qz - 2.f * qx * qw;
-        o[12] = 2.f * qx * qz - 2.f * qy * qw; o[13] = 2.f * qy * qz + 2.f * qx * qw; o[14] = 1.0f - 2.f * qx * qx - 2.f * qy * qy;
-#endif
     } else {
 #pragma unroll
         for (int a = 0; a < 9; ++a) o[6 + a] = q.R[a];
@@ -831,8 +761,9 @@ __device__ __forceinline__ uint32_t group_mask(int lane) { return (KG == 32) ? Q
 // a14 in one pass over the env's obstacles: the 3x3 SDF patch (get_surround_sdfs, obstacles/utils.py:5-27; the min over
 // obstacles commutes with the sqrt) and the first obstacle the drone touches (collision_detection, obstacles/utils.py:31-43:
 // 2-D distance <= arm + size/2, lowest index wins) -- the centre cell of the patch IS that distance.
-// brute-force form: every obstacle against every patch point
-__device__ __forceinline__ void obstacle_sdf_and_hit_all(const DevConst &c, const float2 *ob, float px, float py, float *r, int &hit)
+// Brute-force form, every obstacle against every patch point: a candidate-list form (patch only for the centres near the drone) ran
+// fewer instructions with less ILP and was slower (cfg3 102.4 -> 110.5 us).
+__device__ __forceinline__ void obstacle_sdf_and_hit(const DevConst &c, const float2 *ob, float px, float py, float *r, int &hit)
 {
     const float gx[3] = { px - c.sdf_res, px, px + c.sdf_res }, gy[3] = { py - c.sdf_res, py, py + c.sdf_res };
     const float obst2 = c.thr_obst * c.thr_obst * 1.0001f;
@@ -852,56 +783,6 @@ __device__ __forceinline__ void obstacle_sdf_and_hit_all(const DevConst &c, cons
             for (int b = 0; b < 3; ++b) md[a * 3 + b] = fminf(md[a * 3 + b], dx2[a] + dy2[b]);
         const float d2 = dx2[1] + dy2[1];
         if (d2 <= obst2 && hit < 0 && __fsqrt_rn(d2) <= c.thr_obst) hit = m;
-    }
-#pragma unroll
-    for (int a = 0; a < 9; ++a) r[a] = sqrtf(md[a]) - c.obst_rad;
-}
-
-// Step-path form.  The nine patch points lie within delta = sqrt(2) * sdf_res of the drone, so an obstacle can be the nearest one of
-// SOME patch point only if its distance from the drone is <= d_min + 2 delta (d_j(s) >= d_j - delta and min_k d_k(s) <= d_min + delta).
-// Pass 1 measures every centre from the drone only (5 instead of ~35 instructions each; it is also the hit test -- the centre point of
-// the patch IS that distance), pass 2 evaluates the 3x3 patch against the few centres inside that bound (typically 1-3 of 12).  The
-// minimum over a subset that contains every possible minimiser is the same number, bit for bit, as the minimum over all centres.
-// More than QS_SDF_LIST candidates, or more than 16 obstacles: the brute-force form.
-#ifndef QS_SDF_LIST
-#define QS_SDF_LIST 0           // measured SLOWER than the brute-force form (cfg3 102.4 -> 110.5 us): fewer instructions but less ILP. Off.
-#endif
-__device__ __forceinline__ void obstacle_sdf_and_hit(const DevConst &c, const float2 *ob, float px, float py, float *r, int &hit)
-{
-    if (QS_SDF_LIST == 0 || c.M > 16) { obstacle_sdf_and_hit_all(c, ob, px, py, r, hit); return; }
-    const float obst2 = c.thr_obst * c.thr_obst * 1.0001f;
-    float d2[16], dmin2 = 10000.0f;
-    hit = -1;
-#pragma unroll
-    for (int m = 0; m < 16; ++m) {
-        if (m < c.M) {                                                  // warp-uniform
-            const float2 xy = ob[m];
-            const float dx = px - xy.x, dy = py - xy.y;
-            d2[m] = dx * dx + dy * dy;
-            dmin2 = fminf(dmin2, d2[m]);
-            if (d2[m] <= obst2 && hit < 0 && __fsqrt_rn(d2[m]) <= c.thr_obst) hit = m;
-        } else d2[m] = 3.0e38f;
-    }
-    const float lim = sqrtf(dmin2) + 2.8285f * c.sdf_res, lim2 = lim * lim * 1.0001f;    // 2 sqrt(2) sdf_res, widened against round-off
-    uint32_t list = 0u;
-    int n = 0;
-#pragma unroll
-    for (int m = 0; m < 16; ++m)
-        if (d2[m] <= lim2) { list |= (n < QS_SDF_LIST) ? ((uint32_t)m << (8 * n)) : 0u; ++n; }
-    if (__builtin_expect(n > QS_SDF_LIST, 0)) { int h2; obstacle_sdf_and_hit_all(c, ob, px, py, r, h2); return; }
-    const float gx[3] = { px - c.sdf_res, px, px + c.sdf_res }, gy[3] = { py - c.sdf_res, py, py + c.sdf_res };
-    float md[9];
-#pragma unroll
-    for (int a = 0; a < 9; ++a) md[a] = 10000.0f;                       // (100)^2: the value the patch carries when there is no obstacle at all
-    for (int t = 0; t < n; ++t) {
-        const float2 xy = ob[(list >> (8 * t)) & 255u];
-        float dx2[3], dy2[3];
-#pragma unroll
-        for (int a = 0; a < 3; ++a) { float dx = gx[a] - xy.x, dy = gy[a] - xy.y; dx2[a] = dx * dx; dy2[a] = dy * dy; }
-#pragma unroll
-        for (int a = 0; a < 3; ++a)
-#pragma unroll
-            for (int b = 0; b < 3; ++b) md[a * 3 + b] = fminf(md[a * 3 + b], dx2[a] + dy2[b]);
     }
 #pragma unroll
     for (int a = 0; a < 9; ++a) r[a] = sqrtf(md[a]) - c.obst_rad;
@@ -958,11 +839,7 @@ __device__ __forceinline__ void group_obs_tail(const DevConst &c, const float2 *
                         r[3] = clampf(b.x - vs[0], -6.f, 6.f); r[4] = clampf(b.y - vs[1], -6.f, 6.f); r[5] = clampf(b.z - vs[2], -6.f, 6.f);
                     }
                 }
-#ifndef QS_AB_GENERIC_RANK
             } else if (KG <= 8) {
-#else
-            } else if (KG <= 0) {
-#endif
                 // stable rank count with the ranks packed 4 bits per candidate: one compare + one select + one add per pair.
                 // Lanes that are not candidates (self, j >= K) carry +inf and therefore rank behind every real candidate, so a
                 // rank below V (< K - 1) always belongs to a real one.  The packed form also lets the row writes be a rolled
@@ -1037,7 +914,7 @@ __device__ __forceinline__ void group_obs_tail(const DevConst &c, const float2 *
     }
     if (OBST && SDF && valid) {
         int hit;
-        obstacle_sdf_and_hit_all(c, ob, q.p[0], q.p[1], o + c.S + ((c.nbr_type == QS_NEIGHBOR_POS_VEL) ? 6 * c.V : 0), hit);
+        obstacle_sdf_and_hit(c, ob, q.p[0], q.p[1], o + c.S + ((c.nbr_type == QS_NEIGHBOR_POS_VEL) ? 6 * c.V : 0), hit);
     }
 }
 
@@ -1083,33 +960,6 @@ __device__ __forceinline__ void group_reset(const DevConst &c, const DevPtrs &P,
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
-// TMA bulk store shared -> global of one contiguous run (16-byte aligned, size a multiple of 16), tracked by the issuing
-// thread's bulk async-group
-__device__ __forceinline__ void bulk_store_1d(void *dst_gmem, const void *src_smem, uint32_t bytes)
-{
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst_gmem), "r"(smem_u32(src_smem)), "r"(bytes) : "memory");
-    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-}
-// the issuing thread waits until its bulk stores have finished READING shared memory (the source may then be overwritten)
-__device__ __forceinline__ void bulk_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-// make this thread's shared-memory writes visible to the async proxy (TMA) before a bulk store reads them
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-// The warp's observation tile (rows contiguous in global memory) leaves shared memory as ONE TMA bulk store issued by lane 0
-// when the run is 16-byte aligned (it is for every BASELINE shape: K * D * 4 bytes per env is a multiple of 16); the caller
-// must call bulk_store_wait_read() on lane 0 + __syncwarp() before the tile is written again or the block exits.
-__device__ __forceinline__ bool warp_store_tile_bulk(const float *tile, float *dst, int count, int lane)
-{
-    if (((((size_t)dst) & 15) == 0) && ((count & 3) == 0)) {
-        fence_async_smem();
-        __syncwarp();
-        if (lane == 0) bulk_store_1d(dst, tile, (uint32_t)count * 4u);
-        return true;
-    }
-    for (int i = lane; i < count; i += 32) __stcs(dst + i, tile[i]);
-    return false;
-}
-
 // coalesced copy of the warp's observation tile (rows contiguous in global memory) out of shared memory
 __device__ __forceinline__ void warp_store_tile(const float *tile, float *dst, int count, int lane)
 {
@@ -1125,79 +975,22 @@ __device__ __forceinline__ void warp_store_tile(const float *tile, float *dst, i
 // ----------------------------------------------------------------------------------------------------------------
 // The step kernel: QuadrotorEnvMulti.step (quadrotor_multi.py:521-842) for every env, one launch.
 // ----------------------------------------------------------------------------------------------------------------
-// PERSIST = false: one warp-tile (32 lanes = 32/KG envs) per warp, state read straight from HBM.
-// PERSIST = true : grid = resident blocks only; every warp loops over warp-tiles and the 12 x 512 B of per-drone input of
-//                  its NEXT tile (9 state planes, distance ring + windows, actions) are fetched by TMA bulk copies
-//                  (cp.async.bulk -> shared memory, completion on a per-warp mbarrier) while the current tile is being
-//                  computed, so the one exposed HBM latency at the top of the kernel (12 % of the stall samples of the
-//                  non-persistent form, profiles/README.md) is paid once per warp instead of once per tile.
-enum { PF_SLOTS = 12, PF_RING = 9, PF_SUMS = 10, PF_ACT = 11 };
+// One warp-tile (32 lanes = 32/KG envs) per warp, state read straight from HBM.  A persistent form (resident grid, TMA bulk
+// prefetch of the next warp-tile) was measured slower and removed: profiles/README.md.
 
-__device__ __forceinline__ void mbar_init(uint64_t *bar, int count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t phase)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "QS_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra QS_DONE;\n"
-        "bra QS_WAIT;\n"
-        "QS_DONE:\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(phase) : "memory");
-}
-__device__ __forceinline__ void tma_load_1d(void *dst_smem, const void *src_gmem, uint32_t bytes, uint64_t *bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst_smem)),
-                 "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-
-// 4-byte asynchronous global -> shared copy (LDGSTS): the per-env scalars of the next warp-tile travel without a register
+// 4-byte asynchronous global -> shared copy (LDGSTS): the per-env scalars travel without a register
 __device__ __forceinline__ void cp_async4(void *dst_smem, const void *src_gmem)
 {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(dst_smem)), "l"(src_gmem) : "memory");
 }
-// 16-byte asynchronous global -> shared copy (LDGSTS.128): data that is consumed late in the step travels without holding registers
-__device__ __forceinline__ void cp_async16(void *dst_smem, const void *src_gmem)
-{
-    // no "memory" clobber: the copy must not fence the surrounding prologue loads (the reads of the destination sit behind
-    // cp_async_wait_all(), which does clobber memory)
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(dst_smem)), "l"(src_gmem));
-}
-__device__ __forceinline__ void prefetch_row(const void *p)
-{
-#if QS_PREFETCH == 2
-    asm volatile("prefetch.global.L1 [%0];" ::"l"(p));
-#else
-    asm volatile("prefetch.global.L2 [%0];" ::"l"(p));
-#endif
-}
+__device__ __forceinline__ void prefetch_row(const void *p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
-
-// lane 0 of a warp: fetch the inputs of warp-tile `wt` (rows gi0 .. gi0+cnt-1 of every plane) into the warp's buffer
-__device__ __forceinline__ void prefetch_tile(const DevPtrs &P, const float4 *actions, float4 *pf, uint64_t *bar, int gi0, int cnt)
-{
-    const uint32_t bytes = (uint32_t)cnt * 16u;
-    mbar_expect_tx(bar, bytes * PF_SLOTS);
-#pragma unroll
-    for (int s = 0; s < PL_COUNT; ++s) tma_load_1d(pf + s * 32, P.plane[s] + gi0, bytes, bar);    // PL_* order == slot order
-    tma_load_1d(pf + PF_ACT * 32, actions + gi0, bytes, bar);
-}
 
 // FEAT: compile-time feature set (bit 0 obstacles, bit 1 downwash).  The big optional passes are specialised away instead of
 // being skipped at run time: a cfg2 launch then carries none of their code or registers (an "uber-kernel" with run-time
 // flags cost the plain 8-quad swarm 9 % when the obstacle / downwash code was reshaped).
-template <int KG, bool PERSIST, int FEAT>
+template <int KG, int FEAT>
 __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_kernel(const __grid_constant__ DevConst c, const __grid_constant__ DevPtrs P,
                                                    const float4 *__restrict__ actions, float *__restrict__ obs,
                                                    float *__restrict__ rew, uint8_t *__restrict__ done, float *__restrict__ term_obs,
@@ -1216,7 +1009,6 @@ __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_ke
     const int row = (lane / KG) * c.K + d;
     float *orow = tile + (size_t)row * c.D;
     const int n_wt = (c.N + GPW - 1) / GPW;                             // warp-tiles
-    const int wt_stride = PERSIST ? (int)gridDim.x * warps_per_block : n_wt;
     // obstacle centres of this warp-tile's envs (GPW x M float2), staged once per tile: the hit test and the SDF read each of
     // them K times, and the serial `first hit wins` loop would otherwise chain M dependent global loads
     const size_t ob_off = ((size_t)warps_per_block * 256 + (size_t)warps_per_block * rows_per_warp * c.D + 3) & ~(size_t)3;
@@ -1226,25 +1018,11 @@ __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_ke
     // formation scenarios (never with obstacles): the scenario rows of this warp-tile's envs live where the obstacle centres would
     float4 *sc_sm = reinterpret_cast<float4 *>(smem + ob_off) + (size_t)warp_in_block * (GPW * (QS_SC_COUNT / 4));
     const float4 *sc_env = sc_sm + (lane / KG) * (QS_SC_COUNT / 4);
-    // prefetch buffer + mbarrier of this warp (PERSIST only), 16-byte aligned
-    const size_t pf_off = (ob_off + (size_t)warps_per_block * ob_per_warp * 2 + 3) & ~(size_t)3;
-    // parking area of the plain form (QS_PARK): goal / distance ring / window sums of every thread, 3 x blockDim float4, behind the
-    // staged obstacle centres or scenario rows
-    constexpr bool PARK = QS_PARK && !PERSIST && !QS_EARLY_RNG;        // the two users of the per-thread scratch slots exclude each other
+    // per-thread scratch slots behind the staged obstacle centres or scenario rows: 4 x blockDim float4 (the step's pre-generated
+    // normals), then 3 ints per thread (tick, svd counter, reset-first flag)
     const size_t park_off = (ob_off + (OBST ? (size_t)warps_per_block * ob_per_warp * 2 : (SCEN ? (size_t)warps_per_block * GPW * QS_SC_COUNT : 0)) + 3) & ~(size_t)3;
-    float4 *park = reinterpret_cast<float4 *>(smem + park_off) + threadIdx.x;
-    const int park_stride = blockDim.x;
-    float4 *pf = reinterpret_cast<float4 *>(smem + pf_off) + (size_t)warp_in_block * PF_SLOTS * 32;
-    uint64_t *bar = reinterpret_cast<uint64_t *>(smem + pf_off + (size_t)warps_per_block * PF_SLOTS * 32 * 4) + warp_in_block;
-    // per-env scalars (tick, svd counter, RNG step counter) of the next tile: 3 x GPW ints per warp behind the mbarriers.  Kept in
-    // registers they were spilled right after the load, which stalled the warp for the whole HBM latency (profiles/README.md v5)
-    int *sc = reinterpret_cast<int *>(smem + pf_off + (size_t)warps_per_block * PF_SLOTS * 32 * 4 + (size_t)warps_per_block * 2) + warp_in_block * (3 * GPW);
-    uint32_t phase = 0u;
     int wt = (int)blockIdx.x * warps_per_block + warp_in_block;
-#ifndef QS_HOT_MODE
-#define QS_HOT_MODE 1           // 0: reset-first scheduling compiled out
-#endif
-    constexpr bool HOT_OK = QS_HOT_MODE && !PERSIST && QS_EARLY_RNG && (FEAT & 5) != 0 && KG < 32;     // same rule as qs_create's e->hot
+    constexpr bool HOT_OK = (FEAT & 5) != 0 && KG < 32;                // same rule as qs_create's e->hot
     const bool HOT = HOT_OK && P.hot_flag_cur != nullptr;   // warp-uniform (the flag travels with the early-draw scalars)
     bool hot_role = false;
     if (HOT) {
@@ -1256,17 +1034,8 @@ __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_ke
             hot_role = true;
         } else wt -= P.hot_blocks * warps_per_block;
     }
-    if (PERSIST) {
-        if (lane == 0) mbar_init(bar, 1);
-        __syncwarp();
-        if (wt < n_wt) {
-            if (lane == 0) prefetch_tile(P, actions, pf, bar, wt * GPW * c.K, max(0, min(GPW, c.N - wt * GPW)) * c.K);
-            const int e0 = wt * GPW + lane / KG;
-            if (e0 < c.N && d == 0) { cp_async4(sc + lane / KG, P.tick + e0); cp_async4(sc + GPW + lane / KG, P.svd_ctr + e0); }
-            cp_async_commit();
-        }
-    }
-    for (; wt < n_wt; wt += wt_stride) {
+    // at most one trip: the loop shape is kept because an early `return` for wt >= n_wt compiles to different (longer) code
+    for (; wt < n_wt; wt += n_wt) {
     const int warp_env0 = wt * GPW;                                     // first env of this warp-tile
     const int env = warp_env0 + lane / KG;
     const bool valid = env < c.N && d < c.K;
@@ -1296,10 +1065,11 @@ __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_ke
     // generator is inlined in a rolled 4-trip loop (a call would make the compiler move in-flight load destinations out of the
     // callee's registers first, i.e. wait for the loads) and parks its 16 normals in the thread's shared-memory slots, so they
     // hold no registers while the dynamics run.
-    constexpr bool EARLY = QS_EARLY_RNG && !PERSIST;
-    constexpr int PFM = (QS_PREFETCH >= 0) ? QS_PREFETCH : ((SCEN || KG >= 32) ? 1 : 0);
+    // PFM: prefetch the state rows into L2 before the draws -- measured per variant (profiles/README.md round 2)
+    constexpr int PFM = (SCEN || KG >= 32) ? 1 : 0;
     float4 *nz = reinterpret_cast<float4 *>(smem + park_off) + threadIdx.x;      // [4][blockDim.x]
     const int nz_stride = blockDim.x;
+    int *sl = reinterpret_cast<int *>(smem + park_off + 16 * blockDim.x) + 3 * threadIdx.x;
     auto early_draws = [&]() {
         const int nblk = c.sense_noise ? 4 : 1;
 #pragma unroll 1
@@ -1312,96 +1082,60 @@ __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_ke
             nz[i * nz_stride] = n;
         }
     };
-    if (PERSIST) {
-        cp_async_wait_all();
-        __syncwarp();
-        if (env < c.N) {
-            tick = sc[lane / KG]; svd = sc[GPW + lane / KG];
-            g.gid = (uint32_t)(c.env_id_offset + env);
-        }
-        mbar_wait(bar, phase);
-        phase ^= 1u;
-        if (valid) {
-            load_drone_smem(pf, row, q);
-            act = pf[PF_ACT * 32 + row];
-            ring = pf[PF_RING * 32 + row];
-            sums = pf[PF_SUMS * 32 + row];
-        }
-        __syncwarp();                                                   // every lane has read the buffer: refill it for the next tile
-        const int wn = wt + wt_stride;
-        if (wn < n_wt) {
-            if (lane == 0) prefetch_tile(P, actions, pf, bar, wn * GPW * c.K, max(0, min(GPW, c.N - wn * GPW)) * c.K);
-            const int e1 = wn * GPW + lane / KG;
-            if (e1 < c.N && d == 0) { cp_async4(sc + lane / KG, P.tick + e1); cp_async4(sc + GPW + lane / KG, P.svd_ctr + e1); }
-            cp_async_commit();
-        }
-    } else {
-        // Every prologue load is UNCONDITIONAL on a clamped, always-valid row (lanes past the batch / past K re-read a valid row and are
-        // overwritten below): one straight-line block, so that all loads are issued before the first consumer.  Under `if (valid)` the
-        // compiler closed the divergent region with register moves of the loaded values in front of the per-env scalar loads -- a
-        // second serialised HBM round trip at the top of every warp (profiles/tools/prologue_check.py guards this in the SASS).
-        const int env_c = min(env, c.N - 1), gi_c = env_c * c.K + min(d, c.K - 1);
-        g.gid = (uint32_t)(c.env_id_offset + env_c);
-        if (EARLY && PFM) {
-            // Pending register loads in front of the generator loop make the compiler copy some of their destinations out of the loop's
-            // registers first -- i.e. wait for the first load.  So the rows are PREFETCHED (no destination registers), the draws run
-            // while they travel from HBM, and the loads proper follow as cache hits.
+    // Every prologue load is UNCONDITIONAL on a clamped, always-valid row (lanes past the batch / past K re-read a valid row and are
+    // overwritten below): one straight-line block, so that all loads are issued before the first consumer.  Under `if (valid)` the
+    // compiler closed the divergent region with register moves of the loaded values in front of the per-env scalar loads -- a
+    // second serialised HBM round trip at the top of every warp (profiles/tools/prologue_check.py guards this in the SASS).
+    const int env_c = min(env, c.N - 1), gi_c = env_c * c.K + min(d, c.K - 1);
+    g.gid = (uint32_t)(c.env_id_offset + env_c);
+    if (PFM) {
+        // Pending register loads in front of the generator loop make the compiler copy some of their destinations out of the loop's
+        // registers first -- i.e. wait for the first load.  So the rows are PREFETCHED (no destination registers), the draws run
+        // while they travel from HBM, and the loads proper follow as cache hits.
 #pragma unroll
-            for (int pl = 0; pl < PL_COUNT; ++pl) prefetch_row(P.plane[pl] + gi_c);
-            prefetch_row(actions + gi_c);
-            if (d == 0) { prefetch_row(P.tick + env_c); prefetch_row(P.svd_ctr + env_c); }
-            int *sl = reinterpret_cast<int *>(smem + park_off + 16 * blockDim.x) + 3 * threadIdx.x;
-            if (HOT) { cp_async4(sl + 2, P.hot_flag_cur + min(wt, n_wt - 1)); cp_async_commit(); }
-            early_draws();
-            if (HOT) {
-                cp_async_wait_all();
-                if (!hot_role && sl[2] != 0) {
-                    if (lane == 0 && wt < n_wt) P.hot_flag_cur[wt] = 0;
-                    return;
-                }
+        for (int pl = 0; pl < PL_COUNT; ++pl) prefetch_row(P.plane[pl] + gi_c);
+        prefetch_row(actions + gi_c);
+        if (d == 0) { prefetch_row(P.tick + env_c); prefetch_row(P.svd_ctr + env_c); }
+        if (HOT) { cp_async4(sl + 2, P.hot_flag_cur + min(wt, n_wt - 1)); cp_async_commit(); }
+        early_draws();
+        if (HOT) {
+            cp_async_wait_all();
+            if (!hot_role && sl[2] != 0) {
+                if (lane == 0 && wt < n_wt) P.hot_flag_cur[wt] = 0;
+                return;
             }
         }
-        if (EARLY && !PFM) {
-            // The two per-env scalars travel global -> shared (LDGSTS) and are read after the draws below: as pending register loads
-            // the compiler copied them out of the generator loop's registers first, i.e. waited for them before the loop.
-            int *sl = reinterpret_cast<int *>(smem + park_off + 16 * blockDim.x) + 3 * threadIdx.x;
-            cp_async4(sl, P.tick + env_c); cp_async4(sl + 1, P.svd_ctr + env_c);
-            if (HOT) cp_async4(sl + 2, P.hot_flag_cur + min(wt, n_wt - 1));
-            cp_async_commit();
-        } else { tick = P.tick[env_c]; svd = P.svd_ctr[env_c]; }
-        if (SCEN) {                                                     // scenario row: loaded with the state, parked in shared memory
-#pragma unroll
-            for (int k = 0; k < (QS_SC_COUNT / 4 + KG - 1) / KG; ++k)
-                sc_row[k] = P.scen[(size_t)env_c * (QS_SC_COUNT / 4) + min(d + k * KG, QS_SC_COUNT / 4 - 1)];
-        }
-        load_drone<!PARK>(P, gi_c, q);
-        act = __ldcs(actions + gi_c);
-        // The last-5-s window sums (:762-767) are only needed in the last 500 steps of an episode, but the load is unconditional: a
-        // predicate on `tick` made the compiler wait for the tick load BEFORE issuing the state loads (79.0 -> 76.6 us for 16 extra
-        // bytes read per drone-step).  QS_PARK: goal, distance ring and window sums are not needed before the dynamics have run
-        // (~1100 instructions), so they go global -> shared directly (LDGSTS) and hold no registers meanwhile.
-        if (PARK) {
-            cp_async16(park, P.plane[PL_GOAL] + gi_c);
-            cp_async16(park + park_stride, P.plane[PL_DIST_RING] + gi_c);
-            cp_async16(park + 2 * park_stride, P.plane[PL_DIST_SUMS] + gi_c);
-            cp_async_commit();
-        } else {
-            ring = __ldcs(P.plane[PL_DIST_RING] + gi_c);
-            sums = __ldcs(P.plane[PL_DIST_SUMS] + gi_c);
-        }
+        tick = P.tick[env_c]; svd = P.svd_ctr[env_c];
+    } else {
+        // The two per-env scalars travel global -> shared (LDGSTS) and are read after the draws below: as pending register loads
+        // the compiler copied them out of the generator loop's registers first, i.e. waited for them before the loop.
+        cp_async4(sl, P.tick + env_c); cp_async4(sl + 1, P.svd_ctr + env_c);
+        if (HOT) cp_async4(sl + 2, P.hot_flag_cur + min(wt, n_wt - 1));
+        cp_async_commit();
     }
-    if (EARLY && !PFM) {
+    if (SCEN) {                                                         // scenario row: loaded with the state, parked in shared memory
+#pragma unroll
+        for (int k = 0; k < (QS_SC_COUNT / 4 + KG - 1) / KG; ++k)
+            sc_row[k] = P.scen[(size_t)env_c * (QS_SC_COUNT / 4) + min(d + k * KG, QS_SC_COUNT / 4 - 1)];
+    }
+    load_drone(P, gi_c, q);
+    act = __ldcs(actions + gi_c);
+    // The last-5-s window sums (:762-767) are only needed in the last 500 steps of an episode, but the load is unconditional: a
+    // predicate on `tick` made the compiler wait for the tick load BEFORE issuing the state loads (79.0 -> 76.6 us for 16 extra
+    // bytes read per drone-step).
+    ring = __ldcs(P.plane[PL_DIST_RING] + gi_c);
+    sums = __ldcs(P.plane[PL_DIST_SUMS] + gi_c);
+    if (!PFM) {
         early_draws();
         cp_async_wait_all();
-        const int *sl = reinterpret_cast<const int *>(smem + park_off + 16 * blockDim.x) + 3 * threadIdx.x;
         tick = sl[0]; svd = sl[1];
         if (HOT && !hot_role && sl[2] != 0) {                           // a hot block processes this tile in this step
             if (lane == 0 && wt < n_wt) P.hot_flag_cur[wt] = 0;         // leave the buffer clean for its next use
             return;
         }
     }
-    if (!PERSIST && env >= c.N) { tick = 0; svd = 0; }                 // first consumer of a loaded value: after the draws
-    if (SCEN && !PERSIST) {
+    if (env >= c.N) { tick = 0; svd = 0; }                              // first consumer of a loaded value: after the draws
+    if (SCEN) {
         if (env < c.N) {
 #pragma unroll
             for (int k = 0; k < (QS_SC_COUNT / 4 + KG - 1) / KG; ++k)
@@ -1442,7 +1176,7 @@ __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_ke
 #pragma unroll
     for (int m = 0; m < 4; ++m) cmd[m] = 0.5f * (clampf(a4[m], -1.0f, 1.0f) + 1.0f);
     if (valid) {
-        const float4 nv = EARLY ? nz[0] : rng_n4v(g, SITE_OU, d, 0, 0);   // OUNoiseNumba.noise, numba_utils.py:101-105
+        const float4 nv = nz[0];                                       // OUNoiseNumba.noise, numba_utils.py:101-105
         const float n[4] = { nv.x, nv.y, nv.z, nv.w };
 #pragma unroll
         for (int m = 0; m < 4; ++m) q.ou[m] = q.ou[m] + (c.ou_theta * (0.0f - q.ou[m]) + c.ou_sigma * n[m]);
@@ -1452,13 +1186,7 @@ __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_ke
             if (fire) svd = 0;
             dynamics_substep(c, g, d, q, cmd, s, fire);
         }
-#if QS_EARLY_STORE
         store_motor_planes(P, gi, q);                                  // final (a reset below rewrites them): 12 registers less from here on
-#endif
-    }
-    if (PARK) {
-        cp_async_wait_all();                                           // this thread's parked rows have landed
-        if (valid) { const float4 k = park[0]; q.goal[0] = k.x; q.goal[1] = k.y; q.goal[2] = k.z; }
     }
     // ---- compute_reward_weighted (quadrotor_single.py:34-92), dt = physics dt
     const bool on_floor = (q.flags & F_ON_FLOOR) != 0;
@@ -1480,12 +1208,6 @@ __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_ke
     const uint32_t bad_ballot = __ballot_sync(QS_FULL, bad) & gmask;
     const bool all_done = (tick > c.ep_len) || (bad_ballot != 0u);     // quadrotor_single.py:366-367
 
-#ifdef QS_BULK_STORE
-    if (PERSIST) {                                                      // the previous tile's bulk store has read the observation tile
-        if (lane == 0) bulk_store_wait_read();
-        __syncwarp();
-    }
-#endif
     // ---- 1.1 drone-drone collisions (collisions/quadrotors.py:63-103, quadrotor_multi.py:537-568)
     uint32_t rowmask = 0u;
     float prox = 0.f;
@@ -1559,7 +1281,6 @@ __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_ke
     if (OBST) scen_now = (q.flags & F_SCEN_OSTATIC) ? QS_SCENARIO_O_STATIC_SAME_GOAL : QS_SCENARIO_O_RANDOM;
     // distance_to_goal log: reached-goal flag from the mean of the last 5 entries, and the 1/3/5 s windows (:651-655, 762-767)
     if (valid) {
-        if (PARK) { ring = park[park_stride]; sums = park[2 * park_stride]; }
         float dlog = c.dt * dist;                                      // -rewraw_pos
         if (tick >= 5 && !(q.flags & F_REACHED)) {
             float m5 = (ring.x + ring.y + ring.z + ring.w + dlog) / 5.0f;
@@ -1696,7 +1417,7 @@ __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_ke
         SensorNoise sn;
         sn.n = sn.m = sn.l = make_float4(0.f, 0.f, 0.f, 0.f);
         if (c.sense_noise) {
-            if (__builtin_expect(flag, 0) || !EARLY) sn = sensor_noise(g, flag ? SITE_SENSOR_IMPULSE : SITE_SENSOR, d);
+            if (__builtin_expect(flag, 0)) sn = sensor_noise(g, flag ? SITE_SENSOR_IMPULSE : SITE_SENSOR, d);
             else { sn.n = nz[nz_stride]; sn.m = nz[2 * nz_stride]; sn.l = nz[3 * nz_stride]; }
         }
         self_obs(c, sn, q, orow);
@@ -1774,24 +1495,18 @@ __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_ke
             }
             int scen = 0;
             if (bad_ballot) {                                           // do not let NaNs leak through the persistent noise state
-#if QS_EARLY_STORE
                 if (valid) { const float4 h = P.plane[PL_OU][gi]; q.ou[0] = h.x; q.ou[1] = h.y; q.ou[2] = h.z; q.ou[3] = h.w; }   // written above by this thread
-#endif
 #pragma unroll
                 for (int m = 0; m < 4; ++m) q.ou[m] = isfinite(q.ou[m]) ? q.ou[m] : 0.f;
-#if QS_EARLY_STORE
                 if (valid) P.plane[PL_OU][gi] = make_float4(q.ou[0], q.ou[1], q.ou[2], q.ou[3]);
-#endif
                 if (!isfinite(vs[0] + vs[1] + vs[2])) { vs[0] = vs[1] = vs[2] = 0.f; }
             }
             group_reset<KG, OBST, SCEN>(c, P, g, env, d, valid, gmask, tile + (size_t)(lane / KG) * c.K * c.D, c.K * c.D,
                                         OBST ? ob_sm + (lane / KG) * c.M : nullptr, q, scen);
-#if QS_EARLY_STORE
             if (valid) {                                                // the motor lag restarts at rest (quadrotor_dynamics.py:176-178)
                 P.plane[PL_ROT_DAMP][gi] = make_float4(0.f, 0.f, 0.f, 0.f);
                 P.plane[PL_CMDS_DAMP][gi] = make_float4(0.f, 0.f, 0.f, 0.f);
             }
-#endif
             tick = 0;
             if (valid) {
                 if (d == 0) {
@@ -1818,7 +1533,7 @@ __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_ke
 
     // ---- write back
     if (valid) {
-        store_drone<!QS_EARLY_STORE>(P, gi, q, SCEN || all_done);
+        store_drone<false>(P, gi, q, SCEN || all_done);   // the motor planes were written after the dynamics
         if (d == 0) { P.tick[env] = tick; P.svd_ctr[env] = svd; }
     }
     if (HOT) {
@@ -1830,17 +1545,9 @@ __global__ void __launch_bounds__(QS_STEP_MAXTHREADS, QS_STEP_MINBLOCKS) step_ke
         }
     }
     __syncwarp();
-#ifdef QS_BULK_STORE
-    if (warp_rows > 0) warp_store_tile_bulk(tile, obs + (size_t)warp_env0 * c.K * c.D, warp_rows * c.D, lane);
-    if (!PERSIST && lane == 0) bulk_store_wait_read();                  // shared memory must outlive the copy
-#else
     if (warp_rows > 0) warp_store_tile(tile, obs + (size_t)warp_env0 * c.K * c.D, warp_rows * c.D, lane);
-#endif
-    __syncwarp();                                                       // the tile and the exchange buffer are reused by the next warp-tile
+    __syncwarp();
     }   // warp-tile loop
-#ifdef QS_BULK_STORE
-    if (PERSIST && lane == 0) bulk_store_wait_read();
-#endif
 }
 
 // ----------------------------------------------------------------------------------------------------------------

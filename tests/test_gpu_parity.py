@@ -426,37 +426,6 @@ def test_episode_stats_match_oracle():
     assert gs["agents_success"] + gs["agents_deadlock"] + gs["agents_collided"] == 2 * N * K
 
 
-@pytest.mark.parametrize("name,n_envs", [("cfg2_k8", 203), ("odd_k3", 77), ("cfg4_k32", 9), ("cfg3_obst_k8", 61), ("single_k1", 333)])
-def test_persistent_tma_kernel_is_bitwise_the_plain_kernel(name, n_envs, monkeypatch):
-    """The persistent form of the step kernel (warp-tile loop, TMA bulk prefetch of the next tile through an mbarrier)
-    computes exactly what the one-tile-per-warp form computes: same bits in obs / rew / done / state, including partial
-    last tiles, non-power-of-two K, resets inside the window, and several tiles per warp (grid forced to 3 blocks)."""
-    import torch
-    kw = dict(CONFIGS[name], num_envs=n_envs, ep_time=0.12)
-    cfg = QuadSimConfig(seed=17, **kw)
-    monkeypatch.setenv("QS_PERSIST", "0")
-    plain = _sim(cfg)
-    monkeypatch.setenv("QS_PERSIST", "1")
-    monkeypatch.setenv("QS_PERSIST_BLOCKS", "3")
-    pers = _sim(cfg)
-    monkeypatch.delenv("QS_PERSIST"); monkeypatch.delenv("QS_PERSIST_BLOCKS")
-    assert torch.equal(plain.reset(), pers.reset())
-    rs = np.random.RandomState(4)
-    n_done = 0
-    for s in range(30):
-        a = torch.from_numpy(action_batch(rs, cfg.num_envs * cfg.num_agents, "uniform")).cuda()
-        o1, r1, d1 = plain.step(a)
-        o2, r2, d2 = pers.step(a)
-        assert torch.equal(o1, o2) and torch.equal(r1, r2) and torch.equal(d1, d2), f"step {s}"
-        assert torch.equal(plain.terminal_obs, pers.terminal_obs)
-        n_done += int(d1.any())
-    assert n_done >= 2
-    s1, s2 = plain.get_state(), pers.get_state()
-    for k in s1:
-        assert torch.equal(s1[k], s2[k]), k
-    assert plain.episode_stats() == pers.episode_stats()
-
-
 # ------------------------------------------------------------------------------------------------------------------
 # oracle parity AT THE BENCHMARKED LAUNCH SHAPES (BASELINE.json configs[1..4]): 128-thread blocks, full grids
 # ------------------------------------------------------------------------------------------------------------------
