@@ -381,6 +381,28 @@ enum { QS_RI_RAW_POS = 0,           /* rewraw_pos = rewraw_main; fork mode: goal
        QS_RI_COUNT = 8 };
 int qs_set_reward_info(qs_env *env, float *rew_info);
 
+/* Snapshots: the whole simulator state of a handle as one self-describing HOST blob, for checkpoints and exact resumes
+ * (reference: the env side of SB3 model.save / CheckpointCallback, which the reference cannot restore at all).  A step after
+ * qs_restore is bitwise the step the snapshotted handle would have taken next.
+ *   Layout (native byte order): uint32 magic "QSSN" | uint32 QS_SNAPSHOT_VERSION | uint64 sizeof(qs_config) | at offset 16 the
+ *   handle's current qs_config, qs_set_param changes included | uint32 RNG launch counter | uint32 section count | uint64 bytes of
+ *   every section | the sections, dense, in a fixed order: the state planes; per-env tick, svd counter, episode counters; obstacle
+ *   centres [N, QS_MAX_OBSTACLES] (use_obstacles only); scenario rows (formation scenarios only); episode records (env rows, drone
+ *   rows); qs_stats; fork mode: the PID / heading planes, evader, per-env fork flags.  A section absent in the mode has size 0.
+ *   Section sizes depend on N, K and the mode only, never on the launch shape, so a snapshot restores into any handle created
+ *   with the same qs_config, seed and env_id_offset included: a shard restores into its own handle only.
+ *   Not stored: the launch count, the reset-first scheduling lists (qs_restore empties them, as qs_create leaves them), the
+ *   staging buffers of the *_host calls, and the qs_set_reward_info pointer (the target handle keeps its own).
+ * Both calls take pinned or pageable host memory and return after `stream` has drained.  qs_snapshot writes
+ * qs_snapshot_size(env) bytes (`bytes` may be larger).  qs_restore needs `bytes` equal to the target's size; it checks the header
+ * and every qs_config field except the qs_set_param ones (those are taken from the snapshot) before it copies anything, and on a
+ * mismatch returns QS_ERR_SHAPE (blob: magic, version, sizes) or QS_ERR_BAD_CONFIG (configuration) with the first differing
+ * field named in qs_last_error, leaving the handle untouched. */
+#define QS_SNAPSHOT_VERSION 1
+size_t qs_snapshot_size(const qs_env *env);                                   /* 0 for NULL */
+int    qs_snapshot(qs_env *env, void *dst_host, size_t bytes, void *stream);
+int    qs_restore(qs_env *env, const void *src_host, size_t bytes, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

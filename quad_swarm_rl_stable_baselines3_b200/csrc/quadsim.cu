@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 
 #include <cmath>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -141,6 +142,7 @@ struct qs_env {
     // reset-first scheduling of the upstream step kernel (DevPtrs::hot_*): three rotating buffers in the slab
     int *hot_list[3], *hot_cnt[3], *hot_flag[3];
     int hot_cap, hot_blocks; unsigned hot_phase; bool hot;
+    size_t hot_bytes;       // the three buffers back to back from hot_cnt[0]
     uint32_t rng_step;      // Philox counter word 1: +1 per step / reset call (+ fork.substeps per fork step); the same for every env of the handle
     bool host_ready;        // staging buffers of the *_host entry points are allocated
     std::string err;
@@ -352,6 +354,102 @@ static int ensure_host_buffers(qs_env *e)
     return QS_OK;
 }
 
+// the qs_config field a QS_PARAM_* key sets (nullptr for an unknown key)
+static double *param_field(qs_config &c, int key)
+{
+    switch (key) {
+        case QS_PARAM_REW_POS: return &c.rew_pos;
+        case QS_PARAM_REW_EFFORT: return &c.rew_effort;
+        case QS_PARAM_REW_CRASH: return &c.rew_crash;
+        case QS_PARAM_REW_ORIENT: return &c.rew_orient;
+        case QS_PARAM_REW_SPIN: return &c.rew_spin;
+        case QS_PARAM_REW_QUADCOL_BIN: return &c.rew_quadcol_bin;
+        case QS_PARAM_REW_QUADCOL_BIN_SMOOTH_MAX: return &c.rew_quadcol_bin_smooth_max;
+        case QS_PARAM_REW_QUADCOL_BIN_OBST: return &c.rew_quadcol_bin_obst;
+        case QS_PARAM_CAPTURE_RADIUS: return &c.fork.capture_radius;
+        default: return nullptr;
+    }
+}
+
+// ---- snapshots (include/quadsim.h) -------------------------------------------------------------------------------------------
+// Every qs_config field except the reserved words, in declaration order: qs_restore compares field by field (padding bytes carry
+// no meaning) so that its message can name the first field that differs.  Arrays compare as a whole.
+#define QS_CONFIG_FIELDS(X)                                                                                                      \
+    X(api_version) X(num_envs) X(num_agents) X(scenario) X(obs_repr) X(neighbor_obs_type) X(neighbor_visible_num)             \
+    X(use_obstacles) X(use_downwash) X(apply_collision_force) X(sense_noise) X(ep_len) X(sim_steps) X(svd_period)               \
+    X(obst_area_len) X(obst_area_wid) X(num_obstacles) X(env_mode) X(cube_dim) X(seed) X(env_id_offset) X(dt) X(room_dims)     \
+    X(gravity) X(mass) X(inertia) X(thrust_max) X(torque_max) X(prop_cross) X(prop_ccw) X(arm) X(motor_tau_up)                 \
+    X(motor_tau_down) X(motor_linearity) X(vel_damp) X(damp_omega_quadratic) X(omega_max) X(floor_mu) X(ou_theta) X(ou_sigma) \
+    X(sense_pos_std) X(sense_vel_std) X(sense_gyro_std) X(rew_pos) X(rew_effort) X(rew_crash) X(rew_orient) X(rew_spin)       \
+    X(rew_quadcol_bin) X(rew_quadcol_bin_smooth_max) X(rew_quadcol_bin_obst) X(collision_hitbox_radius)                        \
+    X(collision_falloff_radius) X(spawn_box) X(spawn_min_z) X(obst_size) X(sdf_resolution) X(approach_goal_metric)             \
+    X(fork.substeps) X(fork.capture_radius) X(fork.rew_existence) X(fork.rew_captor) X(fork.rew_helper)                        \
+    X(fork.max_angular_rate) X(fork.chaser_speed) X(fork.evader_v_max) X(fork.evader_dt) X(fork.evader_arena)                   \
+    X(fork.spawn_ring) X(fork.evader_r_min) X(fork.evader_r_span) X(fork.pid) X(fork.rate_out_scale) X(fork.mixer)             \
+    X(fork.ctrl_mass) X(fork.ctrl_g) X(fork.ctrl_kf) X(fork.ctrl_min_rpm) X(fork.ctrl_max_rpm) X(fork.cam_focal_length)       \
+    X(fork.cam_target_size) X(fork.cam_pixel_noise) X(fork.cam_fov_deg) X(fork.cam_resolution) X(fork.cam_num)
+
+#define QS_FIELD_BYTES(f) + sizeof(((const qs_config *)nullptr)->f)
+static_assert(0 QS_CONFIG_FIELDS(QS_FIELD_BYTES) + 3 * sizeof(int32_t) == sizeof(qs_config),
+              "QS_CONFIG_FIELDS must list every qs_config field but reserved0, fork.reserved and fork.reserved2");
+#undef QS_FIELD_BYTES
+
+static const char *first_config_difference(const qs_config &a, const qs_config &b)
+{
+#define QS_CMP_FIELD(f) if (memcmp(&a.f, &b.f, sizeof(a.f)) != 0) return #f;
+    QS_CONFIG_FIELDS(QS_CMP_FIELD)
+#undef QS_CMP_FIELD
+    return nullptr;
+}
+
+// Sections of a snapshot, in blob order.  Sizes follow from N, K and the mode alone (never from the slab's alignment or the launch
+// shape); a section the mode does not have is 0 bytes.
+enum { SEC_PLANES = 0, SEC_TICK = SEC_PLANES + PL_COUNT, SEC_SVD, SEC_ECNT, SEC_OBST, SEC_SCEN, SEC_EP_REC, SEC_EP_AGENT, SEC_STATS,
+       SEC_FPLANES, SEC_EVADER = SEC_FPLANES + FP_COUNT, SEC_FFLAGS, SEC_COUNT };
+
+struct SnapSection { void *dev; size_t bytes; };
+
+static void snapshot_sections(const qs_env *e, SnapSection s[SEC_COUNT])
+{
+    const size_t N = (size_t)e->cfg.num_envs, nd = N * e->cfg.num_agents;
+    for (int i = 0; i < SEC_COUNT; ++i) s[i] = { nullptr, 0 };
+    for (int p = 0; p < PL_COUNT; ++p) s[SEC_PLANES + p] = { e->dp.plane[p], nd * sizeof(float4) };
+    s[SEC_TICK] = { e->dp.tick, N * sizeof(int) };
+    s[SEC_SVD] = { e->dp.svd_ctr, N * sizeof(int) };
+    s[SEC_ECNT] = { e->dp.ecnt, N * EC_COUNT * sizeof(int) };
+    if (e->cfg.use_obstacles) s[SEC_OBST] = { e->dp.obst_xy, N * QS_MAX_OBSTACLES * sizeof(float2) };
+    if (e->dp.scen) s[SEC_SCEN] = { e->dp.scen, N * QS_SC_COUNT * sizeof(float) };
+    s[SEC_EP_REC] = { e->dp.ep_rec, N * QS_ER_COUNT * sizeof(int) };
+    s[SEC_EP_AGENT] = { e->dp.ep_agent, nd * sizeof(float4) };
+    s[SEC_STATS] = { e->dp.stats, sizeof(qs_stats) };
+    if (e->fork) {
+        for (int p = 0; p < FP_COUNT; ++p) s[SEC_FPLANES + p] = { e->fp.plane[p], nd * sizeof(float4) };
+        s[SEC_EVADER] = { e->fp.evader, N * sizeof(float2) };
+        s[SEC_FFLAGS] = { e->fp.flags, N * sizeof(int) };
+    }
+}
+
+static std::string section_name(int i)
+{
+    static const char *const names[] = { "tick", "svd_ctr", "episode counters", "obst_xy", "scenario", "ep_rec", "ep_agent", "stats" };
+    if (i < SEC_TICK) return "state plane " + std::to_string(i - SEC_PLANES);
+    if (i < SEC_FPLANES) return names[i - SEC_TICK];
+    if (i < SEC_EVADER) return "fork plane " + std::to_string(i - SEC_FPLANES);
+    return i == SEC_EVADER ? "evader" : "fork flags";
+}
+
+static const uint32_t SNAP_MAGIC = 0x4E535351u;     // the bytes "QSSN"
+
+struct SnapHeader {
+    uint32_t magic, version;
+    uint64_t config_size;
+    qs_config cfg;
+    uint32_t rng_step, sections;
+    uint64_t section_bytes[SEC_COUNT];
+};
+static_assert(offsetof(SnapHeader, cfg) == 16, "include/quadsim.h documents the configuration at offset 16");
+static_assert(sizeof(qs_config) % 8 == 0, "the snapshot header has no padding");
+
 extern "C" {
 
 size_t qs_config_size(void) { return sizeof(qs_config); }
@@ -423,6 +521,7 @@ int qs_create(const qs_config *cfg, int device, qs_env **out)
     e->hot_cap = 128; e->hot_blocks = e->hot_cap / warps;
     size_t o_hot[3];
     for (int b3 = 0; b3 < 3; ++b3) { o_hot[b3] = off; off += align((size_t)(e->hot_cap + 64 + n_wt) * sizeof(int)); }
+    e->hot_bytes = off - o_hot[0];
     size_t fplane_off[FP_COUNT] = {0}, o_evader = 0, o_fflags = 0;
     if (e->fork) {
         for (int p = 0; p < FP_COUNT; ++p) { fplane_off[p] = off; off += align(nd * sizeof(float4)); }
@@ -712,18 +811,9 @@ int qs_set_state(qs_env *e, const qs_state_view *view, void *stream) { return st
 int qs_set_param(qs_env *e, int key, double value)
 {
     if (!e) return QS_ERR_NULL;
-    switch (key) {
-        case QS_PARAM_REW_POS: e->cfg.rew_pos = value; break;
-        case QS_PARAM_REW_EFFORT: e->cfg.rew_effort = value; break;
-        case QS_PARAM_REW_CRASH: e->cfg.rew_crash = value; break;
-        case QS_PARAM_REW_ORIENT: e->cfg.rew_orient = value; break;
-        case QS_PARAM_REW_SPIN: e->cfg.rew_spin = value; break;
-        case QS_PARAM_REW_QUADCOL_BIN: e->cfg.rew_quadcol_bin = value; break;
-        case QS_PARAM_REW_QUADCOL_BIN_SMOOTH_MAX: e->cfg.rew_quadcol_bin_smooth_max = value; break;
-        case QS_PARAM_REW_QUADCOL_BIN_OBST: e->cfg.rew_quadcol_bin_obst = value; break;
-        case QS_PARAM_CAPTURE_RADIUS: e->cfg.fork.capture_radius = value; break;
-        default: return fail(e, QS_ERR_BAD_CONFIG, "qs_set_param: unknown key");
-    }
+    double *field = param_field(e->cfg, key);
+    if (!field) return fail(e, QS_ERR_BAD_CONFIG, "qs_set_param: unknown key");
+    *field = value;
     fill_const(e->cfg, e->dc);
     fill_fork(e->cfg, e->fc);
     return QS_OK;
@@ -768,6 +858,95 @@ int qs_episode_records_host(qs_env *e, int32_t *env_rec_host, float *agent_rec_h
     if (env_rec_host) QS_CUDA(e, cudaMemcpyAsync(env_rec_host, e->dp.ep_rec, N * QS_ER_COUNT * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
     if (agent_rec_host) QS_CUDA(e, cudaMemcpyAsync(agent_rec_host, e->dp.ep_agent, nd * sizeof(float4), cudaMemcpyDeviceToHost, s));
     QS_CUDA(e, cudaStreamSynchronize(s));
+    return QS_OK;
+}
+
+size_t qs_snapshot_size(const qs_env *e)
+{
+    if (!e) return 0;
+    SnapSection sec[SEC_COUNT];
+    snapshot_sections(e, sec);
+    size_t n = sizeof(SnapHeader);
+    for (int i = 0; i < SEC_COUNT; ++i) n += sec[i].bytes;
+    return n;
+}
+
+int qs_snapshot(qs_env *e, void *dst_host, size_t bytes, void *stream)
+{
+    if (!e || !dst_host) return fail(e, QS_ERR_NULL, "qs_snapshot: null argument");
+    const size_t need = qs_snapshot_size(e);
+    if (bytes < need)
+        return fail(e, QS_ERR_SHAPE, "qs_snapshot: the buffer has " + std::to_string(bytes) + " bytes, the snapshot " + std::to_string(need));
+    DeviceGuard guard(e->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    SnapSection sec[SEC_COUNT];
+    snapshot_sections(e, sec);
+    SnapHeader h;
+    memset(&h, 0, sizeof(h));
+    h.magic = SNAP_MAGIC; h.version = QS_SNAPSHOT_VERSION; h.config_size = sizeof(qs_config);
+    h.cfg = e->cfg; h.rng_step = e->rng_step; h.sections = SEC_COUNT;
+    for (int i = 0; i < SEC_COUNT; ++i) h.section_bytes[i] = sec[i].bytes;
+    memcpy(dst_host, &h, sizeof(h));
+    char *p = (char *)dst_host + sizeof(h);
+    for (int i = 0; i < SEC_COUNT; ++i) {
+        if (!sec[i].bytes) continue;
+        QS_CUDA(e, cudaMemcpyAsync(p, sec[i].dev, sec[i].bytes, cudaMemcpyDeviceToHost, s));
+        p += sec[i].bytes;
+    }
+    QS_CUDA(e, cudaStreamSynchronize(s));
+    return QS_OK;
+}
+
+int qs_restore(qs_env *e, const void *src_host, size_t bytes, void *stream)
+{
+    if (!e || !src_host) return fail(e, QS_ERR_NULL, "qs_restore: null argument");
+    // everything is checked before the first copy: a rejected snapshot leaves the handle as it was
+    const char *src = (const char *)src_host;
+    uint32_t magic = 0, version = 0;
+    if (bytes >= 8) { memcpy(&magic, src, 4); memcpy(&version, src + 4, 4); }
+    if (magic != SNAP_MAGIC) return fail(e, QS_ERR_SHAPE, "qs_restore: magic: not a simulator snapshot");
+    if (version != QS_SNAPSHOT_VERSION)
+        return fail(e, QS_ERR_SHAPE, "qs_restore: version: snapshot format " + std::to_string(version) + ", this library reads " +
+                                     std::to_string(QS_SNAPSHOT_VERSION));
+    if (bytes < sizeof(SnapHeader)) return fail(e, QS_ERR_SHAPE, "qs_restore: bytes: " + std::to_string(bytes) + " is shorter than the header");
+    SnapHeader h;
+    memcpy(&h, src, sizeof(h));
+    if (h.config_size != sizeof(qs_config))
+        return fail(e, QS_ERR_SHAPE, "qs_restore: config_size: the snapshot's qs_config has " + std::to_string(h.config_size) + " bytes, this library's " +
+                                     std::to_string(sizeof(qs_config)));
+    qs_config want = e->cfg;                                            // the qs_set_param values come from the snapshot
+    for (int k = 0; k < QS_PARAM_COUNT; ++k) *param_field(want, k) = *param_field(h.cfg, k);
+    if (const char *f = first_config_difference(want, h.cfg))
+        return fail(e, QS_ERR_BAD_CONFIG, std::string("qs_restore: ") + f + ": the snapshot's configuration differs from the handle's");
+    SnapSection sec[SEC_COUNT];
+    snapshot_sections(e, sec);
+    if (h.sections != SEC_COUNT) return fail(e, QS_ERR_SHAPE, "qs_restore: sections: " + std::to_string(h.sections) + ", expected " + std::to_string((int)SEC_COUNT));
+    size_t need = sizeof(SnapHeader);
+    for (int i = 0; i < SEC_COUNT; ++i) {
+        if (h.section_bytes[i] != sec[i].bytes)
+            return fail(e, QS_ERR_SHAPE, "qs_restore: section " + section_name(i) + ": " + std::to_string(h.section_bytes[i]) + " bytes, expected " +
+                                         std::to_string(sec[i].bytes));
+        need += sec[i].bytes;
+    }
+    if (bytes != need)
+        return fail(e, QS_ERR_SHAPE, "qs_restore: bytes: the blob has " + std::to_string(bytes) + ", a snapshot of this handle " + std::to_string(need));
+    DeviceGuard guard(e->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    const char *p = src + sizeof(SnapHeader);
+    for (int i = 0; i < SEC_COUNT; ++i) {
+        if (!sec[i].bytes) continue;
+        QS_CUDA(e, cudaMemcpyAsync(sec[i].dev, p, sec[i].bytes, cudaMemcpyHostToDevice, s));
+        p += sec[i].bytes;
+    }
+    // reset-first lists as qs_create leaves them: zero counts and flags make every warp-tile a regular block's (the hot blocks find
+    // no listed tile and return), and the step results do not depend on the schedule
+    QS_CUDA(e, cudaMemsetAsync(e->hot_cnt[0], 0, e->hot_bytes, s));
+    QS_CUDA(e, cudaStreamSynchronize(s));
+    e->cfg = want;
+    e->rng_step = h.rng_step;
+    e->hot_phase = 0;
+    fill_const(e->cfg, e->dc);
+    fill_fork(e->cfg, e->fc);
     return QS_OK;
 }
 

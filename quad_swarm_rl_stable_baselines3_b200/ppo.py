@@ -23,7 +23,7 @@ from __future__ import annotations
 
 import math
 import time
-from dataclasses import dataclass
+from dataclasses import asdict, dataclass
 from typing import Dict, Optional
 
 import torch
@@ -286,6 +286,7 @@ class DevicePPO:
         self._flat = None
         self.obs = sim.reset().clone()
         self.total_agent_steps = 0
+        self._rollout_pending = False                             # collect() filled the buffers, update() has not consumed them
         self.fused = None
         if self.p.fused_rollout and self.device.type == "cuda":
             from . import fused_policy
@@ -324,6 +325,7 @@ class DevicePPO:
                 last_v = self.policy.value(self.obs).float()
             self.adv, self.ret = compute_gae(self.rew_buf, self.val_buf, self.done_buf, last_v, p.gamma, p.gae_lambda)
         self._sync()
+        self._rollout_pending = True
         n = self.obs.shape[0]
         self.total_agent_steps += n * p.n_steps * self.world
         return {"rollout_s": time.perf_counter() - t0, "mean_reward": float(self.rew_buf.mean()),
@@ -391,6 +393,7 @@ class DevicePPO:
         if self.fused is not None:
             self.fused.sync()                                          # re-pack the updated weights for the next rollout
         self._sync()
+        self._rollout_pending = False
         out = dict(zip(("pg", "vf", "ent", "kl", "clip_frac"), (acc / max(nb, 1)).tolist()))
         out["update_s"] = time.perf_counter() - t0
         out["minibatches"] = nb
@@ -407,3 +410,53 @@ class DevicePPO:
             if log:
                 log(row)
         return hist
+
+    # ---- checkpoints (SB3 model.save / CheckpointCallback) ---------------------------------------------------------
+    CHECKPOINT_VERSION = 1
+
+    def save(self, path) -> None:
+        """Write a checkpoint between iterations: configurations, policy and Adam state, step count, the last observation, the torch
+        RNG states (exploration noise, minibatch permutations) and the exact simulator snapshot.  Only tensors and plain containers,
+        so `torch.load(path, weights_only=True)` reads it.  Under torchrun every rank saves its own file (its env shard).  The rollout
+        buffers are not saved: saving between collect() and update() raises RuntimeError."""
+        if self._rollout_pending:
+            raise RuntimeError("DevicePPO.save: collect() filled a rollout that update() has not used yet; save between iterations")
+        self._sync()
+        ckpt = {
+            "version": self.CHECKPOINT_VERSION,
+            "ppo_config": asdict(self.p),
+            "sim_config": asdict(self.cfg),
+            "policy": self.policy.state_dict(),
+            "optimizer": self.opt.state_dict(),
+            "total_agent_steps": self.total_agent_steps,
+            "obs": self.obs.cpu(),
+            "rng_cpu": torch.get_rng_state(),
+            "rng_cuda": torch.cuda.get_rng_state(self.device) if self.device.type == "cuda" else None,
+            "sim": self.sim.snapshot(),
+        }
+        torch.save(ckpt, path)
+
+    def load(self, path) -> None:
+        """Resume from `save(path)` on a freshly built DevicePPO whose simulator has the same configuration (the simulator rejects
+        another one; the policy architecture must match exactly).  The live PPOConfig keeps the optimisation hyperparameters: the
+        learning rate is set back to `self.p.learning_rate` after Adam's state is loaded.  The next collect() continues the saved
+        run bitwise."""
+        ckpt = torch.load(path, map_location="cpu", weights_only=True)
+        if ckpt.get("version") != self.CHECKPOINT_VERSION:
+            raise ValueError(f"DevicePPO.load: checkpoint format {ckpt.get('version')!r}, this code reads {self.CHECKPOINT_VERSION}")
+        if tuple(ckpt["obs"].shape) != tuple(self.obs.shape):
+            raise ValueError(f"DevicePPO.load: checkpoint observations {tuple(ckpt['obs'].shape)}, this run's {tuple(self.obs.shape)}")
+        self.sim.restore(ckpt["sim"])
+        self.policy.load_state_dict(ckpt["policy"], strict=True)
+        self.opt.load_state_dict(ckpt["optimizer"])
+        for g in self.opt.param_groups:
+            g["lr"] = self.p.learning_rate
+        self.total_agent_steps = int(ckpt["total_agent_steps"])
+        self.obs.copy_(ckpt["obs"])
+        torch.set_rng_state(ckpt["rng_cpu"])
+        if self.device.type == "cuda":
+            torch.cuda.set_rng_state(ckpt["rng_cuda"], self.device)
+        self._rollout_pending = False
+        if self.fused is not None:
+            self.fused.sync()
+        self._sync()

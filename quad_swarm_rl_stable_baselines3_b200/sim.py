@@ -14,7 +14,7 @@ import numpy as np
 import torch
 
 from . import _capi
-from .config import PARAM_KEYS, QS_ER_COUNT, QS_SC_COUNT, QsStateViewC, QsStatsC, QuadSimConfig
+from .config import PARAM_KEYS, QS_ER_COUNT, QS_SC_COUNT, QsConfigC, QsStateViewC, QsStatsC, QuadSimConfig
 
 _STATE_SHAPES = {"pos": (3, torch.float32), "vel": (3, torch.float32), "rot": (9, torch.float32),
                  "omega": (3, torch.float32), "rot_damp": (4, torch.float32), "cmds_damp": (4, torch.float32),
@@ -251,6 +251,35 @@ class QuadSwarmSim:
             rc = self._lib.qs_episode_records_host(self._h, env.ctypes.data, agent.ctypes.data, self._stream())
         _capi.check(self._h, rc, "qs_episode_records_host")
         return env, agent
+
+    # snapshots: exact save / resume ------------------------------------------------------------------
+    def snapshot(self) -> Dict[str, torch.Tensor]:
+        """The whole simulator state (`qs_snapshot`, include/quadsim.h) plus the last observation, on the host:
+        {"blob": uint8 pinned CPU tensor, "obs": float32 CPU tensor [N*K, D]}.  `restore` on any handle created with the same
+        configuration continues bitwise where this one stands."""
+        n = int(self._lib.qs_snapshot_size(self._h))
+        blob = torch.empty(n, dtype=torch.uint8, pin_memory=True)
+        with torch.cuda.device(self.device):
+            rc = self._lib.qs_snapshot(self._h, C.c_void_p(blob.data_ptr()), n, self._stream())
+        _capi.check(self._h, rc, "qs_snapshot")
+        return {"blob": blob, "obs": self.obs.cpu()}
+
+    def restore(self, snap: Dict[str, torch.Tensor]) -> torch.Tensor:
+        """Load a `snapshot()` into this handle (`qs_restore` rejects one of another configuration and leaves the handle as it was).
+        The snapshot's reward coefficients / capture radius replace this handle's.  Returns the restored observation (self.obs)."""
+        blob = torch.as_tensor(snap["blob"]).detach().to("cpu", torch.uint8).contiguous().reshape(-1)
+        obs = torch.as_tensor(snap["obs"])
+        if obs.numel() != self.obs.numel():
+            raise ValueError(f"snapshot obs has {obs.numel()} values, this simulator's observation {self.obs.numel()}")
+        with torch.cuda.device(self.device):
+            rc = self._lib.qs_restore(self._h, C.c_void_p(blob.data_ptr()), blob.numel(), self._stream())
+        _capi.check(self._h, rc, "qs_restore")
+        self.obs.copy_(obs.reshape(self.obs.shape))
+        # the qs_config of the snapshot sits at offset 16 of the blob (include/quadsim.h)
+        c = QsConfigC.from_buffer_copy(blob[16:16 + C.sizeof(QsConfigC)].numpy().tobytes())
+        self.rew_coeff_overrides = {k: getattr(c, "rew_" + k) for k in PARAM_KEYS if k != "capture_radius"
+                                    and getattr(c, "rew_" + k) != getattr(self._c, "rew_" + k)}
+        return self.obs
 
     # parameters / stats ------------------------------------------------------------------------------
     def set_rew_coeff(self, **coeffs):
