@@ -64,6 +64,44 @@ CONFIGS = {
                         obs_repr="xyz_vxyz_R_omega_floor", ep_time=0.3),
 }
 
+# Every feature variant of the step and reset kernels at the lane-group widths 2, 4, 16 and 32 (KG = the power of two >= K, the
+# lanes of one env), with K below the width wherever it can be so that padding lanes exist, and the neighbour-selection paths of
+# the obstacle variants that no other case reaches.  The path of group_obs_tail (quadsim_kernels.cuh) that each case reaches is
+# noted with V: "first minimum" when (KG >= 16 or obstacles and KG >= 4) and 3 V < 2 (KG - 1); else the packed rank count for
+# KG <= 8; else the all-pairs rank count; "all" when V = K - 1.
+# Run by test_reset_parity (explicit and masked reset) here and test_staggered_parity (step) in test_gpu_staggered.py.
+# name: (config kwargs, envs, action kind); the envs leave the last warp-tile partial.
+_OBST = dict(use_obstacles=True, obs_repr="xyz_vxyz_R_omega_floor")
+WIDTH_CELLS = {
+    "feat0_k2": (dict(num_agents=2, neighbor_visible_num=1), 27, "uniform"),                                    # all
+    "feat1_obst_k2": (dict(num_agents=2, quads_mode="o_random", neighbor_visible_num=1, **_OBST), 27, "hover"),  # all
+    "feat2_downwash_k2": (dict(num_agents=2, use_downwash=True, neighbor_visible_num=1), 27, "uniform"),         # all
+    "feat3_obst_downwash_k2": (dict(num_agents=2, quads_mode="mix", use_downwash=True, neighbor_visible_num=1, **_OBST), 27, "hover"),
+    "feat6_runaway_downwash_k2": (dict(num_agents=2, quads_mode="run_away", use_downwash=True, neighbor_visible_num=1), 27, "hover"),
+    "feat1_obst_k3_v1": (dict(num_agents=3, quads_mode="o_random", neighbor_visible_num=1, **_OBST), 21, "hover"),      # first minimum
+    "feat2_downwash_k3": (dict(num_agents=3, use_downwash=True, neighbor_visible_num=1), 21, "uniform"),                # packed
+    "feat3_obst_downwash_k3": (dict(num_agents=3, quads_mode="mix", use_downwash=True, neighbor_visible_num=2, **_OBST), 21, "hover"),
+    "feat6_mix_downwash_k3": (dict(num_agents=3, quads_mode="mix", use_downwash=True, neighbor_visible_num=1), 21, "hover"),  # packed
+    "feat0_k16_v12": (dict(num_agents=16, neighbor_visible_num=12), 13, "uniform"),                          # all-pairs: 36 >= 30
+    "feat1_obst_k13_v10": (dict(num_agents=13, quads_mode="o_random", neighbor_visible_num=10, **_OBST), 13, "hover"),  # all-pairs: 30 >= 30
+    "feat2_downwash_k12_vall": (dict(num_agents=12, use_downwash=True, neighbor_visible_num=-1), 13, "uniform"),         # all
+    "feat3_obst_downwash_k13": (dict(num_agents=13, quads_mode="mix", use_downwash=True, **_OBST), 13, "hover"),        # first minimum
+    "feat6_mix_downwash_k12": (dict(num_agents=12, quads_mode="mix", use_downwash=True), 13, "hover"),                 # first minimum
+    "feat0_k29_v24": (dict(num_agents=29, neighbor_visible_num=24), 9, "uniform"),                           # all-pairs: 72 >= 62
+    "feat1_obst_k27": (dict(num_agents=27, quads_mode="o_random", **_OBST), 9, "hover"),                               # first minimum
+    "feat2_downwash_k27_vall": (dict(num_agents=27, use_downwash=True, neighbor_visible_num=-1), 9, "uniform"),         # all
+    "feat3_obst_downwash_k29_v22": (dict(num_agents=29, quads_mode="mix", use_downwash=True, neighbor_visible_num=22, **_OBST), 9,
+                                    "hover"),                                                                          # all-pairs: 66 >= 62
+    "feat6_mix_downwash_k27": (dict(num_agents=27, quads_mode="mix", use_downwash=True), 9, "hover"),                  # first minimum
+    "feat1_obst_k4_v2": (dict(num_agents=4, quads_mode="o_random", neighbor_visible_num=2, **_OBST), 21, "hover"),     # packed: 6 >= 6
+    "feat1_obst_k7_v5": (dict(num_agents=7, quads_mode="o_random", neighbor_visible_num=5, **_OBST), 11, "hover"),     # packed: 15 >= 14
+    "feat3_obst_downwash_k6_vall": (dict(num_agents=6, quads_mode="mix", use_downwash=True, neighbor_visible_num=-1, **_OBST), 11,
+                                    "hover"),                                                                          # all
+    "feat1_obst_k12_vall": (dict(num_agents=12, quads_mode="o_random", neighbor_visible_num=-1, **_OBST), 13, "hover"),  # all
+    "feat1_obst_k29_vall": (dict(num_agents=29, quads_mode="o_random", neighbor_visible_num=-1, **_OBST), 9, "hover"),   # all
+}
+CONFIGS.update({name: dict(num_envs=n, ep_time=0.3, **kw) for name, (kw, n, _) in WIDTH_CELLS.items()})
+
 
 def make_pair(name, seed=3):
     cfg = QuadSimConfig(seed=seed, **CONFIGS[name])
@@ -132,28 +170,52 @@ def test_philox_contract_bit_exact():
             np.testing.assert_allclose([f[2 + 2 * p], f[3 + 2 * p]], [rad * np.cos(ang), rad * np.sin(ang)], atol=2e-6)
 
 
+def check_reset(cfg, obs, st, oracles, envs):
+    """The reset envs `envs` of the kernel's observations `obs` and state `st` (host arrays) against their oracles, just reset."""
+    K = cfg.num_agents
+    rows = (envs[:, None] * K + np.arange(K)[None, :]).reshape(-1)
+    ref = np.concatenate([oracles[e].reset() for e in envs])
+    os_ = oracle_state([oracles[e] for e in envs])
+    # a yaw-rejection tie (cos >= 0.5 in fp32 vs fp64) may flip one drone's accepted attempt: allow a handful
+    bad = np.abs(st["rot"][rows] - os_["rot"]).max(axis=1) > 1e-5
+    for i in np.unique(np.flatnonzero(bad) // K):
+        proved, m = tie_proven(oracles[envs[i]], ("yaw",))
+        assert proved, f"env {envs[i]}: spawn yaw differs without a rejection tie (margins in fp32 ulps: {m})"
+    ok = ~bad
+    np.testing.assert_allclose(st["pos"][rows][ok], os_["pos"][ok], atol=2e-6)
+    np.testing.assert_allclose(st["goal"][rows], os_["goal"], atol=1e-6)
+    okrows = np.repeat(ok.reshape(len(envs), K).all(axis=1), K)
+    np.testing.assert_allclose(obs[rows][okrows], ref[okrows], atol=2e-5)
+    if cfg.use_obstacles:
+        for e in envs:
+            np.testing.assert_allclose(st["obst_xy"][e, :cfg.num_obstacles], oracles[e].get_state()["obst_xy"], atol=1e-6)
+    assert (st["tick"][envs] == 0).all()
+
+
 @pytest.mark.parametrize("name", list(CONFIGS))
 def test_reset_parity(name):
+    """A full reset, then a masked one: the envs it names (one of them in the partial last warp-tile) against a second oracle
+    reset, the others' observation rows and state bitwise unchanged."""
     cfg, sim, oracles = make_pair(name)
+    N, K = cfg.num_envs, cfg.num_agents
     obs = sim.reset().cpu().numpy()
-    ref = np.concatenate([o.reset() for o in oracles])
-    assert obs.shape == ref.shape == (cfg.num_envs * cfg.num_agents, cfg.obs_dim)
+    assert obs.shape == (N * K, cfg.obs_dim)
     st = {k: v.cpu().numpy() for k, v in sim.get_state().items()}
-    os_ = oracle_state(oracles)
-    # a yaw-rejection tie (cos >= 0.5 in fp32 vs fp64) may flip one drone's accepted attempt: allow a handful
-    bad = np.abs(st["rot"] - os_["rot"]).max(axis=1) > 1e-5
-    for e in np.unique(np.flatnonzero(bad) // cfg.num_agents):
-        proved, m = tie_proven(oracles[e], ("yaw",))
-        assert proved, f"env {e}: spawn yaw differs without a rejection tie (margins in fp32 ulps: {m})"
-    ok = ~bad
-    np.testing.assert_allclose(st["pos"][ok], os_["pos"][ok], atol=2e-6)
-    np.testing.assert_allclose(st["goal"], os_["goal"], atol=1e-6)
-    okrows = np.repeat(ok.reshape(cfg.num_envs, cfg.num_agents).all(axis=1), cfg.num_agents)
-    np.testing.assert_allclose(obs[okrows], ref[okrows], atol=2e-5)
-    if cfg.use_obstacles:
-        for e, o in enumerate(oracles):
-            np.testing.assert_allclose(st["obst_xy"][e, :cfg.num_obstacles], o.get_state()["obst_xy"], atol=1e-6)
-    assert (st["tick"] == 0).all() and (st["step_ctr"] == 1).all()
+    check_reset(cfg, obs, st, oracles, np.arange(N))
+    assert (st["step_ctr"] == 1).all()
+
+    mask = np.zeros(N, bool)
+    mask[[1, N // 2, N - 1]] = True
+    obs2 = sim.reset(torch.from_numpy(mask)).cpu().numpy()
+    st2 = {k: v.cpu().numpy() for k, v in sim.get_state().items()}
+    check_reset(cfg, obs2, st2, oracles, np.flatnonzero(mask))     # the oracles' second reset draws from the same counter
+    keep_rows = np.repeat(~mask, K)
+    assert np.array_equal(obs2[keep_rows].view(np.int32), obs[keep_rows].view(np.int32)), "masked-out observation rows changed"
+    for k, v in st.items():
+        if k == "step_ctr":                                         # the handle's launch counter, reported per env
+            continue
+        sel = keep_rows if v.shape[0] == N * K else ~mask
+        assert np.array_equal(st2[k][sel].view(np.uint8), v[sel].view(np.uint8)), f"state {k} of a masked-out env changed"
 
 
 def run_parity(name, cfg, sim, oracles, kind, steps, hook=None, check_records=True, record_envs=None):
@@ -506,14 +568,18 @@ FEATS = {
     "feat6_scenarios_downwash": dict(num_agents=8, quads_mode="mix", use_downwash=True),
     "k32": dict(num_agents=32),
     "k3": dict(num_agents=3, neighbor_visible_num=1),
+    "fork_k4": dict(env_mode="fork", num_agents=4, capture_radius=2.6),
+    "fork_k12_sangle_v5": dict(env_mode="fork", num_agents=12, capture_radius=2.2, obs_repr="cdist_cdistdot_dist_distdot_sangle_angledot",
+                               neighbor_obs_type="dist_sangle", neighbor_visible_num=5),
 }
 
 
 @pytest.mark.parametrize("name", list(FEATS))
 def test_block_64_and_128_are_bitwise_identical(name, monkeypatch):
     """The launch shape is not part of the result: 64- and 128-thread blocks (the small-batch and the large-batch default) produce
-    the same bits in every feature variant of the step kernel, including partial last blocks and auto-resets."""
-    cfg = QuadSimConfig(seed=23, num_envs=301, ep_time=0.15, **FEATS[name])
+    the same bits in every feature variant of the step kernel and in the fork kernel, including partial last blocks and auto-resets."""
+    make = QuadSimConfig.fork_default if FEATS[name].get("env_mode") == "fork" else QuadSimConfig
+    cfg = make(seed=23, num_envs=301, ep_time=0.15, **FEATS[name])
     sims = []
     for blk in ("64", "128"):
         monkeypatch.setenv("QS_BLOCK", blk)
@@ -524,7 +590,8 @@ def test_block_64_and_128_are_bitwise_identical(name, monkeypatch):
     rs = np.random.RandomState(6)
     n_done = 0
     for s in range(40):
-        a = torch.from_numpy(action_batch(rs, cfg.num_envs * cfg.num_agents, "uniform" if s % 2 else "hover")).cuda()
+        a = action_batch(rs, cfg.num_envs * cfg.num_agents, "uniform" if s % 2 else "hover")
+        a = torch.from_numpy(np.ascontiguousarray(a[:, :a_sim.A])).cuda()
         o1, r1, d1 = a_sim.step(a)
         o2, r2, d2 = b_sim.step(a)
         assert torch.equal(o1, o2) and torch.equal(r1, r2) and torch.equal(d1, d2), f"step {s}"

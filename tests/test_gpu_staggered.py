@@ -22,7 +22,7 @@ if not torch.cuda.is_available():
 
 from oracle import OracleEnv  # noqa: E402
 from quad_swarm_rl_stable_baselines3_b200.config import QuadSimConfig  # noqa: E402
-from test_gpu_parity import SubsetSim, _sim, run_parity  # noqa: E402
+from test_gpu_parity import WIDTH_CELLS, SubsetSim, _sim, run_parity  # noqa: E402
 
 OBST = dict(use_obstacles=True, obs_repr="xyz_vxyz_R_omega_floor")
 HOT_CAP = 128                       # listed warp-tiles per step (qs_create: e->hot_cap)
@@ -54,7 +54,8 @@ class CheckedSim(SubsetSim):
       2. episode records of envs that did not end are bitwise unchanged, those of envs that ended advanced their sequence number
          by one; reset_success (filled with a canary byte before the step) reads 0 for envs that ended (upstream reset() reports
          no success) and the canary elsewhere;
-      3. done == (tick before the step + 1 > ep_len), the only way an upstream episode ends short of a non-finite state.
+      3. done == (tick before the step + 1 > ep_len), the only way an upstream episode ends short of a non-finite state
+         (`ended()`; the fork env overrides it with its own rule).
     It counts the mixed units (some but not all valid envs of a warp-tile end on a step) among the compared envs, and per step the
     warp-tiles of the whole batch with an ending env (what the reset-first scheduling lists).
 
@@ -83,6 +84,15 @@ class CheckedSim(SubsetSim):
     def comparable(self):
         return self._comparable
 
+    def ended(self, tick0, rec1):
+        """The envs that ended in the step just taken [N] bool, after checking the done mask and reset_success of the ended envs
+        against the rule that ends an episode."""
+        sim, N, K = self.sim, self.sim.N, self.K
+        end = tick0 + 1 > self.ep_len
+        assert torch.equal(sim.done.view(N, K), end[:, None].expand(N, K)), "done differs from the episode clocks"
+        assert bool((sim.reset_success[end] == 0).all()), "reset_success"
+        return end
+
     def step(self, a_small):
         sim, N, K = self.sim, self.sim.N, self.K
         tick0 = sim.get_state(("tick",))["tick"]
@@ -90,14 +100,13 @@ class CheckedSim(SubsetSim):
         sim.terminal_obs.fill_(float("nan"))
         sim.reset_success.fill_(self.CANARY)
         out = super().step(a_small)
-        end = tick0 + 1 > self.ep_len
-        assert torch.equal(sim.done.view(N, K), end[:, None].expand(N, K)), "done differs from the episode clocks"
+        rec1 = sim.episode_records()
+        end = self.ended(tick0, rec1)
         keep = ~end
         keep_rows = keep.repeat_interleave(K)
         assert bool(torch.isnan(sim.terminal_obs[keep_rows]).all()), "terminal_obs written for an env that did not end"
         assert not bool(torch.isnan(sim.terminal_obs[~keep_rows]).any()), "terminal_obs incomplete for an env that ended"
-        assert bool((sim.reset_success[keep] == self.CANARY).all()) and bool((sim.reset_success[end] == 0).all()), "reset_success"
-        rec1 = sim.episode_records()
+        assert bool((sim.reset_success[keep] == self.CANARY).all()), "reset_success written for an env that did not end"
         assert torch.equal(rec1["env"][keep], rec0["env"][keep]), "episode record of an env that did not end changed"
         assert torch.equal(rec1["agent"][keep_rows].view(torch.int32), rec0["agent"][keep_rows].view(torch.int32)), \
             "per-drone episode record of an env that did not end changed"
@@ -159,6 +168,7 @@ STAGGER = {
     "feat0_k32": (dict(num_agents=32), 9, "uniform"),
     # ... and on its sequential fallback: one drone's tile row is 28 floats < obst_scratch_floats(12, 1) = 84
     "feat1_obst_k1_fallback": (dict(num_agents=1, quads_mode="mix", neighbor_obs_type="none", neighbor_visible_num=0, **OBST), 137, "hover"),
+    **WIDTH_CELLS,                      # every feature variant at the widths 2, 4, 16 and 32 (test_gpu_parity.py)
 }
 
 
