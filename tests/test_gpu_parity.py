@@ -13,7 +13,7 @@ torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 
 from oracle import OracleEnv, philox  # noqa: E402
-from quad_swarm_rl_stable_baselines3_b200.config import QuadSimConfig  # noqa: E402
+from quad_swarm_rl_stable_baselines3_b200.config import OBS_REPR_DIM, QuadSimConfig  # noqa: E402
 
 REL_TOL = 1e-5          # north_star tolerance on pos/vel/rot/omega after one step
 PHYS = ("pos", "vel", "rot", "omega", "rot_damp", "cmds_damp", "ou")
@@ -218,10 +218,11 @@ def test_reset_parity(name):
         assert np.array_equal(st2[k][sel].view(np.uint8), v[sel].view(np.uint8)), f"state {k} of a masked-out env changed"
 
 
-def run_parity(name, cfg, sim, oracles, kind, steps, hook=None, check_records=True, record_envs=None):
+def run_parity(name, cfg, sim, oracles, kind, steps, hook=None, check_records=True, record_envs=None, goal_atol=None):
     """Every step: copy the GPU state into the oracle, step both with the same actions, compare everything.
     `record_envs`, if given, is called after each step and returns a bool mask [N]: the envs whose just-finished episode record
-    is compared (default: every env that finished)."""
+    is compared (default: every env that finished).  `goal_atol`, if given, is called with the state before and after the step
+    and returns the goal tolerance per drone [N*K] (default 3e-6 for every drone)."""
     K, N = cfg.num_agents, cfg.num_envs
     rs = np.random.RandomState(11)
     worst = dict(pos=0.0, vel=0.0, rot=0.0, omega=0.0, obs=0.0, rew=0.0)
@@ -301,12 +302,30 @@ def run_parity(name, cfg, sim, oracles, kind, steps, hook=None, check_records=Tr
         worst["omega"] = max(worst["omega"], relerr(st["omega"][rows], os_["omega"][rows], 1.0))
         if "scenario" in st:
             ref_rows = np.stack([o.get_scenario() for o in oracles])
-            np.testing.assert_allclose(st["goal"][rows], os_["goal"][rows], atol=3e-6, err_msg=f"step {s}: goals")
+            gtol = 3e-6 if goal_atol is None else goal_atol(pre, st)[rows][:, None]
+            gbad = ~(np.abs(st["goal"][rows] - os_["goal"][rows]) <= gtol + 1e-7 * np.abs(os_["goal"][rows]))   # assert_allclose's rule
+            assert not gbad.any(), f"step {s}: goals of drones {np.flatnonzero(rows)[gbad.any(axis=1)]} differ by more than the tolerance"
             assert np.array_equal(st["scenario"][env_ok][:, [0, 1, 9, 10]], ref_rows[env_ok][:, [0, 1, 9, 10]]), f"step {s}: scenario ids / timers"
             np.testing.assert_allclose(st["scenario"][env_ok], ref_rows[env_ok], atol=3e-6, err_msg=f"step {s}: scenario rows")
             worst["goal"] = max(worst.get("goal", 0.0), float(np.abs(st["goal"][rows] - os_["goal"][rows]).max()))
             cnt["goal_moves"] = cnt.get("goal_moves", 0) + int((np.abs(st["goal"] - pre["goal"]).max(axis=1) > 0).reshape(N, K).any(axis=1).sum())
-        worst["obs"] = max(worst["obs"], relerr(obs[rows], ref_obs[rows], 1.0))
+        # neighbour rows chosen by rank (V < K - 1): a different choice or order is a discrete disagreement, accepted for an env
+        # only when the oracle's ranking had two candidates within the rank bound; that env's neighbour columns are then skipped
+        obs_c = obs
+        if cfg.neighbor_obs_type == "pos_vel" and 0 < cfg.visible < K - 1:
+            nb = slice(OBS_REPR_DIM[cfg.obs_repr], OBS_REPR_DIM[cfg.obs_repr] + 6 * cfg.visible)
+            d_nb = np.abs(obs[:, nb] - ref_obs[:, nb]) / np.maximum(np.abs(ref_obs[:, nb]), 1.0)
+            for e in np.flatnonzero(((d_nb > 5e-5).any(axis=1).reshape(N, K).any(axis=1)) & env_ok):
+                proved, m = tie_proven(oracles[e], ("rank",))
+                cnt["rank_ties"] = cnt.get("rank_ties", 0) + int(proved)
+                if not proved:
+                    cnt["unproven"] += 1
+                    print(f"[{name}] step {s}: neighbour rows of env {e} differ and NO ranking was near a tie (fp32 ulps): {m}")
+                    continue
+                if obs_c is obs:
+                    obs_c = obs.copy()
+                obs_c[e * K:(e + 1) * K, nb] = ref_obs[e * K:(e + 1) * K, nb]
+        worst["obs"] = max(worst["obs"], relerr(obs_c[rows], ref_obs[rows], 1.0))
         worst["rew"] = max(worst["rew"], float(np.abs(rew[rows] - ref_rew[rows]).max()))
         drows = rows & done
         if drows.any():

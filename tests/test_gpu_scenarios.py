@@ -12,7 +12,25 @@ from oracle import OracleEnv  # noqa: E402
 from quad_swarm_rl_stable_baselines3_b200.config import QuadSimConfig  # noqa: E402
 from test_gpu_parity import _sim, oracle_state, run_parity  # noqa: E402
 
-SC_CTL, SC_SIZE, SC_HIGHEST, SC_INCREASE = 9, 2, 4, 10
+SC_FORMATION, SC_SIZE, SC_HIGHEST, SC_LOWEST, SC_CTL, SC_INCREASE = 1, 2, 4, 5, 9, 10
+
+
+def fast_timers(row):
+    """control_step_for_sec is 400..599 control steps in the reference; shorten it to 5 + e % 7 so that the goal-changing branch
+    runs many times inside a short test, every env with its own period.  Rewrites the [N, QS_SC_COUNT] rows in place and returns
+    whether any changed (after a reset the row holds a fresh reference timer again)."""
+    ctl = row[:, SC_CTL]
+    slow = ctl > 50
+    if slow.any():
+        row[:, SC_CTL] = torch.where(slow, 5.0 + (torch.arange(row.shape[0], device=row.device) % 7).float(), ctl)
+    return bool(slow.any())
+
+
+def near_turning_points(row):
+    """dynamic_formations: put the even envs just below / above the turning points of the breathing formation (in place)."""
+    half = torch.arange(row.shape[0], device=row.device) % 2 == 0
+    sign = torch.where(row[:, SC_INCREASE] > 0, 1.0, -1.0)
+    row[:, SC_SIZE] = torch.where(half, sign * (row[:, SC_HIGHEST] - 0.004), row[:, SC_SIZE])
 
 SCENARIO_CONFIGS = {
     # name: (config kwargs, steps, timer override: goals change every few steps instead of every 4-6 s)
@@ -61,20 +79,9 @@ def test_scenario_parity(name):
 
     def hook(s):
         row = sim.get_state(("scenario",))["scenario"]
-        changed = False
-        if fast_timer:
-            # control_step_for_sec is 400..599 control steps in the reference; shorten it so the goal-changing branch runs
-            # many times inside a short test (every env gets its own period)
-            ctl = row[:, SC_CTL]
-            slow = ctl > 50
-            if slow.any():
-                row[:, SC_CTL] = torch.where(slow, 5.0 + (torch.arange(N, device=row.device) % 7).float(), ctl)
-                changed = True
+        changed = fast_timer and fast_timers(row)
         if name.startswith("dynform") and s % 25 == 3:
-            # put half of the envs just below / above the turning points of the breathing formation
-            half = torch.arange(N, device=row.device) % 2 == 0
-            sign = torch.where(row[:, SC_INCREASE] > 0, 1.0, -1.0)
-            row[:, SC_SIZE] = torch.where(half, sign * (row[:, SC_HIGHEST] - 0.004), row[:, SC_SIZE])
+            near_turning_points(row)
             changed = True
         if changed:
             sim.set_state(scenario=row)
