@@ -17,9 +17,11 @@
  *
  * Architecture built: self encoder S -> 256 -> 256, deep-sets neighbour encoder ('mean_embed') W -> 256 -> 256 averaged over V neighbours,
  * optional obstacle encoder O -> 256 -> 256, feed-forward [self | neighbour | obstacle] (512 or 768) -> 512, all tanh; heads 512 -> A (actor) and 512 -> 1 (critic).
+ * qp_create_encoder(QP_NBR_MLP) builds the 'mlp' neighbour encoder instead (QuadNeighborhoodEncoderMlp, quad_multi_model.py:104-122: the
+ * W * V neighbour columns as one vector -> 256 -> 256 -> 256), for W * V <= 40 and without the obstacle encoder.
  * bf16 operands, fp32 accumulation (tcgen05 tensor cores); biases, heads and outputs fp32.  Sampling and log-probabilities stay with the
- * caller (state-independent log-std diagonal Gaussian, ActorCriticPolicyCustom.py:312).  Not built: the 'attention' and 'mlp' neighbour
- * encoders, widths other than 256.
+ * caller (state-independent log-std diagonal Gaussian, ActorCriticPolicyCustom.py:312).  Not built: the 'attention' neighbour encoder,
+ * 'mlp' with the obstacle encoder or with W * V > 40, widths other than 256.
  *
  * All pointers are CUDA device addresses unless stated; `stream` is a cudaStream_t passed as void*.  Calls return 0 or a negative
  * qp_status; qp_last_error() gives a message.  A handle is bound to one device and is not thread-safe.
@@ -40,6 +42,9 @@ extern "C" {
 
 typedef enum { QP_OK = 0, QP_ERR_NULL = -1, QP_ERR_BAD_CONFIG = -2, QP_ERR_CUDA = -3 } qp_status;
 
+/* neighbour encoder of a handle (qp_create_encoder) */
+enum { QP_NBR_DEEPSETS = 0, QP_NBR_MLP = 1 };
+
 typedef struct {
     int32_t api_version; /* QP_API_VERSION */
     int32_t self_dim;    /* S: 18 / 19 / 24 (quad_utils.py:30-38); S <= 24 */
@@ -54,20 +59,24 @@ typedef struct {
 typedef struct {
     const float *self_w1, *self_b1; /* [256, S], [256] */
     const float *self_w2, *self_b2; /* [256, 256], [256] */
-    const float *nbr_w1, *nbr_b1;   /* [256, W], [256]   (ignored when num_nbr == 0) */
+    const float *nbr_w1, *nbr_b1;   /* [256, W] ([256, W * V] for QP_NBR_MLP), [256]   (ignored when num_nbr == 0) */
     const float *nbr_w2, *nbr_b2;   /* [256, 256], [256] */
     const float *ff_w, *ff_b;       /* [512, 512] ([512, 768] when obst_dim > 0), [512]; input = [self | neighbour | obstacle encoder];
                                        without neighbours (num_nbr == 0) the neighbour block must be zeros */
     const float *head_w, *head_b;   /* actor: [A, 512], [A]; critic: [1, 512], [1] */
     const float *obst_w1, *obst_b1; /* [256, O], [256]   (since version 2; read only when obst_dim > 0) */
     const float *obst_w2, *obst_b2; /* [256, 256], [256] */
+    const float *nbr_w3, *nbr_b3;   /* [256, 256], [256]   (read only by QP_NBR_MLP handles: the encoder's third layer) */
 } qp_tower_weights;
 
 typedef struct qp_policy qp_policy;
 
 size_t qp_config_size(void);
 const char *qp_last_error(const qp_policy *p);
-int qp_create(const qp_config *cfg, int device, qp_policy **out);
+int qp_create(const qp_config *cfg, int device, qp_policy **out);   /* = qp_create_encoder(cfg, QP_NBR_DEEPSETS, device, out) */
+/* a handle with the given neighbour encoder.  QP_NBR_MLP requires num_nbr >= 1, nbr_dim * num_nbr <= 40 and obst_dim == 0, else
+ * QP_ERR_BAD_CONFIG; so does an unknown nbr_encoder. */
+int qp_create_encoder(const qp_config *cfg, int nbr_encoder, int device, qp_policy **out);
 int qp_destroy(qp_policy *p);
 int64_t qp_launch_count(const qp_policy *p);
 

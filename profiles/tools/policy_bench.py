@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """Fused tcgen05 policy forward vs the torch module it replaces, one JSON line per case:
   * cfg2: the rollout batch of BASELINE configs[4] (65536 envs x 8 quads = 524288 observation rows, obs 54: S 18, W 6, V 6);
-  * cfg3_obstacles: the same number of rows of the obstacle scenario's observation (BASELINE configs[2]: obs 40 = S 19, W 6, V 2, O 9).
+  * cfg3_obstacles: the same number of rows of the obstacle scenario's observation (BASELINE configs[2]: obs 40 = S 19, W 6, V 2, O 9);
+  * cfg2_mlp: cfg2's rows with the MLP neighbour encoder (neighbor_encoder="mlp": the 36 neighbour columns as one vector -> 256 -> 256 -> 256).
 Device time per forward (CUDA events on the launching stream, median of `reps` after warm-up), achieved dense TFLOP/s (and, when
 MEASURED_PEAKS.json is present, the fraction of its sustained bf16 peak); the card's name and power limit go into every line.
 python policy_bench.py [rows] [reps] [case ...]"""
@@ -20,10 +21,11 @@ from quad_swarm_rl_stable_baselines3_b200.ppo import QuadActorCritic  # noqa: E4
 
 rows = int(sys.argv[1]) if len(sys.argv) > 1 else 524288
 reps = int(sys.argv[2]) if len(sys.argv) > 2 else 20
-CASES = {
-    "cfg2": lambda: QuadSimConfig(num_envs=8, num_agents=8),
-    "cfg3_obstacles": lambda: QuadSimConfig(num_envs=8, num_agents=8, quads_mode="mix", use_obstacles=True, obs_repr="xyz_vxyz_R_omega_floor",
-                                            neighbor_visible_num=2),
+CASES = {   # name: (config, neighbour encoder)
+    "cfg2": (lambda: QuadSimConfig(num_envs=8, num_agents=8), "mean_embed"),
+    "cfg3_obstacles": (lambda: QuadSimConfig(num_envs=8, num_agents=8, quads_mode="mix", use_obstacles=True, obs_repr="xyz_vxyz_R_omega_floor",
+                                             neighbor_visible_num=2), "mean_embed"),
+    "cfg2_mlp": (lambda: QuadSimConfig(num_envs=8, num_agents=8), "mlp"),
 }
 cases = sys.argv[3:] or list(CASES)
 dev = torch.device("cuda:0")
@@ -49,15 +51,18 @@ def timed(fn):
 
 
 for case in cases:
-    cfg = CASES[case]()
+    make, encoder = CASES[case]
+    cfg = make()
     torch.manual_seed(0)
-    pol = QuadActorCritic(cfg).to(dev)
+    pol = QuadActorCritic(cfg, neighbor_encoder=encoder).to(dev)
     fp = FusedPolicy(pol, dev)
     obs = torch.randn(rows, cfg.obs_dim, device=dev)
     S, W, V, O, A = fp.S, fp.W, fp.V, fp.O, fp.A
     ff_in = 256 * (1 + (V > 0) + (O > 0))
-    # multiply-adds per row and tower: self encoder, V neighbour passes, obstacle encoder, feed-forward; heads A (actor) and 1 (critic)
-    flop_row = 2 * 2 * (S * 256 + 256 * 256 + V * (W * 256 + 256 * 256) + (O * 256 + 256 * 256 if O else 0) + ff_in * 512 + 512 * (A + 1) / 2)
+    # multiply-adds per row and tower: self encoder, V neighbour passes (MLP: one W V -> 256 -> 256 -> 256 pass), obstacle encoder, feed-forward;
+    # heads A (actor) and 1 (critic)
+    nbr = W * V * 256 + 2 * 256 * 256 if encoder == "mlp" else V * (W * 256 + 256 * 256)
+    flop_row = 2 * 2 * (S * 256 + 256 * 256 + nbr + (O * 256 + 256 * 256 if O else 0) + ff_in * 512 + 512 * (A + 1) / 2)
 
     def eager_fp32():
         with torch.no_grad():
@@ -67,7 +72,8 @@ for case in cases:
         with torch.no_grad(), torch.autocast("cuda", dtype=torch.bfloat16):
             return pol.action_net(pol.actor(obs)), pol.value(obs)
 
-    policy = f"2 towers x (self {S}-256-256" + (f", deep-sets {W}-256-256 x {V}" if V else "") + (f", obstacles {O}-256-256" if O else "") + \
+    nbr_desc = (f", MLP neighbours {W * V}-256-256-256" if encoder == "mlp" else f", deep-sets {W}-256-256 x {V}") if V else ""
+    policy = f"2 towers x (self {S}-256-256" + nbr_desc + (f", obstacles {O}-256-256" if O else "") + \
         f", ff {ff_in}-512, heads {A}/1)"
     out = {"case": case, "rows": rows, "obs_dim": cfg.obs_dim, "flop_per_row": flop_row, "policy": policy, "card": card}
     for name, fn in (("fused_tcgen05", lambda: fp.forward(obs)), ("torch_bf16_autocast", eager_bf16), ("torch_fp32", eager_fp32)):

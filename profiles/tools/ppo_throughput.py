@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """BASELINE.json configs[4] "with PPO update": rollout (policy inference + simulator) and update throughput of the device
 PPO loop.  Single GPU: python ppo_throughput.py [envs] [n_steps] [config] [rollout]; N GPUs: torchrun --nproc-per-node N ppo_throughput.py ...
-config: "cfg2" (default: 8 quads, deep-sets neighbours) or "cfg3" (the obstacle scenario of configs[2]: mix, obstacles, S 19, V 2);
+config: "cfg2" (default: 8 quads, deep-sets neighbours), "cfg2_mlp" (cfg2 with the MLP neighbour encoder) or "cfg3" (the obstacle
+scenario of configs[2]: mix, obstacles, S 19, V 2);
 rollout: "fused" (default: the tcgen05 forward where the architecture is covered) or "torch" (PPOConfig.fused_rollout = False)."""
 import json
 import os
@@ -20,8 +21,8 @@ envs = int(sys.argv[1]) if len(sys.argv) > 1 else 65536
 n_steps = int(sys.argv[2]) if len(sys.argv) > 2 else 32
 config = sys.argv[3] if len(sys.argv) > 3 else "cfg2"
 rollout = sys.argv[4] if len(sys.argv) > 4 else "fused"
-if config not in ("cfg2", "cfg3") or rollout not in ("fused", "torch"):
-    raise SystemExit("config must be cfg2 or cfg3, rollout fused or torch")
+if config not in ("cfg2", "cfg2_mlp", "cfg3") or rollout not in ("fused", "torch"):
+    raise SystemExit("config must be cfg2, cfg2_mlp or cfg3, rollout fused or torch")
 rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
 torch.cuda.set_device(local)
 dev = torch.device("cuda", local)
@@ -31,7 +32,8 @@ extra = dict(quads_mode="mix", use_obstacles=True, obs_repr="xyz_vxyz_R_omega_fl
 cfg = QuadSimConfig(num_envs=envs, num_agents=8, seed=0, env_id_offset=rank * envs, **extra)
 sim = QuadSwarmSim(cfg, device=dev)
 sim.want_terminal_obs = False
-ppo = DevicePPO(sim, cfg, PPOConfig(n_steps=n_steps, batch_size=65536, n_epochs=1, autocast_bf16=True, fused_rollout=rollout == "fused"))
+ppo = DevicePPO(sim, cfg, PPOConfig(n_steps=n_steps, batch_size=65536, n_epochs=1, autocast_bf16=True, fused_rollout=rollout == "fused",
+                                    neighbor_encoder="mlp" if config == "cfg2_mlp" else "mean_embed"))
 ppo.learn(1)                                                    # warm-up (cuBLAS heuristics, allocator)
 hist = ppo.learn(2)
 n = envs * 8
@@ -43,7 +45,8 @@ if world > 1:
 if rank == 0:
     roll, upd = float(t[0]), float(t[1])
     enc = ppo.policy.actor
-    arch = f"self {enc.S}-256-256" + (f", deep-sets neighbours {enc.W}x{enc.V}-256-256" if enc.V else "") + (f", obstacles {enc.O}-256-256" if enc.O else "")
+    nbr = f", MLP neighbours {enc.W * enc.V}-256-256-256" if enc.kind == "mlp" else f", deep-sets neighbours {enc.W}x{enc.V}-256-256" if enc.V else ""
+    arch = f"self {enc.S}-256-256" + nbr + (f", obstacles {enc.O}-256-256" if enc.O else "")
     print(json.dumps({"config": config, "rollout_forward": "tcgen05 kernel" if ppo.fused is not None else "torch bf16 autocast",
                       "n_gpus": world, "envs_per_gpu": envs, "agents": 8, "n_steps": n_steps,
                       "rollout_drone_steps_per_s": world * n * n_steps / roll, "update_samples_per_s": world * n * n_steps / upd,

@@ -25,7 +25,7 @@ EXPORTS = ("qs_config_size", "qs_stats_size", "qs_api_version", "qs_last_error",
            "qs_reset_host", "qs_step_host", "qs_get_state", "qs_set_state", "qs_set_param", "qs_episode_stats",
            "qs_episode_records", "qs_episode_records_host", "qs_set_reward_info", "qs_snapshot_size", "qs_snapshot", "qs_restore")
 # every symbol include/quadpolicy.h declares (fused policy forward, csrc/policy_kernels.cu)
-POLICY_EXPORTS = ("qp_config_size", "qp_last_error", "qp_create", "qp_destroy", "qp_launch_count", "qp_set_weights", "qp_forward", "qp_gae", "qp_bias_tanh", "qp_bias_tanh_backward", "qp_bias_tanh_mean", "qp_bias_tanh_mean_backward", "qp_bias_tanh_backward_first", "qp_bias_tanh_backward_first_workspace")
+POLICY_EXPORTS = ("qp_config_size", "qp_last_error", "qp_create", "qp_create_encoder", "qp_destroy", "qp_launch_count", "qp_set_weights", "qp_forward", "qp_gae", "qp_bias_tanh", "qp_bias_tanh_backward", "qp_bias_tanh_mean", "qp_bias_tanh_mean_backward", "qp_bias_tanh_backward_first", "qp_bias_tanh_backward_first_workspace")
 
 
 KG_VALUES = (1, 2, 4, 8, 16, 32)
@@ -115,6 +115,7 @@ def lib():
     L.qp_last_error.restype = C.c_char_p
     L.qp_last_error.argtypes = [vp]
     L.qp_create.argtypes = [vp, i32, C.POINTER(vp)]
+    L.qp_create_encoder.argtypes = [vp, i32, i32, C.POINTER(vp)]
     L.qp_destroy.argtypes = [vp]
     L.qp_launch_count.argtypes = [vp]
     L.qp_launch_count.restype = C.c_int64

@@ -28,6 +28,9 @@
 //   so the self part is written once per tile and each neighbour pass rewrites one 16-byte chunk per row.
 //   Obstacle encoder (the OB instantiation, qp_config.obst_dim > 0; quad_multi_model.py's obstacle MLP, O -> 256 -> 256): runs after the self
 //   encoder on stream 1's x tile, whose self slots then hold the O obstacle columns; the feed-forward (K = 768) has one accumulator, ACC0.
+//   MLP neighbour encoder (the MLP instantiation, qp_create_encoder(QP_NBR_MLP); quad_multi_model.py's QuadNeighborhoodEncoderMlp, the W V
+//   neighbour columns as one vector -> 256 -> 256 -> 256): no per-neighbour passes; its three layers stream through the ring after the self
+//   encoder.  Layer 1 reads neighbour inputs 0-31 from stream 1's x tile and inputs 32-39 from the neighbour slots of stream 0's, so W V <= 40.
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <stdint.h>
@@ -63,7 +66,15 @@ constexpr int STREAM_CHUNKS = STREAM_BYTES / CHUNK;                  // 41
 constexpr int MAX_OBST = SELF_PAD;
 constexpr int OBST_BYTES = 2 * CHUNK1 + 8 * CHUNK + 16 * CHUNK;
 constexpr int OBST_CHUNKS = OBST_BYTES / CHUNK;                      // 25
-constexpr size_t tower_img_bytes(int obst_dim) { return (size_t)(RES_BYTES + STREAM_BYTES + (obst_dim > 0 ? OBST_BYTES : 0)); }   // 819200 / 1228800
+// MLP neighbour encoder (compile-time variant): streamed per tile on top, after the self encoder: layer 1 (two K = 32 images per half, stream 1's
+// x tile and stream 0's neighbour slots), layers 2 and 3; the image has no resident block
+constexpr int MAX_MLP_IN = 32 + NBR_PAD;
+constexpr int MLP_BYTES = 4 * CHUNK1 + 16 * CHUNK;
+constexpr int MLP_CHUNKS = MLP_BYTES / CHUNK;                        // 18
+constexpr size_t tower_img_bytes(int obst_dim, bool mlp)             // 819200 / 1228800 / 966656 (MLP)
+{
+    return mlp ? (size_t)(STREAM_BYTES + MLP_BYTES) : (size_t)(RES_BYTES + STREAM_BYTES + (obst_dim > 0 ? OBST_BYTES : 0));
+}
 
 // fp32 side parameters of one tower
 struct TowerParams {
@@ -71,6 +82,7 @@ struct TowerParams {
     float head_wt[FF * MAX_ACT];            // [512][8]: transposed nn.Linear.weight, zero-padded
     float head_b[MAX_ACT];
     float obst_bias[2 * H];                 // b_obst1, b_obst2 (read through L1: shared memory has no room left)
+    float nbr_b3[H];                        // MLP neighbour encoder: b_nbr3 (read through L1, like the obstacle biases)
 };
 constexpr int B_SELF1 = 0, B_SELF2 = H, B_NBR1 = 2 * H, B_NBR2 = 3 * H, B_FF = 4 * H, N_BIAS = 4 * H + FF;
 
@@ -215,11 +227,12 @@ __device__ __noinline__ void issue_chunk_ts(uint32_t acc, uint32_t a_col, uint32
     __syncwarp();
 }
 // first layers: the 128 x 32 x tile (shared memory) against an (N = 128) x (K = 32) image
+template <bool FIRST = true>
 __device__ __noinline__ void issue_l1_ss(uint32_t acc, uint32_t x_addr, uint32_t w_addr)
 {
     const uint64_t ad = DESC_X | (uint64_t)(x_addr >> 4), bd = DESC_W32 | (uint64_t)(w_addr >> 4);
     if (elect_one()) {
-        mma_ss(acc, ad, bd, IDESC, 0u);
+        mma_ss(acc, ad, bd, IDESC, FIRST ? 0u : 1u);
         mma_ss(acc, ad + 256u, bd + 16u, IDESC, 1u);       // next K-half of the x tile: 2 chunks of 2048 B
     }
     __syncwarp();
@@ -294,10 +307,12 @@ static_assert(sizeof(Smem) <= 232448, "shared-memory map exceeds the 227 KB a bl
 // element (row, k) of an x tile: K-chunk (8 elements, 16 B) major, then 8-row groups of 128 B: LBO = 2048, SBO = 128
 __device__ __forceinline__ uint32_t xoff(int row, int kchunk) { return (uint32_t)(kchunk * 2048 + (row >> 3) * 128 + (row & 7) * 16); }
 
-// OB: with the obstacle encoder (a compile-time variant, so that the plain kernel keeps its register allocation and code layout)
-template <bool OB>
+// OB: with the obstacle encoder, MLP: with the MLP neighbour encoder instead of deep-sets (compile-time variants, so that the plain kernel keeps
+// its register allocation and code layout)
+template <bool OB, bool MLP>
 __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const KernelArgs<OB> a)
 {
+    static_assert(!(OB && MLP), "the MLP neighbour encoder is built without the obstacle encoder");
     extern __shared__ __align__(128) uint8_t smem_raw[];
     Smem &sm = *reinterpret_cast<Smem *>(smem_raw);
     const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
@@ -329,7 +344,8 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Kernel
     // Feed-forward input [self | neighbour mean | obstacle]: R10 | R11 | -- without obstacles (the quarters ping-pong between ACC0 and ACC1);
     // R10 | ACC1 | R11 with them: the three 256-wide activations leave one accumulator, ACC0, for all four quarters
     constexpr uint32_t R_MEAN = OB ? ACC1 : R11;
-    const int S = a.S, W = a.W, V = a.V, A = a.A;
+    // V: deep-sets neighbour passes (none with the MLP encoder, whose W V inputs are one vector)
+    const int S = a.S, W = a.W, V = MLP ? 0 : a.V, A = a.A;
     const int n_tiles = (a.n + TILE_M - 1) / TILE_M;
     // phase bookkeeping, advanced identically by every role: items issued per stream, tiles, ring chunks
     uint32_t n_it0 = 0u, n_it1 = 0u, n_tile = 0u, n_chunk = 0u;
@@ -345,10 +361,11 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Kernel
         if (warp == 9) {
             for (int tower = 0; tower < 2; ++tower) {
                 // the whole tower image, in consumption order, once per tile: [neighbour encoder (9 chunks, skipped without neighbours) |
-                // self L1 | self L2 x 8 | (OB: obstacle L1 | obstacle L2 x 8) | feed-forward x 32 (OB: x 48)]
+                // self L1 | self L2 x 8 | (OB: obstacle L1 | obstacle L2 x 8) (MLP: L1 x 2 | L2 x 8 | L3 x 8) | feed-forward x 32 (OB: x 48)];
+                // the MLP image starts at the self encoder
                 if (lane == 0) {
-                    const uint8_t *img = a.wimg[tower] + (V > 0 ? 0 : RES_BYTES);
-                    const int n_loads = (V > 0 ? RES_CHUNKS : 0) + STREAM_CHUNKS + (OB ? OBST_CHUNKS : 0);
+                    const uint8_t *img = a.wimg[tower] + (V > 0 || MLP ? 0 : RES_BYTES);
+                    const int n_loads = (V > 0 ? RES_CHUNKS : 0) + STREAM_CHUNKS + (OB ? OBST_CHUNKS : 0) + (MLP ? MLP_CHUNKS : 0);
                     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
                         for (int i = 0; i < n_loads; ++i) {
                             const uint32_t slot = n_chunk % STAGES;
@@ -488,18 +505,62 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Kernel
                                 if (tr) { if (lane == 0) a.trace[tm] = clock64(); tm += 1; }
                             }
                         }
+                        if constexpr (MLP) {
+                            // ---- MLP neighbour encoder layer 1: per half, K = 32 against stream 1's x tile (inputs 0-31), then K = 32 against
+                            //      stream 0's (inputs 32-39 in its neighbour slots; this image is zero in the self slots)
+                            {
+                                const uint32_t sa = ring_take();
+                                n_chunk += 1;
+                                const uint32_t sb = ring_take();
+                                n_chunk += 1;
+                                for (int s = 0; s < 2; ++s) {
+                                    wait_prev(s);
+                                    issue_l1_ss(tmem + (s ? ACC1 : ACC0), xb1, ring0 + sa * (uint32_t)CHUNK + (uint32_t)s * CHUNK1);
+                                    issue_l1_ss<false>(tmem + (s ? ACC1 : ACC0), xb0, ring0 + sb * (uint32_t)CHUNK + (uint32_t)s * CHUNK1);
+                                    commit_one(&sm.acc_full[s]);
+                                    N_ITEM_INC(s);
+                                    if (tr) { if (lane == 0) a.trace[tm] = clock64(); tm += 1; }
+                                }
+                                commit_one(&sm.empty[sa]);
+                                commit_one(&sm.empty[sb]);
+                            }
+                            // ---- layers 2 and 3: A = R11, output back into R11 (in place: the epilogue writes it once BOTH halves have completed)
+                            for (int layer = 0; layer < 2; ++layer) {
+                                wait_prev(0);
+                                wait_prev(1);
+                                for (int s = 0; s < 2; ++s) {
+#pragma unroll
+                                    for (int c = 0; c < 4; ++c) {
+                                        const uint32_t slot = ring_take();
+                                        if (c == 0) issue_chunk_ts<true>(tmem + (s ? ACC1 : ACC0), tmem + R11, ring0 + slot * (uint32_t)CHUNK);
+                                        else issue_chunk_ts<false>(tmem + (s ? ACC1 : ACC0), tmem + R11 + (uint32_t)c * 32u, ring0 + slot * (uint32_t)CHUNK);
+                                        held[c] = slot;
+                                        n_chunk += 1;
+                                    }
+#pragma unroll
+                                    for (int c = 0; c < 4; ++c) commit_one(&sm.empty[held[c]]);
+                                    commit_one(&sm.acc_full[s]);
+                                    N_ITEM_INC(s);
+                                    if (tr) { if (lane == 0) a.trace[tm] = clock64(); tm += 1; }
+                                }
+                            }
+                        }
                         // ---- feed-forward: four quarters of 128 outputs, K = 512 (OB: 768): chunks 0-3 read R10 (self encoder), chunks 4-7 R_MEAN
-                        //      (neighbour mean, written by the epilogue warps while the first half of quarter 0 runs), OB: chunks 8-11 R11 (obstacle)
+                        //      (neighbour mean, written by the epilogue warps while the first half of quarter 0 runs; MLP: the encoder's output,
+                        //      whose second half is written meanwhile), OB: chunks 8-11 R11 (obstacle)
                         constexpr int FF_CHUNKS = OB ? 12 : 8;
                         for (int qtr = 0; qtr < 4; ++qtr) {
                             const int s = OB ? 0 : (qtr & 1);
                             wait_prev(s);
-                            if (qtr == 0) wait_prev(1);
+                            if (qtr == 0 && !MLP) wait_prev(1);
 #pragma unroll
                             for (int c = 0; c < FF_CHUNKS; ++c) {
                                 const uint32_t slot = ring_take();
                                 const uint32_t acol = tmem + (c < 4 ? R10 + (uint32_t)c * 32u : c < 8 ? R_MEAN + (uint32_t)(c - 4) * 32u : R11 + (uint32_t)(c - 8) * 32u);
-                                if (c == 4 && qtr == 0) { mbar_wait(&sm.mean_ready, (n_tile - 1u) & 1u); tc_fence_after(); }
+                                if (c == 4 && qtr == 0) {
+                                    if constexpr (MLP) wait_prev(1);
+                                    else { mbar_wait(&sm.mean_ready, (n_tile - 1u) & 1u); tc_fence_after(); }
+                                }
                                 if (c == 0) issue_chunk_ts<true>(tmem + (s ? ACC1 : ACC0), acol, ring0 + slot * (uint32_t)CHUNK);
                                 else issue_chunk_ts<false>(tmem + (s ? ACC1 : ACC0), acol, ring0 + slot * (uint32_t)CHUNK);
                                 held[c & 3] = slot;
@@ -590,7 +651,18 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Kernel
                         for (int i = 0; i < 8; ++i) f[i] = (live && kc * 8 + i < S) ? __ldg(orow + kc * 8 + i) : 0.f;
                         const uint4 u = make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
                         *reinterpret_cast<uint4 *>(sm.xbuf[0] + xoff(row_l, kc)) = u;
-                        if constexpr (!OB) *reinterpret_cast<uint4 *>(sm.xbuf[1] + xoff(row_l, kc)) = u;
+                        if constexpr (!OB && !MLP) *reinterpret_cast<uint4 *>(sm.xbuf[1] + xoff(row_l, kc)) = u;
+                    }
+                } else if constexpr (MLP) {
+                    // the W V neighbour inputs (columns S ..): 0-31 fill stream 1's tile, 32-39 the neighbour slots of stream 0's
+                    const int WV = W * a.V;
+#pragma unroll
+                    for (int kc = 0; kc < MAX_MLP_IN / 8; ++kc) {
+                        float f[8];
+#pragma unroll
+                        for (int i = 0; i < 8; ++i) f[i] = (live && kc * 8 + i < WV) ? __ldg(orow + S + kc * 8 + i) : 0.f;
+                        *reinterpret_cast<uint4 *>(kc < 4 ? sm.xbuf[1] + xoff(row_l, kc) : sm.xbuf[0] + xoff(row_l, 3)) =
+                            make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
                     }
                 } else {
                     if (V > 0) *reinterpret_cast<uint4 *>(sm.xbuf[0] + xoff(row_l, 3)) = nbr_chunk(0);
@@ -664,9 +736,21 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Kernel
                     asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS) : "memory");
                     tc_fence_after();
                 }
+                if constexpr (MLP) {
+                    // ---- MLP neighbour encoder layer 1 -> hidden in R11 (the self encoder's layer-2 MMAs, R11's last readers, have completed)
+                    for (int s = 0; s < 2; ++s) { wait_acc(s); epi_to_tmem(s ? ACC1 : ACC0, sm.bias + B_NBR1, s, R11); item_done(s); }
+                    // ---- layers 2 and 3 -> R11 in place: both halves' MMAs must have completed before either half is written.  The feed-forward
+                    //      reads R10 while layer 3's second half is written (its issuer waits for that half before its 5th K chunk)
+                    for (int layer = 0; layer < 2; ++layer) {
+                        const float *bias = layer == 0 ? sm.bias + B_NBR2 : P->nbr_b3;
+                        wait_acc(0);
+                        wait_acc(1);
+                        for (int s = 0; s < 2; ++s) { epi_to_tmem(s ? ACC1 : ACC0, bias, s, R11); item_done(s); }
+                    }
+                }
                 // ---- neighbour mean -> R_MEAN (no neighbours: zeros, like an absent encoder half).  Its last readers (R11: the self encoder's
                 //      layer-2 MMAs; OB, ACC1: the epilogue above) are done; the feed-forward reads it from its 5th K chunk on
-                {
+                if constexpr (!MLP) {
                     const float inv = V > 0 ? 1.0f / (float)V : 0.f;
 #pragma unroll
                     for (int h = 0; h < 2; ++h)
@@ -746,7 +830,7 @@ __global__ void __launch_bounds__(THREADS, 1) policy_forward_kernel(const Kernel
 // ---- weight packing: nn.Linear weight [out, in] fp32 -> chunk images (bf16, canonical K-major core-matrix layout) ----------------
 // image of rows n0 .. n0+127 and kc input slots of W: byte offset of element (n, k) = (n / 8) * SBO + (k / 8) * 128 + (n % 8) * 16 +
 // (k % 8) * 2, SBO = (kc / 8) * 128.  Slot k reads input column k0 + k, or -- first layers, `split` > 0 -- column k for k < split and
-// column len1 + (k - split) behind it (the [self | neighbour] K layout); columns beyond the matrix are zero.
+// column k0 + len1 + (k - split) behind it (the [self | neighbour] K layout); columns beyond the matrix are zero.
 __global__ void pack_chunk_kernel(const float *w, int out_dim, int in_dim, int n0, int k0, int kc, int split, int len1, uint8_t *img)
 {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
@@ -754,7 +838,7 @@ __global__ void pack_chunk_kernel(const float *w, int out_dim, int in_dim, int n
     const int n = idx / kc, k = idx % kc;
     const int gn = n0 + n;
     int gk = k0 + k;
-    if (split > 0) gk = k < split ? (k < len1 ? k : -1) : len1 + (k - split);
+    if (split > 0) gk = k < split ? (k < len1 ? k : -1) : k0 + len1 + (k - split);
     const float v = (gn < out_dim && gk >= 0 && gk < in_dim) ? w[(size_t)gn * in_dim + gk] : 0.f;
     const size_t off = (size_t)(n / 8) * ((size_t)(kc / 8) * 128) + (size_t)(k / 8) * 128 + (size_t)(n % 8) * 16 + (size_t)(k % 8) * 2;
     *reinterpret_cast<__nv_bfloat16 *>(img + off) = __float2bfloat16_rn(v);
@@ -1073,6 +1157,7 @@ static void launch_bwd_w(int in_dim, int grid, int threads, cudaStream_t s, cons
 
 struct qp_policy {
     qp_config cfg;
+    int nbr_encoder;        // QP_NBR_DEEPSETS / QP_NBR_MLP
     int device, sms;
     uint8_t *wimg[2];
     TowerParams *params[2];
@@ -1096,7 +1181,9 @@ extern "C" {
 const char *qp_last_error(const qp_policy *p) { return p ? p->err.c_str() : g_qp_err.c_str(); }
 size_t qp_config_size(void) { return sizeof(qp_config); }
 
-int qp_create(const qp_config *cfg, int device, qp_policy **out)
+int qp_create(const qp_config *cfg, int device, qp_policy **out) { return qp_create_encoder(cfg, QP_NBR_DEEPSETS, device, out); }
+
+int qp_create_encoder(const qp_config *cfg, int nbr_encoder, int device, qp_policy **out)
 {
     if (!cfg || !out) return qp_fail(nullptr, QP_ERR_NULL, "qp_create: null argument");
     *out = nullptr;
@@ -1109,20 +1196,29 @@ int qp_create(const qp_config *cfg, int device, qp_policy **out)
         return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create: self_dim must be in [1, 24], nbr_dim in [0, 8]");
     if (c.act_dim < 1 || c.act_dim > MAX_ACT) return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create: act_dim out of [1, 8]");
     if (c.obst_dim < 0 || c.obst_dim > MAX_OBST) return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create: obst_dim out of [0, 24]");
+    if (nbr_encoder != QP_NBR_DEEPSETS && nbr_encoder != QP_NBR_MLP)
+        return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create_encoder: unknown nbr_encoder (QP_NBR_DEEPSETS = 0, QP_NBR_MLP = 1)");
+    const bool mlp = nbr_encoder == QP_NBR_MLP;
+    if (mlp && (c.num_nbr < 1 || c.nbr_dim < 1))
+        return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create_encoder: the MLP neighbour encoder needs num_nbr >= 1 and nbr_dim >= 1");
+    if (mlp && c.nbr_dim * c.num_nbr > MAX_MLP_IN)
+        return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create_encoder: the MLP neighbour encoder takes nbr_dim * num_nbr <= 40 inputs");
+    if (mlp && c.obst_dim > 0)
+        return qp_fail(nullptr, QP_ERR_BAD_CONFIG, "qp_create_encoder: the MLP neighbour encoder is built without the obstacle encoder (obst_dim must be 0)");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || device < 0 || device >= ndev) return qp_fail(nullptr, QP_ERR_CUDA, "qp_create: no such CUDA device");
     int prev = 0;
     cudaGetDevice(&prev);
     cudaSetDevice(device);
     qp_policy *p = new qp_policy();
-    p->cfg = c; p->device = device; p->launches = 0; p->trace = nullptr; p->max_grid = 0;
+    p->cfg = c; p->nbr_encoder = nbr_encoder; p->device = device; p->launches = 0; p->trace = nullptr; p->max_grid = 0;
     if (const char *g = getenv("QP_MAX_GRID")) p->max_grid = atoi(g);
     p->stagger = STAGGER_CLK;
     if (const char *g = getenv("QP_STAGGER")) p->stagger = atoi(g);
     p->wimg[0] = p->wimg[1] = nullptr; p->params[0] = p->params[1] = nullptr;
     cudaDeviceGetAttribute(&p->sms, cudaDevAttrMultiProcessorCount, device);
     cudaError_t r = cudaSuccess;
-    const size_t img_bytes = tower_img_bytes(c.obst_dim);
+    const size_t img_bytes = tower_img_bytes(c.obst_dim, mlp);
     for (int t = 0; t < 2 && r == cudaSuccess; ++t) {
         r = cudaMalloc(&p->wimg[t], img_bytes);
         if (r == cudaSuccess) r = cudaMemset(p->wimg[t], 0, img_bytes);
@@ -1130,8 +1226,9 @@ int qp_create(const qp_config *cfg, int device, qp_policy **out)
         if (r == cudaSuccess) r = cudaMemset(p->params[t], 0, sizeof(TowerParams));
     }
     if (r == cudaSuccess)
-        r = c.obst_dim > 0 ? cudaFuncSetAttribute(policy_forward_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem))
-                           : cudaFuncSetAttribute(policy_forward_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
+        r = mlp              ? cudaFuncSetAttribute(policy_forward_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem))
+            : c.obst_dim > 0 ? cudaFuncSetAttribute(policy_forward_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem))
+                             : cudaFuncSetAttribute(policy_forward_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
     cudaSetDevice(prev);
     if (r != cudaSuccess) {
         for (int t = 0; t < 2; ++t) { cudaFree(p->wimg[t]); cudaFree(p->params[t]); }
@@ -1163,6 +1260,9 @@ int qp_set_weights(qp_policy *p, int tower, const qp_tower_weights *w, void *str
     const int S = p->cfg.self_dim, O = p->cfg.obst_dim;
     if (O > 0 && (!w->obst_w1 || !w->obst_b1 || !w->obst_w2 || !w->obst_b2))       // a handle without obstacles never reads these fields
         return qp_fail(p, QP_ERR_NULL, "qp_set_weights: null obstacle-encoder pointer (obst_dim > 0)");
+    const bool mlp = p->nbr_encoder == QP_NBR_MLP;
+    if (mlp && (!w->nbr_w3 || !w->nbr_b3))                                          // a deep-sets handle never reads these fields
+        return qp_fail(p, QP_ERR_NULL, "qp_set_weights: null nbr_w3 / nbr_b3 (MLP neighbour encoder)");
     cudaStream_t s = (cudaStream_t)stream;
     const int n_out = tower == 0 ? p->cfg.act_dim : 1;
     uint8_t *img = p->wimg[tower];
@@ -1170,16 +1270,16 @@ int qp_set_weights(qp_policy *p, int tower, const qp_tower_weights *w, void *str
     auto pack = [&](const float *src, int out_dim, int in_dim, int n0, int k0, int kc, int split, int len1, uint8_t *dst) {
         pack_chunk_kernel<<<(NH * kc + 255) / 256, 256, 0, s>>>(src, out_dim, in_dim, n0, k0, kc, split, len1, dst);
     };
-    // resident block: neighbour L1 halves, neighbour L2 (half, K chunk)
-    if (p->cfg.num_nbr > 0) {
+    // resident block: neighbour L1 halves, neighbour L2 (half, K chunk); the MLP image has none
+    if (p->cfg.num_nbr > 0 && !mlp) {
         // phi reads the neighbour row alone: its W inputs sit in K slots 24..31 (the x tile's neighbour chunk), the self slots meet zeros
         for (int h = 0; h < 2; ++h) pack(w->nbr_w1, H, p->cfg.nbr_dim, NH * h, 0, 32, SELF_PAD, 0, img + (size_t)h * CHUNK1);
         for (int h = 0; h < 2; ++h)
             for (int c = 0; c < 4; ++c) pack(w->nbr_w2, H, H, NH * h, 64 * c, 64, 0, 0, img + 2 * CHUNK1 + (size_t)(h * 4 + c) * CHUNK);
     }
     // streamed block, in consumption order: self L1 halves, self L2 (half, chunk), [obstacle L1 halves, obstacle L2 (half, chunk),]
-    // feed-forward (quarter, chunk)
-    uint8_t *st = img + RES_BYTES;
+    // [MLP L1 (image, half), MLP L2 and L3 (half, chunk),] feed-forward (quarter, chunk)
+    uint8_t *st = img + (mlp ? 0 : RES_BYTES);
     auto pack_encoder = [&](const float *w1, int in_dim, const float *w2) {
         // layer 1 reads K slots 0 .. in_dim - 1 of its x tile; the neighbour slots (24..31) meet zeros
         for (int h = 0; h < 2; ++h) pack(w1, H, in_dim, NH * h, 0, 32, SELF_PAD, in_dim, st + (size_t)h * CHUNK1);
@@ -1190,6 +1290,19 @@ int qp_set_weights(qp_policy *p, int tower, const qp_tower_weights *w, void *str
     };
     pack_encoder(w->self_w1, S, w->self_w2);
     if (O > 0) pack_encoder(w->obst_w1, O, w->obst_w2);
+    if (mlp) {
+        // layer 1, per half: K slots 0..31 = inputs 0..31 (stream 1's x tile), then slots 24..31 = inputs 32..39 (stream 0's neighbour
+        // slots) with zeros in the self slots
+        const int in_dim = p->cfg.nbr_dim * p->cfg.num_nbr;
+        for (int h = 0; h < 2; ++h) pack(w->nbr_w1, H, in_dim, NH * h, 0, 32, 0, 0, st + (size_t)h * CHUNK1);
+        for (int h = 0; h < 2; ++h) pack(w->nbr_w1, H, in_dim, NH * h, 32, 32, SELF_PAD, 0, st + (size_t)(2 + h) * CHUNK1);
+        st += 4 * CHUNK1;
+        for (const float *wl : { w->nbr_w2, w->nbr_w3 }) {
+            for (int h = 0; h < 2; ++h)
+                for (int c = 0; c < 4; ++c) pack(wl, H, H, NH * h, 64 * c, 64, 0, 0, st + (size_t)(h * 4 + c) * CHUNK);
+            st += 8 * CHUNK;
+        }
+    }
     const int ff_chunks = O > 0 ? 12 : 8, ff_in = 64 * ff_chunks;         // K = [self | neighbour (| obstacle)]
     for (int qtr = 0; qtr < 4; ++qtr)
         for (int c = 0; c < ff_chunks; ++c) pack(w->ff_w, FF, ff_in, NH * qtr, 64 * c, 64, 0, 0, st + (size_t)(qtr * ff_chunks + c) * CHUNK);
@@ -1202,6 +1315,7 @@ int qp_set_weights(qp_policy *p, int tower, const qp_tower_weights *w, void *str
         QP_CUDA(p, cudaMemcpyAsync(P->bias + B_NBR2, w->nbr_b2, H * sizeof(float), dd, s));
     }
     QP_CUDA(p, cudaMemcpyAsync(P->bias + B_FF, w->ff_b, FF * sizeof(float), dd, s));
+    if (mlp) QP_CUDA(p, cudaMemcpyAsync(P->nbr_b3, w->nbr_b3, H * sizeof(float), dd, s));
     if (O > 0) {
         QP_CUDA(p, cudaMemcpyAsync(P->obst_bias, w->obst_b1, H * sizeof(float), dd, s));
         QP_CUDA(p, cudaMemcpyAsync(P->obst_bias + H, w->obst_b2, H * sizeof(float), dd, s));
@@ -1346,8 +1460,9 @@ int qp_forward(qp_policy *p, const float *obs, int n, int obs_stride, float *mea
     const int tiles = (n + TILE_M - 1) / TILE_M;
     int grid = tiles < p->sms ? tiles : p->sms;
     if (p->max_grid > 0 && grid > p->max_grid) grid = p->max_grid;
-    if (a.O > 0) policy_forward_kernel<true><<<grid, THREADS, sizeof(Smem), (cudaStream_t)stream>>>(a);
-    else policy_forward_kernel<false><<<grid, THREADS, sizeof(Smem), (cudaStream_t)stream>>>(static_cast<const Args &>(a));
+    if (p->nbr_encoder == QP_NBR_MLP) policy_forward_kernel<false, true><<<grid, THREADS, sizeof(Smem), (cudaStream_t)stream>>>(static_cast<const Args &>(a));
+    else if (a.O > 0) policy_forward_kernel<true, false><<<grid, THREADS, sizeof(Smem), (cudaStream_t)stream>>>(a);
+    else policy_forward_kernel<false, false><<<grid, THREADS, sizeof(Smem), (cudaStream_t)stream>>>(static_cast<const Args &>(a));
     p->launches += 1;
     QP_CUDA(p, cudaGetLastError());
     return QP_OK;

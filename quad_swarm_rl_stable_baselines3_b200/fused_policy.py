@@ -4,6 +4,8 @@ swarm_rl/models/quad_multi_model.py:333-354).  One kernel launch per batch of ob
 
 The torch module (`ppo.QuadActorCritic`) stays the owner of the parameters and is what the PPO update differentiates; this class
 re-packs its weights into the kernel's bf16 tile images (`sync()`, once per rollout) and evaluates mean / value for the rollout.
+Built for the deep-sets ('mean_embed') and 'mlp' neighbour encoders and for none; `supported()` tells which policies stay on the torch
+path (the 'attention' encoder, 'mlp' with the obstacle encoder or with more than 40 neighbour inputs).
 There is no fallback: on a box without the CUDA library the constructor raises."""
 from __future__ import annotations
 
@@ -15,6 +17,8 @@ from . import _capi
 
 
 QP_API_VERSION = 2
+QP_NBR = {"mean_embed": 0, "none": 0, "mlp": 1}          # qp_create_encoder's nbr_encoder: QP_NBR_DEEPSETS, QP_NBR_MLP
+MLP_MAX_INPUTS = 40                                      # W * V the MLP neighbour encoder's first layer reads (two K = 32 x-tile slots)
 
 
 class QpConfigC(C.Structure):
@@ -23,18 +27,22 @@ class QpConfigC(C.Structure):
 
 class QpTowerWeightsC(C.Structure):
     FIELDS = ("self_w1", "self_b1", "self_w2", "self_b2", "nbr_w1", "nbr_b1", "nbr_w2", "nbr_b2", "ff_w", "ff_b", "head_w", "head_b",
-              "obst_w1", "obst_b1", "obst_w2", "obst_b2")
+              "obst_w1", "obst_b1", "obst_w2", "obst_b2", "nbr_w3", "nbr_b3")
     _fields_ = [(n, C.c_void_p) for n in FIELDS]
 
 
 def supported(policy) -> bool:
     """The architecture the kernel is built for: deep-sets ('mean_embed') or no neighbour encoder, optionally the obstacle encoder
-    (9 SDF inputs), hidden 256."""
+    (9 SDF inputs), or the 'mlp' neighbour encoder with at most 40 inputs (W * V) and no obstacle encoder; hidden 256."""
     enc = policy.actor
-    return (enc.kind in ("mean_embed", "none") and enc.O in (0, 9) and enc.self_encoder[0].out_features == 256
-            and enc.S <= 24 and enc.W <= 8 and policy.action_net.out_features <= 8 and (enc.kind == "none" or enc.neighbor[0].out_features == 256)
+    if enc.kind == "mlp" and (enc.O != 0 or enc.W * enc.V > MLP_MAX_INPUTS):
+        return False
+    return (enc.kind in ("mean_embed", "mlp", "none") and enc.O in (0, 9) and enc.self_encoder[0].out_features == 256
+            and enc.S <= 24 and enc.W <= 8 and policy.action_net.out_features <= 8
+            and (enc.kind == "none" or all(m.out_features == 256 for m in enc.neighbor if isinstance(m, torch.nn.Linear)))
             and (enc.O == 0 or enc.obstacle[0].out_features == 256))
-    # 'attention' (the fork's default, quad_multi_model.py:42-102) and 'mlp' stay on the torch path
+    # 'attention' (the fork's default, quad_multi_model.py:42-102: rows depend on other rows through its .repeat(V, 1)), 'mlp' with the
+    # obstacle encoder (no tensor-memory region left for its output) and 'mlp' with W * V > 40 stay on the torch path
 
 
 def gae(rewards: torch.Tensor, values: torch.Tensor, dones: torch.Tensor, last_values: torch.Tensor, gamma: float, lam: float):
@@ -166,13 +174,15 @@ def bias_tanh_mean_backward(grad_mean: torch.Tensor, y: torch.Tensor, V: int):
 class FusedPolicy:
     def __init__(self, policy, device):
         if not supported(policy):
-            raise ValueError("the fused policy kernel is built for hidden 256, deep-sets / no neighbour encoder, optional obstacle encoder, S <= 24, W <= 8")
+            raise ValueError("the fused policy kernel is built for hidden 256, deep-sets / no neighbour encoder with an optional obstacle encoder, "
+                             "or the MLP neighbour encoder with W * V <= 40 and no obstacle encoder; S <= 24, W <= 8")
         self.policy = policy
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise RuntimeError("FusedPolicy runs on CUDA devices only (no CPU path)")
         enc = policy.actor
-        self.S, self.W, self.V, self.O = enc.S, enc.W, (enc.V if enc.kind == "mean_embed" else 0), enc.O
+        self.kind = enc.kind
+        self.S, self.W, self.V, self.O = enc.S, enc.W, (enc.V if enc.kind in ("mean_embed", "mlp") else 0), enc.O
         self.A = policy.action_net.out_features
         self._lib = _capi.lib()
         cfg = QpConfigC(QP_API_VERSION, self.S, self.W, self.V, 256, self.A, self.O)
@@ -180,9 +190,9 @@ class FusedPolicy:
             raise RuntimeError("qp_config layout mismatch")
         h = C.c_void_p()
         with torch.cuda.device(self.device):
-            rc = self._lib.qp_create(C.byref(cfg), self.device.index or 0, C.byref(h))
+            rc = self._lib.qp_create_encoder(C.byref(cfg), QP_NBR[self.kind], self.device.index or 0, C.byref(h))
         if rc != 0:
-            raise RuntimeError(f"qp_create failed ({rc}): {self._lib.qp_last_error(None).decode()}")
+            raise RuntimeError(f"qp_create_encoder failed ({rc}): {self._lib.qp_last_error(None).decode()}")
         self._h = h
         self._keep = []
         self.sync()
@@ -217,6 +227,8 @@ class FusedPolicy:
             if self.V > 0:
                 t.update({"nbr_w1": enc.neighbor[0].weight, "nbr_b1": enc.neighbor[0].bias,
                           "nbr_w2": enc.neighbor[2].weight, "nbr_b2": enc.neighbor[2].bias})
+            if self.kind == "mlp":
+                t.update({"nbr_w3": enc.neighbor[4].weight, "nbr_b3": enc.neighbor[4].bias})
             if self.O > 0:
                 t.update({"obst_w1": enc.obstacle[0].weight, "obst_b1": enc.obstacle[0].bias,
                           "obst_w2": enc.obstacle[2].weight, "obst_b2": enc.obstacle[2].bias})

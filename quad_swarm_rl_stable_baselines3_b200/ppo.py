@@ -11,8 +11,9 @@ with a `QuadMultiEncoder` per tower (swarm_rl/models/quad_multi_model.py:250-354
 state-independent log-std diagonal Gaussian (log_std_init 0, no squashing), xavier-uniform initialisation.  The dense layers
 of the torch module are plain PyTorch (cuBLAS) and are what the update differentiates; at rollout time the forward runs on the
 hand-written tcgen05 kernel (`fused_policy.py`, csrc/policy_kernels.cu: both towers and heads in one launch, activations in
-tensor memory; deep-sets or no neighbour encoder, with or without the obstacle encoder; parity against this module in
-tests/test_gpu_policy.py and tests/test_gpu_policy_obstacles.py) and GAE on `qp_gae` (one launch).  Nothing of SB3's
+tensor memory; deep-sets or no neighbour encoder, with or without the obstacle encoder, or the 'mlp' neighbour encoder with at most
+40 inputs and no obstacle encoder; parity against this module in tests/test_gpu_policy.py, tests/test_gpu_policy_obstacles.py and
+tests/test_gpu_policy_mlp.py; the 'attention' encoder and the other 'mlp' policies stay on the torch path) and GAE on `qp_gae` (one launch).  Nothing of SB3's
 arithmetic is pinned by a reference test (SB3 is not installed in the build image) -- "parity unpinned" for the update; the
 GAE recursion is tested against a numpy restatement of SB3's `RolloutBuffer.compute_returns_and_advantage`.
 
