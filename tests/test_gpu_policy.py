@@ -173,27 +173,89 @@ def test_device_ppo_uses_the_fused_rollout():
 
 
 def test_two_policies_and_argument_checks():
-    """Two handles alive at once (a training policy and an evaluation copy, as sb_train.py keeps them), interleaved forwards; the C-ABI
-    rejects bad shapes with a message instead of launching."""
+    """Handles of every built variant alive at once (a training policy and an evaluation copy, as sb_train.py keeps them, of each
+    encoder): deep-sets (cfg2 and the fork's), obstacle, MLP, and an MLP handle made from the six-field version-1 qp_config.  Their
+    forwards interleave on the default stream and a second one, and each output equals, bit for bit, the same handle's forward run alone;
+    repacking one handle's weights and then destroying another leave the remaining handles' outputs bitwise unchanged.  The C-ABI rejects
+    bad shapes with a message instead of launching."""
     import ctypes as C
     import torch
     from quad_swarm_rl_stable_baselines3_b200 import _capi
-    from quad_swarm_rl_stable_baselines3_b200.fused_policy import FusedPolicy
+    from quad_swarm_rl_stable_baselines3_b200.fused_policy import QP_NBR, FusedPolicy
     from quad_swarm_rl_stable_baselines3_b200.ppo import QuadActorCritic
     dev = torch.device("cuda:0")
-    torch.manual_seed(5)
-    pa = QuadActorCritic(QuadSimConfig(num_envs=8, num_agents=8)).to(dev)
-    pb = QuadActorCritic(QuadSimConfig.fork_default(num_envs=8)).to(dev)
-    fa, fb = FusedPolicy(pa, dev), FusedPolicy(pb, dev)
-    oa, ob = torch.randn(3000, 54, device=dev), torch.randn(700, pb.actor.S + pb.actor.W * pb.actor.V, device=dev)
-    for _ in range(3):
-        ma, _ = fa.forward(oa)
-        mb, vb = fb.forward(ob)
-    with torch.no_grad():
-        assert float((ma - pa.action_net(pa.actor(oa))).abs().max()) <= TOL_FP32_MAX
-        assert float((mb - pb.action_net(pb.actor(ob))).abs().max()) <= TOL_FP32_MAX
-        assert float((vb - pb.value(ob)).abs().max()) <= TOL_FP32_MAX
     lib = _capi.lib()
+    torch.manual_seed(5)
+    fork_k8 = QuadSimConfig.fork_default(num_envs=8, num_agents=8, neighbor_obs_type="dist_sangle_sheading",
+                                         obs_repr="cdist_cdistdot_dist_distdot_sangle_angledot")           # MLP: 35 inputs
+    pols = {"deepsets": QuadActorCritic(QuadSimConfig(num_envs=8, num_agents=8)),
+            "fork": QuadActorCritic(QuadSimConfig.fork_default(num_envs=8)),
+            "obstacles": QuadActorCritic(QuadSimConfig(num_envs=8, num_agents=8, quads_mode="mix", use_obstacles=True,
+                                                       obs_repr="xyz_vxyz_R_omega_floor", neighbor_visible_num=2)),
+            "mlp": QuadActorCritic(QuadSimConfig(num_envs=8, num_agents=8), neighbor_encoder="mlp"),
+            "mlp_v1": QuadActorCritic(fork_k8, neighbor_encoder="mlp")}
+    rows = {"deepsets": 3000, "fork": 700, "obstacles": 1500, "mlp": 2100, "mlp_v1": 900}
+    obs = {}
+    for k, pol in pols.items():
+        pol.to(dev)
+        with torch.no_grad():                                     # non-zero biases
+            for m in pol.modules():
+                if isinstance(m, torch.nn.Linear):
+                    m.bias.uniform_(-0.3, 0.3)
+        enc = pol.actor
+        obs[k] = torch.randn(rows[k], enc.S + enc.W * enc.V + enc.O, device=dev) * 0.8
+    fps = {k: FusedPolicy(pol, dev) for k, pol in pols.items()}
+    assert fps["obstacles"].O == 9 and fps["mlp"].kind == "mlp" and fps["mlp_v1"].kind == "mlp"
+
+    # version 1: the struct ends before obst_dim (a C caller of the first release)
+    class QpConfigV1(C.Structure):
+        _fields_ = [(n, C.c_int32) for n in ("api_version", "self_dim", "nbr_dim", "num_nbr", "hidden", "act_dim")]
+
+    f1, h1 = fps["mlp_v1"], C.c_void_p()
+    assert lib.qp_create_encoder(C.byref(QpConfigV1(1, f1.S, f1.W, f1.V, 256, f1.A)), QP_NBR["mlp"], 0, C.byref(h1)) == 0 and h1.value
+    lib.qp_destroy(f1._h)
+    f1._h = h1                                                    # the same policy, packed into the version-1 handle
+    f1.sync()
+
+    alone = {}
+    for k, fp in fps.items():
+        alone[k] = fp.forward(obs[k])
+        torch.cuda.synchronize()
+        pol = pols[k]
+        with torch.no_grad():
+            assert float((alone[k][0] - pol.action_net(pol.actor(obs[k]))).abs().max()) <= TOL_FP32_MAX, k
+            assert float((alone[k][1] - pol.value(obs[k])).abs().max()) <= TOL_FP32_MAX, k
+
+    def interleaved():
+        """Three rounds over the live handles; each round alternates them between the default stream and a second one."""
+        main, side = torch.cuda.current_stream(dev), torch.cuda.Stream(dev)
+        side.wait_stream(main)
+        outs = []
+        for r in range(3):
+            for i, k in enumerate(fps):
+                with torch.cuda.stream(side if (i + r) % 2 else main):
+                    outs.append((k, fps[k].forward(obs[k])))
+        torch.cuda.synchronize()
+        for k, (m, v) in outs:
+            assert torch.equal(m, alone[k][0]) and torch.equal(v, alone[k][1]), k
+
+    interleaved()
+    with torch.no_grad():                                         # new weights in one handle ...
+        for p in pols["mlp"].parameters():
+            p.add_(0.05 * torch.randn_like(p))
+    fps["mlp"].sync()
+    m, v = fps["mlp"].forward(obs["mlp"])
+    torch.cuda.synchronize()
+    assert float((m - alone["mlp"][0]).abs().max()) > 0.05
+    with torch.no_grad():
+        assert float((m - pols["mlp"].action_net(pols["mlp"].actor(obs["mlp"]))).abs().max()) <= TOL_FP32_MAX
+    alone["mlp"] = (m, v)
+    interleaved()                                                 # ... the others unchanged
+    fps.pop("obstacles").close()                                  # one handle destroyed: the others unchanged
+    interleaved()
+
+    fa = fps["deepsets"]
+    oa = obs["deepsets"]
     mean, value = torch.empty(10, 4, device=dev), torch.empty(10, device=dev)
     s = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
     assert lib.qp_forward(fa._h, oa.data_ptr(), 10, 40, mean.data_ptr(), value.data_ptr(), s) == -2      # stride shorter than S + V*W
@@ -202,4 +264,5 @@ def test_two_policies_and_argument_checks():
     assert lib.qp_forward(fa._h, oa.data_ptr(), 0, 54, mean.data_ptr(), value.data_ptr(), s) == -2
     with pytest.raises(ValueError):
         fa.forward(oa.double())
-    fa.close(); fb.close()
+    for fp in fps.values():
+        fp.close()

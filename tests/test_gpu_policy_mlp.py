@@ -226,28 +226,30 @@ def test_device_ppo_leaves_unbuilt_mlp_policies_on_torch(which):
 
 
 def test_device_ppo_mlp_config_uses_the_fused_rollout():
+    """cfg2 (W * V = 36) and the fork env (W 2, V 3: its policy's first layers have 6 inputs and train through _FirstBiasTanh)."""
     import numpy as np
     import torch
     from quad_swarm_rl_stable_baselines3_b200.ppo import DevicePPO, PPOConfig
     from quad_swarm_rl_stable_baselines3_b200.sim import QuadSwarmSim
-    cfg = cfg2(num_envs=128, ep_time=0.3, seed=2)
-    sim = QuadSwarmSim(cfg, device="cuda:0")
-    sim.want_terminal_obs = False
-    n_steps = 8
-    ppo = DevicePPO(sim, cfg, PPOConfig(n_steps=n_steps, batch_size=4096, n_epochs=1, neighbor_encoder="mlp"))
-    assert ppo.fused is not None and ppo.fused.kind == "mlp" and ppo.fused.V == 6
-    w0 = torch.cat([p.detach().reshape(-1).clone() for p in ppo.policy.parameters()])
-    l0, s0 = ppo.fused.launch_count, sim.launch_count
-    hist = ppo.learn(2)
-    assert ppo.fused.launch_count - l0 == 2 * (n_steps + 1)          # one launch per env step + the bootstrap value
-    assert sim.launch_count - s0 == 2 * n_steps
-    for r in hist:
-        assert all(np.isfinite(r[k]) for k in ("pg", "vf", "ent", "kl", "mean_reward"))
-    w1 = torch.cat([p.detach().reshape(-1) for p in ppo.policy.parameters()])
-    assert bool(torch.isfinite(w1).all()) and not torch.equal(w0, w1)
-    obs = make_obs(ppo.policy, 700)
-    m, v = fused_forward(ppo.fused, obs, 700)                         # update() packed the optimiser's weights again
-    with torch.no_grad():
-        x = obs[:700]
-        r_mean, r_value = ppo.policy.action_net(ppo.policy.actor(x)), ppo.policy.value(x)
-    assert float((m - r_mean).abs().max()) <= TOL_FP32_MAX and float((v - r_value).abs().max()) <= TOL_FP32_MAX
+    for cfg, V in ((cfg2(num_envs=128, ep_time=0.3, seed=2), 6), (QuadSimConfig.fork_default(num_envs=256, ep_time=1.0, seed=3), 3)):
+        sim = QuadSwarmSim(cfg, device="cuda:0")
+        sim.want_terminal_obs = False
+        n_steps = 8
+        ppo = DevicePPO(sim, cfg, PPOConfig(n_steps=n_steps, batch_size=4096, n_epochs=1, neighbor_encoder="mlp"))
+        assert ppo.fused is not None and ppo.fused.kind == "mlp" and ppo.fused.V == V
+        w0 = torch.cat([p.detach().reshape(-1).clone() for p in ppo.policy.parameters()])
+        l0, s0 = ppo.fused.launch_count, sim.launch_count
+        hist = ppo.learn(2)
+        assert ppo.fused.launch_count - l0 == 2 * (n_steps + 1)          # one launch per env step + the bootstrap value
+        assert sim.launch_count - s0 == 2 * n_steps
+        for r in hist:
+            assert all(np.isfinite(r[k]) for k in ("pg", "vf", "ent", "kl", "mean_reward"))
+        w1 = torch.cat([p.detach().reshape(-1) for p in ppo.policy.parameters()])
+        assert bool(torch.isfinite(w1).all()) and not torch.equal(w0, w1)
+        obs = make_obs(ppo.policy, 700)
+        m, v = fused_forward(ppo.fused, obs, 700)                         # update() packed the optimiser's weights again
+        with torch.no_grad():
+            x = obs[:700]
+            r_mean, r_value = ppo.policy.action_net(ppo.policy.actor(x)), ppo.policy.value(x)
+        assert float((m - r_mean).abs().max()) <= TOL_FP32_MAX and float((v - r_value).abs().max()) <= TOL_FP32_MAX
+        ppo.fused.close()

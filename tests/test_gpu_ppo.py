@@ -79,21 +79,39 @@ def test_fused_bias_tanh_layer_matches_autograd(dtype_name):
         assert torch.equal(a(x), b(x))
 
 
+FORK_K8 = dict(num_agents=8, neighbor_obs_type="dist_sangle_sheading", obs_repr="cdist_cdistdot_dist_distdot_sangle_angledot")
+TRAINING_TOWERS = {
+    # name: (config, hidden, neighbor_hidden, neighbour encoder)
+    "cfg2": (lambda: QuadSimConfig(num_envs=2, num_agents=8), 256, 256, "mean_embed"),
+    "k5_v3_narrow": (lambda: QuadSimConfig(num_envs=2, num_agents=5, neighbor_visible_num=3), 64, 48, "mean_embed"),
+    "cfg2_mlp": (lambda: QuadSimConfig(num_envs=2, num_agents=8), 256, 256, "mlp"),                   # 36 neighbour inputs
+    # S 6 and W * V 6: the self encoder's and the MLP's first layers take _FirstBiasTanh on a strided slice of the observation
+    "fork_mlp": (lambda: QuadSimConfig.fork_default(num_envs=2), 256, 256, "mlp"),
+    "fork_k8_sheading_mlp": (lambda: QuadSimConfig.fork_default(num_envs=2, **FORK_K8), 256, 256, "mlp"),   # S 7, 35 neighbour inputs
+    "fork": (lambda: QuadSimConfig.fork_default(num_envs=2), 256, 256, "mean_embed"),
+    "cfg3_obstacles": (lambda: QuadSimConfig(num_envs=2, num_agents=8, quads_mode="mix", use_obstacles=True, use_downwash=True,
+                                             obs_repr="xyz_vxyz_R_omega_floor", neighbor_visible_num=2), 256, 256, "mean_embed"),
+    "no_neighbours": (lambda: QuadSimConfig(num_envs=2, num_agents=1, neighbor_visible_num=0), 256, 256, "mean_embed"),
+}
+
+
 @pytest.mark.parametrize("autocast", [False, True])
 def test_fused_encoder_training_path_matches_plain_autograd(autocast):
-    """The whole tower on CUDA with gradients (TanhMLP pairs + the fused layer-2 / neighbour-mean tail, `qp_bias_tanh_mean[_backward]`) against the
-    same module with the fused path switched off: output and every parameter gradient."""
+    """The whole tower on CUDA with gradients (TanhMLP pairs, `_FirstBiasTanh` on first layers of at most 8 inputs, the fused layer-2 /
+    neighbour-mean tail `qp_bias_tanh_mean[_backward]`) against the same module with the fused path switched off: output and every
+    parameter gradient, for every neighbour encoder the kernels serve (deep-sets, MLP, none) and the obstacle encoder."""
     import torch
     from quad_swarm_rl_stable_baselines3_b200.ppo import QuadEncoder, TanhMLP
     dev = torch.device("cuda:0")
     torch.manual_seed(1)
-    for kw, hidden, nh in ((dict(num_agents=8), 256, 256), (dict(num_agents=5, neighbor_visible_num=3), 64, 48)):
-        enc = QuadEncoder(QuadSimConfig(num_envs=2, **kw), hidden=hidden, neighbor_hidden=nh, neighbor_encoder="mean_embed").to(dev)
+    for name, (make, hidden, nh, kind) in TRAINING_TOWERS.items():
+        enc = QuadEncoder(make(), hidden=hidden, neighbor_hidden=nh, neighbor_encoder=kind).to(dev)
+        assert enc.kind == ("none" if name == "no_neighbours" else kind)
         with torch.no_grad():
             for m in enc.modules():
                 if isinstance(m, torch.nn.Linear):
                     m.bias.uniform_(-0.4, 0.4)
-        D = enc.S + enc.W * enc.V
+        D = enc.S + enc.W * enc.V + enc.O
         obs = torch.randn(1500 + 7, D, device=dev)
         g = torch.randn(obs.shape[0], enc.out_size, device=dev)
         res = []
@@ -108,7 +126,10 @@ def test_fused_encoder_training_path_matches_plain_autograd(autocast):
             finally:
                 TanhMLP.fused = True
         tol = 4e-2 if autocast else 3e-5
-        assert float((res[0][0] - res[1][0]).abs().max()) <= tol
+        d_out = float((res[0][0] - res[1][0]).abs().max())
+        worst = max(float((res[0][1][n] - res[1][1][n]).abs().max()) / max(1.0, float(res[1][1][n].abs().max())) for n in res[0][1])
+        print(f"\n[{name}] autocast={autocast}: max |d out| {d_out:.1e}, max scaled |d grad| {worst:.1e}")
+        assert d_out <= tol, name
         for n in res[0][1]:
             ref = res[1][1][n]
-            assert float((res[0][1][n] - ref).abs().max()) <= tol * max(1.0, float(ref.abs().max())), (kw, n)
+            assert float((res[0][1][n] - ref).abs().max()) <= tol * max(1.0, float(ref.abs().max())), (name, n)
