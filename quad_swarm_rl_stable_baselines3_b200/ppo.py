@@ -13,9 +13,12 @@ of the torch module are plain PyTorch (cuBLAS) and are what the update different
 hand-written tcgen05 kernel (`fused_policy.py`, csrc/policy_kernels.cu: both towers and heads in one launch, activations in
 tensor memory; deep-sets or no neighbour encoder, with or without the obstacle encoder, or the 'mlp' neighbour encoder with at most
 40 inputs and no obstacle encoder; parity against this module in tests/test_gpu_policy.py, tests/test_gpu_policy_obstacles.py and
-tests/test_gpu_policy_mlp.py; the 'attention' encoder and the other 'mlp' policies stay on the torch path) and GAE on `qp_gae` (one launch).  Nothing of SB3's
-arithmetic is pinned by a reference test (SB3 is not installed in the build image) -- "parity unpinned" for the update; the
-GAE recursion is tested against a numpy restatement of SB3's `RolloutBuffer.compute_returns_and_advantage`.
+tests/test_gpu_policy_mlp.py; the 'attention' encoder and the other 'mlp' policies stay on the torch path) and GAE on `qp_gae` (one launch).
+SB3 itself is not installed; tests/test_ppo_reference.py pins `collect` + `update` against a float64 restatement of SB3 2.x's
+`collect_rollouts`, `RolloutBuffer` and `PPO.train`: the rollout buffers (a replay of the simulator reproduces them bitwise, `logp_buf`
+is the log-prob of the stored action, GAE), and for every minibatch, at the device's own parameters, the post-clip gradient (advantage
+normalisation, Gaussian log-prob / entropy, clipped surrogate, value and entropy terms, global-norm clip) and the Adam step (eps 1e-5).
+Measured gradient errors and tolerances are listed there and in DESIGN.md section 11.
 
 Multi-GPU: one process per GPU, each with its own env shard (sharding.py); the only collectives are the gradient all-reduce
 per minibatch (one flat NCCL buffer) and the episode-stat all-reduce per rollout.
@@ -211,7 +214,9 @@ class QuadActorCritic(nn.Module):
                 nn.init.zeros_(m.bias)
 
     def dist(self, obs):
-        mean = self.action_net(self.actor(obs))
+        # float32 Gaussian under bf16 autocast too (SB3's is float32): with the head's bf16 output as loc, act() would sample a bf16
+        # action and take its log-prob with a bf16 (action - mean), which is then not the log-prob of the stored action to fp32 rounding
+        mean = self.action_net(self.actor(obs)).float()
         # validate_args=False: the argument check reads a device boolean on the host (a sync per call, and illegal under graph capture)
         return torch.distributions.Normal(mean, self.log_std.exp().expand_as(mean), validate_args=False)
 
