@@ -390,7 +390,8 @@ int qs_set_reward_info(qs_env *env, float *rew_info);
  *   centres [N, QS_MAX_OBSTACLES] (use_obstacles only); scenario rows (formation scenarios only); episode records (env rows, drone
  *   rows); qs_stats; fork mode: the PID / heading planes, evader, per-env fork flags.  A section absent in the mode has size 0.
  *   Section sizes depend on N, K and the mode only, never on the launch shape, so a snapshot restores into any handle created
- *   with the same qs_config, seed and env_id_offset included: a shard restores into its own handle only.
+ *   with the same qs_config, seed and env_id_offset included: a shard restores into its own handle only (qs_restore_shards below
+ *   moves envs across shard boundaries).
  *   Not stored: the launch count, the reset-first scheduling lists (qs_restore empties them, as qs_create leaves them), the
  *   staging buffers of the *_host calls, and the qs_set_reward_info pointer (the target handle keeps its own).
  * Both calls take pinned or pageable host memory and return after `stream` has drained.  qs_snapshot writes
@@ -402,6 +403,24 @@ int qs_set_reward_info(qs_env *env, float *rew_info);
 size_t qs_snapshot_size(const qs_env *env);                                   /* 0 for NULL */
 int    qs_snapshot(qs_env *env, void *dst_host, size_t bytes, void *stream);
 int    qs_restore(qs_env *env, const void *src_host, size_t bytes, void *stream);
+
+/* Resharded resume: loads this handle's envs, global ids [env_id_offset, env_id_offset + num_envs), from `count` snapshots
+ * (blobs[i], bytes[i] bytes each) that qs_snapshot took on handles of any size -- the rank files of a run saved on another number of
+ * GPUs.  Every env is independent and its random stream is keyed by (global env id, RNG launch counter), so the steps after the call
+ * are bitwise the steps the old shards would have taken.
+ *   Checks, on every blob before the first copy: magic, version, sizeof(qs_config), the section table against the blob's own num_envs,
+ *   K and mode, and bytes[i] equal to the length it implies; every qs_config field equal to the handle's except num_envs,
+ *   env_id_offset and the qs_set_param fields (those must agree among the blobs and are taken from them, as qs_restore does); the
+ *   same RNG launch counter in every blob; env ranges that do not overlap and together cover the handle's range.  Blobs whose range
+ *   does not meet the handle's are ignored, so every new shard may pass the full list of old ones.  On a failure the handle is
+ *   untouched and the call returns QS_ERR_SHAPE (blob layout, env ranges, count < 1) or QS_ERR_BAD_CONFIG (configuration, RNG
+ *   counter) with the first problem named in qs_last_error (the field, or the first env no blob covers); QS_ERR_NULL for NULL arrays.
+ *   Copies: one cudaMemcpyAsync per section per blob, of the slice of the envs this handle holds (every section is env-major).
+ *   The handle's qs_stats become the sum, in blob order, of the stats of the blobs whose first env lies in its range: summed over
+ *   the new handles, the totals are the old ones, each counted once.  The reset-first lists are emptied as qs_restore does.
+ * Pinned or pageable host memory; returns after `stream` has drained.  restore_shards of one blob into a handle of the blob's own
+ * range is qs_restore. */
+int    qs_restore_shards(qs_env *env, const void *const *blobs, const size_t *bytes, int count, void *stream);
 
 #ifdef __cplusplus
 }

@@ -2,12 +2,14 @@
 """Size and wall time of an exact save / resume at training scale: qs_snapshot / qs_restore (pinned and pageable host buffers) and
 DevicePPO.save / load (checkpoint file written under --out).  Configurations: cfg2 and cfg3 at 65536 envs x 8 drones, the fork env at
 65536 x 4.  Every time is a host clock around a call that returns after its stream has drained; median of --reps calls.  Each restore
-is followed by a snapshot compared byte for byte with the restored blob.  The card's name and power limit go into every line.
+is followed by a snapshot compared byte for byte with the restored blob.  Last, a resharded resume: qs_restore_shards of two cfg2
+snapshots of --envs / 2 envs each into one handle of --envs (pinned).  The card's name and power limit go into every line.
 
-    python profiles/tools/snapshot_time.py --out DIR [--envs 65536] [--reps 5]
+    python profiles/tools/snapshot_time.py --out DIR [--envs 65536] [--reps 5] [--only-merge]
 """
 import argparse
 import ctypes as C
+import dataclasses
 import json
 import os
 import subprocess
@@ -19,7 +21,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
-from quad_swarm_rl_stable_baselines3_b200.config import QuadSimConfig  # noqa: E402
+from quad_swarm_rl_stable_baselines3_b200.config import QsConfigC, QuadSimConfig  # noqa: E402
 from quad_swarm_rl_stable_baselines3_b200.ppo import DevicePPO, PPOConfig  # noqa: E402
 from quad_swarm_rl_stable_baselines3_b200.sim import QuadSwarmSim  # noqa: E402
 
@@ -27,6 +29,7 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--out", required=True, help="directory for the checkpoint files and snapshot_time.json")
 ap.add_argument("--envs", type=int, default=65536)
 ap.add_argument("--reps", type=int, default=5)
+ap.add_argument("--only-merge", action="store_true", help="time the resharded resume only")
 args = ap.parse_args()
 if not torch.cuda.is_available():
     raise SystemExit("snapshot_time.py measures on a CUDA device; none is visible")
@@ -67,7 +70,7 @@ def steady_sim(cfg):
 
 
 rows = []
-for name, make in CONFIGS.items():
+for name, make in ({} if args.only_merge else CONFIGS).items():
     cfg = make(args.envs)
     sim = steady_sim(cfg)
     lib, h, st = sim._lib, sim._h, sim._stream()
@@ -113,6 +116,46 @@ for name, make in CONFIGS.items():
     torch.cuda.empty_cache()
     print(json.dumps(row), flush=True)
     rows.append(row)
+
+
+# Resharded resume: the snapshots of two cfg2 shards of --envs / 2 envs merged into one handle of --envs (qs_restore_shards), pinned.
+# Checked afterwards: every env-major section of the merged handle's snapshot is the two shards' sections back to back.
+def sections(raw):
+    """(offset, bytes) of every section of a blob, from its header's table (include/quadsim.h)."""
+    base = 16 + C.sizeof(QsConfigC)
+    count = int(np.frombuffer(raw[base + 4:base + 8].tobytes(), np.uint32)[0])
+    sizes = np.frombuffer(raw[base + 8:base + 8 + 8 * count].tobytes(), np.uint64).astype(np.int64)
+    offs = base + 8 + 8 * count + np.concatenate([[0], np.cumsum(sizes)[:-1]])
+    return list(zip(offs.tolist(), sizes.tolist()))
+
+
+cfg = CONFIGS["cfg2"](args.envs)
+half = args.envs // 2
+parts = [steady_sim(dataclasses.replace(cfg, num_envs=half, env_id_offset=r * half)) for r in range(2)]
+blobs = []
+for p in parts:
+    n = int(p._lib.qs_snapshot_size(p._h))
+    blobs.append(torch.empty(n, dtype=torch.uint8, pin_memory=True))
+    assert p._lib.qs_snapshot(p._h, C.c_void_p(blobs[-1].data_ptr()), n, p._stream()) == 0
+    p.close()
+merged = QuadSwarmSim(cfg, device=dev)
+lib, h, st = merged._lib, merged._h, merged._stream()
+ptrs = (C.c_void_p * 2)(*[b.data_ptr() for b in blobs])
+sizes = (C.c_size_t * 2)(*[b.numel() for b in blobs])
+row = {"config": "cfg2_merge", "envs": cfg.num_envs, "agents": cfg.num_agents, "card": card,
+       "source_blobs": [b.numel() for b in blobs]}
+row["qs_restore_shards_2_to_1_pinned_s"], _ = timed(lambda: lib.qs_restore_shards(h, ptrs, sizes, 2, st), args.reps)
+row["gb_per_s_restore_shards_pinned"] = sum(b.numel() for b in blobs) / row["qs_restore_shards_2_to_1_pinned_s"] / 1e9
+n = int(lib.qs_snapshot_size(h))
+out = torch.empty(n, dtype=torch.uint8, pin_memory=True)
+assert lib.qs_snapshot(h, C.c_void_p(out.data_ptr()), n, st) == 0
+m, b0, b1 = out.numpy(), blobs[0].numpy(), blobs[1].numpy()
+for (om, nm), (o0, n0), (o1, n1) in zip(sections(m), sections(b0), sections(b1)):
+    if nm == 2 * n0 and n0 == n1 and nm > 0:                                   # env-major (the stats section is not)
+        assert np.array_equal(m[om:om + n0], b0[o0:o0 + n0]) and np.array_equal(m[om + n0:om + nm], b1[o1:o1 + n1]), "merge differs"
+merged.close()
+print(json.dumps(row), flush=True)
+rows.append(row)
 
 with open(os.path.join(args.out, "snapshot_time.json"), "w") as f:
     json.dump(rows, f, indent=1)

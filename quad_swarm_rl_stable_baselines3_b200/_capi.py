@@ -23,7 +23,8 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 EXPORTS = ("qs_config_size", "qs_stats_size", "qs_api_version", "qs_last_error", "qs_create", "qs_destroy",
            "qs_num_envs", "qs_num_agents", "qs_obs_dim", "qs_act_dim", "qs_launch_count", "qs_reset", "qs_step",
            "qs_reset_host", "qs_step_host", "qs_get_state", "qs_set_state", "qs_set_param", "qs_episode_stats",
-           "qs_episode_records", "qs_episode_records_host", "qs_set_reward_info", "qs_snapshot_size", "qs_snapshot", "qs_restore")
+           "qs_episode_records", "qs_episode_records_host", "qs_set_reward_info", "qs_snapshot_size", "qs_snapshot", "qs_restore",
+           "qs_restore_shards")
 # every symbol include/quadpolicy.h declares (fused policy forward, csrc/policy_kernels.cu)
 POLICY_EXPORTS = ("qp_config_size", "qp_last_error", "qp_create", "qp_create_encoder", "qp_destroy", "qp_launch_count", "qp_set_weights", "qp_forward", "qp_gae", "qp_bias_tanh", "qp_bias_tanh_backward", "qp_bias_tanh_mean", "qp_bias_tanh_mean_backward", "qp_bias_tanh_backward_first", "qp_bias_tanh_backward_first_workspace")
 
@@ -109,6 +110,7 @@ def lib():
     L.qs_snapshot_size.restype = C.c_size_t
     L.qs_snapshot.argtypes = [vp, vp, C.c_size_t, vp]
     L.qs_restore.argtypes = [vp, vp, C.c_size_t, vp]
+    L.qs_restore_shards.argtypes = [vp, C.POINTER(vp), C.POINTER(C.c_size_t), i32, vp]
     L.qs_philox_probe.argtypes = [C.c_uint32] * 6 + [C.POINTER(C.c_uint32), fp]
     # fused policy forward (include/quadpolicy.h)
     L.qp_config_size.restype = C.c_size_t

@@ -2,12 +2,14 @@
 // Host side: owns the device state planes, converts qs_config to the kernel constant block, picks the launch shape.
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cmath>
 #include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <vector>
 
 #include "launch.h"
 
@@ -402,31 +404,55 @@ static const char *first_config_difference(const qs_config &a, const qs_config &
     return nullptr;
 }
 
+// the formation scenarios keep a per-env scenario row (DevPtrs::scen); static_same_goal, the obstacle scenarios and fork mode do not
+static bool has_scenario_rows(const qs_config &c)
+{
+    return !c.use_obstacles && c.env_mode == QS_MODE_UPSTREAM && c.scenario != QS_SCENARIO_STATIC_SAME_GOAL;
+}
+
 // Sections of a snapshot, in blob order.  Sizes follow from N, K and the mode alone (never from the slab's alignment or the launch
 // shape); a section the mode does not have is 0 bytes.
 enum { SEC_PLANES = 0, SEC_TICK = SEC_PLANES + PL_COUNT, SEC_SVD, SEC_ECNT, SEC_OBST, SEC_SCEN, SEC_EP_REC, SEC_EP_AGENT, SEC_STATS,
        SEC_FPLANES, SEC_EVADER = SEC_FPLANES + FP_COUNT, SEC_FFLAGS, SEC_COUNT };
 
-struct SnapSection { void *dev; size_t bytes; };
+// Every section but the stats is env-major: env e's part is the `row` bytes at e * row (for the per-drone sections the rows of its
+// K drones; the episode counters are [N, EC_COUNT], indexed env * EC_COUNT + k), so the part of an env range is one contiguous slice.
+// The stats are one qs_stats for the whole handle (row 0).
+struct SnapSection { void *dev; size_t bytes, row; };
 
+// the section table of a snapshot of a handle created with `c`, device pointers unset
+static void snapshot_sections(const qs_config &c, SnapSection s[SEC_COUNT])
+{
+    const size_t N = (size_t)c.num_envs, K = (size_t)c.num_agents;
+    auto env_major = [&](int i, size_t row) { s[i] = { nullptr, N * row, row }; };
+    for (int i = 0; i < SEC_COUNT; ++i) s[i] = { nullptr, 0, 0 };
+    for (int p = 0; p < PL_COUNT; ++p) env_major(SEC_PLANES + p, K * sizeof(float4));
+    env_major(SEC_TICK, sizeof(int));
+    env_major(SEC_SVD, sizeof(int));
+    env_major(SEC_ECNT, EC_COUNT * sizeof(int));
+    if (c.use_obstacles) env_major(SEC_OBST, QS_MAX_OBSTACLES * sizeof(float2));
+    if (has_scenario_rows(c)) env_major(SEC_SCEN, QS_SC_COUNT * sizeof(float));
+    env_major(SEC_EP_REC, QS_ER_COUNT * sizeof(int));
+    env_major(SEC_EP_AGENT, K * sizeof(float4));
+    s[SEC_STATS] = { nullptr, sizeof(qs_stats), 0 };
+    if (c.env_mode == QS_MODE_FORK) {
+        for (int p = 0; p < FP_COUNT; ++p) env_major(SEC_FPLANES + p, K * sizeof(float4));
+        env_major(SEC_EVADER, sizeof(float2));
+        env_major(SEC_FFLAGS, sizeof(int));
+    }
+}
+
+// the section table of the handle, with its device pointers
 static void snapshot_sections(const qs_env *e, SnapSection s[SEC_COUNT])
 {
-    const size_t N = (size_t)e->cfg.num_envs, nd = N * e->cfg.num_agents;
-    for (int i = 0; i < SEC_COUNT; ++i) s[i] = { nullptr, 0 };
-    for (int p = 0; p < PL_COUNT; ++p) s[SEC_PLANES + p] = { e->dp.plane[p], nd * sizeof(float4) };
-    s[SEC_TICK] = { e->dp.tick, N * sizeof(int) };
-    s[SEC_SVD] = { e->dp.svd_ctr, N * sizeof(int) };
-    s[SEC_ECNT] = { e->dp.ecnt, N * EC_COUNT * sizeof(int) };
-    if (e->cfg.use_obstacles) s[SEC_OBST] = { e->dp.obst_xy, N * QS_MAX_OBSTACLES * sizeof(float2) };
-    if (e->dp.scen) s[SEC_SCEN] = { e->dp.scen, N * QS_SC_COUNT * sizeof(float) };
-    s[SEC_EP_REC] = { e->dp.ep_rec, N * QS_ER_COUNT * sizeof(int) };
-    s[SEC_EP_AGENT] = { e->dp.ep_agent, nd * sizeof(float4) };
-    s[SEC_STATS] = { e->dp.stats, sizeof(qs_stats) };
-    if (e->fork) {
-        for (int p = 0; p < FP_COUNT; ++p) s[SEC_FPLANES + p] = { e->fp.plane[p], nd * sizeof(float4) };
-        s[SEC_EVADER] = { e->fp.evader, N * sizeof(float2) };
-        s[SEC_FFLAGS] = { e->fp.flags, N * sizeof(int) };
-    }
+    snapshot_sections(e->cfg, s);
+    void *dev[SEC_COUNT] = {};
+    for (int p = 0; p < PL_COUNT; ++p) dev[SEC_PLANES + p] = e->dp.plane[p];
+    dev[SEC_TICK] = e->dp.tick; dev[SEC_SVD] = e->dp.svd_ctr; dev[SEC_ECNT] = e->dp.ecnt; dev[SEC_OBST] = e->dp.obst_xy;
+    dev[SEC_SCEN] = e->dp.scen; dev[SEC_EP_REC] = e->dp.ep_rec; dev[SEC_EP_AGENT] = e->dp.ep_agent; dev[SEC_STATS] = e->dp.stats;
+    for (int p = 0; p < FP_COUNT; ++p) dev[SEC_FPLANES + p] = e->fp.plane[p];
+    dev[SEC_EVADER] = e->fp.evader; dev[SEC_FFLAGS] = e->fp.flags;
+    for (int i = 0; i < SEC_COUNT; ++i) if (s[i].bytes) s[i].dev = dev[i];
 }
 
 static std::string section_name(int i)
@@ -449,6 +475,60 @@ struct SnapHeader {
 };
 static_assert(offsetof(SnapHeader, cfg) == 16, "include/quadsim.h documents the configuration at offset 16");
 static_assert(sizeof(qs_config) % 8 == 0, "the snapshot header has no padding");
+
+// Magic, version, length and sizeof(qs_config) of a blob; copies its header to *h.  On failure `why` names the check first.
+static int read_header(const void *src_host, size_t bytes, SnapHeader *h, std::string &why)
+{
+    const char *src = (const char *)src_host;
+    uint32_t magic = 0, version = 0;
+    if (bytes >= 8) { memcpy(&magic, src, 4); memcpy(&version, src + 4, 4); }
+    if (magic != SNAP_MAGIC) { why = "magic: not a simulator snapshot"; return QS_ERR_SHAPE; }
+    if (version != QS_SNAPSHOT_VERSION) {
+        why = "version: snapshot format " + std::to_string(version) + ", this library reads " + std::to_string(QS_SNAPSHOT_VERSION);
+        return QS_ERR_SHAPE;
+    }
+    if (bytes < sizeof(SnapHeader)) { why = "bytes: " + std::to_string(bytes) + " is shorter than the header"; return QS_ERR_SHAPE; }
+    memcpy(h, src, sizeof(*h));
+    if (h->config_size != sizeof(qs_config)) {
+        why = "config_size: the snapshot's qs_config has " + std::to_string(h->config_size) + " bytes, this library's " +
+              std::to_string(sizeof(qs_config));
+        return QS_ERR_SHAPE;
+    }
+    return QS_OK;
+}
+
+// The header's section table against the expected one; *total = the blob length it implies.
+static int check_sections(const SnapHeader &h, const SnapSection sec[SEC_COUNT], size_t *total, std::string &why)
+{
+    if (h.sections != SEC_COUNT) { why = "sections: " + std::to_string(h.sections) + ", expected " + std::to_string((int)SEC_COUNT); return QS_ERR_SHAPE; }
+    size_t need = sizeof(SnapHeader);
+    for (int i = 0; i < SEC_COUNT; ++i) {
+        if (h.section_bytes[i] != sec[i].bytes) {
+            why = "section " + section_name(i) + ": " + std::to_string(h.section_bytes[i]) + " bytes, expected " + std::to_string(sec[i].bytes);
+            return QS_ERR_SHAPE;
+        }
+        need += sec[i].bytes;
+    }
+    *total = need;
+    return QS_OK;
+}
+
+#define QS_STATS_FIELDS(X)                                                                                                       \
+    X(episodes) X(num_collisions) X(num_collisions_after_settle) X(num_collisions_final_5s) X(num_collisions_with_room)          \
+    X(num_collisions_with_floor) X(num_collisions_with_wall) X(num_collisions_with_ceiling) X(num_collisions_obst_quad)         \
+    X(num_collisions_obst_quad_after_settle) X(agents_success) X(agents_deadlock) X(agents_collided) X(nonfinite_resets)         \
+    X(episodes_success) X(distance_to_goal_1s) X(distance_to_goal_3s) X(distance_to_goal_5s) X(reward_sum)
+
+#define QS_FIELD_BYTES(f) + sizeof(((const qs_stats *)nullptr)->f)
+static_assert(0 QS_STATS_FIELDS(QS_FIELD_BYTES) == sizeof(qs_stats), "QS_STATS_FIELDS must list every qs_stats field");
+#undef QS_FIELD_BYTES
+
+static void add_stats(qs_stats &a, const qs_stats &b)
+{
+#define QS_ADD_FIELD(f) a.f += b.f;
+    QS_STATS_FIELDS(QS_ADD_FIELD)
+#undef QS_ADD_FIELD
+}
 
 extern "C" {
 
@@ -477,7 +557,7 @@ int qs_create(const qs_config *cfg, int device, qs_env **out)
     fill_const(*cfg, e->dc);
     e->fork = cfg->env_mode == QS_MODE_FORK;
     e->A = e->fork ? 2 : 4;
-    const bool scen_feat = !cfg->use_obstacles && cfg->env_mode == QS_MODE_UPSTREAM && cfg->scenario != QS_SCENARIO_STATIC_SAME_GOAL;
+    const bool scen_feat = has_scenario_rows(*cfg);
     e->feat = (cfg->use_obstacles ? 1 : 0) | ((cfg->use_downwash && cfg->num_agents > 1) ? 2 : 0) | (scen_feat ? 4 : 0);
     fill_fork(*cfg, e->fc);
     memset(&e->fp, 0, sizeof(e->fp));
@@ -902,32 +982,17 @@ int qs_restore(qs_env *e, const void *src_host, size_t bytes, void *stream)
     if (!e || !src_host) return fail(e, QS_ERR_NULL, "qs_restore: null argument");
     // everything is checked before the first copy: a rejected snapshot leaves the handle as it was
     const char *src = (const char *)src_host;
-    uint32_t magic = 0, version = 0;
-    if (bytes >= 8) { memcpy(&magic, src, 4); memcpy(&version, src + 4, 4); }
-    if (magic != SNAP_MAGIC) return fail(e, QS_ERR_SHAPE, "qs_restore: magic: not a simulator snapshot");
-    if (version != QS_SNAPSHOT_VERSION)
-        return fail(e, QS_ERR_SHAPE, "qs_restore: version: snapshot format " + std::to_string(version) + ", this library reads " +
-                                     std::to_string(QS_SNAPSHOT_VERSION));
-    if (bytes < sizeof(SnapHeader)) return fail(e, QS_ERR_SHAPE, "qs_restore: bytes: " + std::to_string(bytes) + " is shorter than the header");
     SnapHeader h;
-    memcpy(&h, src, sizeof(h));
-    if (h.config_size != sizeof(qs_config))
-        return fail(e, QS_ERR_SHAPE, "qs_restore: config_size: the snapshot's qs_config has " + std::to_string(h.config_size) + " bytes, this library's " +
-                                     std::to_string(sizeof(qs_config)));
+    std::string why;
+    if (int rc = read_header(src, bytes, &h, why)) return fail(e, rc, "qs_restore: " + why);
     qs_config want = e->cfg;                                            // the qs_set_param values come from the snapshot
     for (int k = 0; k < QS_PARAM_COUNT; ++k) *param_field(want, k) = *param_field(h.cfg, k);
     if (const char *f = first_config_difference(want, h.cfg))
         return fail(e, QS_ERR_BAD_CONFIG, std::string("qs_restore: ") + f + ": the snapshot's configuration differs from the handle's");
     SnapSection sec[SEC_COUNT];
     snapshot_sections(e, sec);
-    if (h.sections != SEC_COUNT) return fail(e, QS_ERR_SHAPE, "qs_restore: sections: " + std::to_string(h.sections) + ", expected " + std::to_string((int)SEC_COUNT));
-    size_t need = sizeof(SnapHeader);
-    for (int i = 0; i < SEC_COUNT; ++i) {
-        if (h.section_bytes[i] != sec[i].bytes)
-            return fail(e, QS_ERR_SHAPE, "qs_restore: section " + section_name(i) + ": " + std::to_string(h.section_bytes[i]) + " bytes, expected " +
-                                         std::to_string(sec[i].bytes));
-        need += sec[i].bytes;
-    }
+    size_t need = 0;
+    if (int rc = check_sections(h, sec, &need, why)) return fail(e, rc, "qs_restore: " + why);
     if (bytes != need)
         return fail(e, QS_ERR_SHAPE, "qs_restore: bytes: the blob has " + std::to_string(bytes) + ", a snapshot of this handle " + std::to_string(need));
     DeviceGuard guard(e->device);
@@ -944,6 +1009,108 @@ int qs_restore(qs_env *e, const void *src_host, size_t bytes, void *stream)
     QS_CUDA(e, cudaStreamSynchronize(s));
     e->cfg = want;
     e->rng_step = h.rng_step;
+    e->hot_phase = 0;
+    fill_const(e->cfg, e->dc);
+    fill_fork(e->cfg, e->fc);
+    return QS_OK;
+}
+
+int qs_restore_shards(qs_env *e, const void *const *blobs, const size_t *bytes, int count, void *stream)
+{
+    if (!e) return QS_ERR_NULL;
+    if (count < 1) return fail(e, QS_ERR_SHAPE, "qs_restore_shards: count: " + std::to_string(count) + ", at least one snapshot is needed");
+    if (!blobs || !bytes) return fail(e, QS_ERR_NULL, "qs_restore_shards: null argument");
+    // every blob is checked before the first copy: a rejected call leaves the handle as it was
+    const int64_t lo = e->cfg.env_id_offset, hi = lo + e->cfg.num_envs;
+    std::vector<SnapHeader> hs((size_t)count);
+    for (int i = 0; i < count; ++i) {
+        const std::string at = "qs_restore_shards: blob " + std::to_string(i) + ": ";
+        if (!blobs[i]) return fail(e, QS_ERR_NULL, at + "null pointer");
+        SnapHeader &h = hs[i];
+        std::string why;
+        if (int rc = read_header(blobs[i], bytes[i], &h, why)) return fail(e, rc, at + why);
+        if (h.cfg.num_envs < 1) return fail(e, QS_ERR_SHAPE, at + "num_envs: " + std::to_string(h.cfg.num_envs));
+        // the env range may differ from the handle's; the qs_set_param values come from the snapshots and must agree among them
+        qs_config want = e->cfg;
+        want.num_envs = h.cfg.num_envs; want.env_id_offset = h.cfg.env_id_offset;
+        for (int k = 0; k < QS_PARAM_COUNT; ++k) *param_field(want, k) = *param_field(h.cfg, k);
+        if (const char *f = first_config_difference(want, h.cfg))
+            return fail(e, QS_ERR_BAD_CONFIG, at + f + ": the snapshot's configuration differs from the handle's");
+        if (i > 0) {
+            qs_config first = hs[0].cfg;
+            first.num_envs = h.cfg.num_envs; first.env_id_offset = h.cfg.env_id_offset;
+            if (const char *f = first_config_difference(first, h.cfg))
+                return fail(e, QS_ERR_BAD_CONFIG, at + f + ": differs from blob 0's (qs_set_param values must agree among the shards)");
+            if (h.rng_step != hs[0].rng_step)
+                return fail(e, QS_ERR_BAD_CONFIG, at + "rng_step: " + std::to_string(h.rng_step) + ", blob 0's " + std::to_string(hs[0].rng_step) +
+                                                  " (the shards of one run stand at the same step)");
+        }
+        SnapSection sec[SEC_COUNT];
+        snapshot_sections(h.cfg, sec);
+        size_t need = 0;
+        if (int rc = check_sections(h, sec, &need, why)) return fail(e, rc, at + why);
+        if (bytes[i] != need)
+            return fail(e, QS_ERR_SHAPE, at + "bytes: the blob has " + std::to_string(bytes[i]) + ", its header describes " + std::to_string(need));
+    }
+    // env ranges: disjoint, and together covering [lo, hi); blobs outside it are ignored
+    auto range = [&](int i) { return std::make_pair((int64_t)hs[i].cfg.env_id_offset, (int64_t)hs[i].cfg.env_id_offset + hs[i].cfg.num_envs); };
+    auto span = [](std::pair<int64_t, int64_t> r) { return "[" + std::to_string(r.first) + ", " + std::to_string(r.second) + ")"; };
+    std::vector<int> order((size_t)count);
+    for (int i = 0; i < count; ++i) order[i] = i;
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return range(a).first < range(b).first; });
+    for (int j = 1; j < count; ++j) {
+        const int a = order[j - 1], b = order[j];
+        if (range(b).first < range(a).second)
+            return fail(e, QS_ERR_SHAPE, "qs_restore_shards: env range: blob " + std::to_string(b) + " " + span(range(b)) + " overlaps blob " +
+                                         std::to_string(a) + " " + span(range(a)));
+    }
+    int64_t covered = lo;                                               // [lo, covered) is in some blob
+    for (int j = 0; j < count && covered < hi; ++j) {
+        const auto r = range(order[j]);
+        if (r.second <= covered) continue;
+        if (r.first > covered) break;
+        covered = r.second;
+    }
+    if (covered < hi)
+        return fail(e, QS_ERR_SHAPE, "qs_restore_shards: env range: gap: env " + std::to_string(covered) + " of the handle's " +
+                                     span({ lo, hi }) + " is in no snapshot");
+
+    DeviceGuard guard(e->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    SnapSection dst[SEC_COUNT];
+    snapshot_sections(e, dst);
+    // qs_stats: the sum of the blobs whose first env is in this handle's range, so that over all handles every blob counts once
+    qs_stats stats;
+    memset(&stats, 0, sizeof(stats));
+    bool have_stats = false;
+    for (int i = 0; i < count; ++i) {
+        const auto r = range(i);
+        const int64_t a = std::max(lo, r.first), b = std::min(hi, r.second);     // envs of blob i that this handle holds
+        SnapSection sec[SEC_COUNT];
+        snapshot_sections(hs[i].cfg, sec);
+        const char *p = (const char *)blobs[i] + sizeof(SnapHeader);
+        for (int k = 0; k < SEC_COUNT; ++k) {
+            if (!sec[k].bytes) continue;
+            if (sec[k].row == 0) {                                      // SEC_STATS
+                if (r.first >= lo && r.first < hi) {
+                    qs_stats x;
+                    memcpy(&x, p, sizeof(x));
+                    if (have_stats) add_stats(stats, x); else stats = x;
+                    have_stats = true;
+                }
+            } else if (a < b) {
+                const size_t row = sec[k].row;
+                QS_CUDA(e, cudaMemcpyAsync((char *)dst[k].dev + (size_t)(a - lo) * row, p + (size_t)(a - r.first) * row, (size_t)(b - a) * row,
+                                           cudaMemcpyHostToDevice, s));
+            }
+            p += sec[k].bytes;
+        }
+    }
+    QS_CUDA(e, cudaMemcpyAsync(e->dp.stats, &stats, sizeof(stats), cudaMemcpyHostToDevice, s));
+    QS_CUDA(e, cudaMemsetAsync(e->hot_cnt[0], 0, e->hot_bytes, s));    // reset-first lists as qs_restore leaves them
+    QS_CUDA(e, cudaStreamSynchronize(s));
+    for (int k = 0; k < QS_PARAM_COUNT; ++k) *param_field(e->cfg, k) = *param_field(hs[0].cfg, k);
+    e->rng_step = hs[0].rng_step;
     e->hot_phase = 0;
     fill_const(e->cfg, e->dc);
     fill_fork(e->cfg, e->fc);

@@ -466,3 +466,94 @@ class DevicePPO:
         if self.fused is not None:
             self.fused.sync()
         self._sync()
+
+    def load_shards(self, paths) -> None:
+        """Resume on another number of GPUs: load this rank's envs from the rank files `save` wrote in a run of any world size, into a
+        freshly built DevicePPO whose simulator config is the saved one but for `num_envs` / `env_id_offset` (e.g. `shard_config` of
+        the same total for the new world size).  Every rank may pass the full list of old files: the files are memory-mapped and only
+        the headers, the replicated policy / Adam state and this rank's slices are read.  Nothing this object keeps refers to the
+        mapped files afterwards, so a later `save` may overwrite them.
+        Checks that every file has the same checkpoint version and step count, bitwise-identical policy and optimizer tensors (the
+        gradient all-reduce keeps them so; ValueError naming the first tensor that differs otherwise) and the same simulator config
+        up to `num_envs` / `env_id_offset`; the simulator then rejects gaps, overlaps and shards of different steps
+        (`QuadSwarmSim.restore_shards`).
+        The simulator continues bitwise where the old shards stood; the policy and Adam state are the saved ones, with the learning
+        rate set back to the live PPOConfig as in `load`.  The torch RNG states stay those this instance was built with: the exploration
+        noise and minibatch order after a resharded resume are not those of any continued run.  A resume on the same number of GPUs
+        should use `load`, which is bitwise."""
+        paths = list(paths)
+        if not paths:
+            raise ValueError("DevicePPO.load_shards: no checkpoint files")
+        cks = [torch.load(p, map_location="cpu", weights_only=True, mmap=True) for p in paths]
+        for p, ck in zip(paths, cks):
+            if ck.get("version") != self.CHECKPOINT_VERSION:
+                raise ValueError(f"DevicePPO.load_shards: {p}: checkpoint format {ck.get('version')!r}, this code reads {self.CHECKPOINT_VERSION}")
+            if ck["total_agent_steps"] != cks[0]["total_agent_steps"]:
+                raise ValueError(f"DevicePPO.load_shards: {p}: total_agent_steps {ck['total_agent_steps']}, {paths[0]}: "
+                                 f"{cks[0]['total_agent_steps']} (files of different iterations)")
+            want = asdict(self.cfg)
+            for k, v in ck["sim_config"].items():
+                if k not in ("num_envs", "env_id_offset") and want.get(k) != v:
+                    raise ValueError(f"DevicePPO.load_shards: {p}: sim_config.{k} is {v!r}, this run's {want.get(k)!r}")
+            rows = ck["sim_config"]["num_envs"] * self.cfg.num_agents
+            if tuple(ck["obs"].shape) != (rows, self.obs.shape[1]):
+                raise ValueError(f"DevicePPO.load_shards: {p}: observations {tuple(ck['obs'].shape)}, its "
+                                 f"{ck['sim_config']['num_envs']} envs need {(rows, self.obs.shape[1])}")
+            for what in ("policy", "optimizer"):
+                name = _first_difference(cks[0][what], ck[what], what)
+                if name is not None:
+                    raise ValueError(f"DevicePPO.load_shards: {p}: {name} differs from {paths[0]}'s (the policy and Adam state of "
+                                     f"the ranks of one run are identical)")
+        self.sim.restore_shards([ck["sim"] for ck in cks])
+        # this rank's rows of the saved observations (DevicePPO.obs; the simulator's own copy came with restore_shards)
+        lo, hi, K = self.cfg.env_id_offset, self.cfg.env_id_offset + self.cfg.num_envs, self.cfg.num_agents
+        for ck in cks:
+            b0 = ck["sim_config"]["env_id_offset"]
+            a, b = max(lo, b0), min(hi, b0 + ck["sim_config"]["num_envs"])
+            if a < b:
+                self.obs[(a - lo) * K:(b - lo) * K].copy_(ck["obs"][(a - b0) * K:(b - b0) * K])
+        self.policy.load_state_dict(cks[0]["policy"], strict=True)            # copies into the parameters
+        # Adam keeps the CPU `step` tensors it is given: hand it copies, or they would stay views of the memory-mapped file, which
+        # a later save to that path truncates under them
+        self.opt.load_state_dict(_owned(cks[0]["optimizer"]))
+        for g in self.opt.param_groups:
+            g["lr"] = self.p.learning_rate
+        self.total_agent_steps = int(cks[0]["total_agent_steps"])
+        self._rollout_pending = False
+        if self.fused is not None:
+            self.fused.sync()
+        self._sync()
+
+
+def _owned(x):
+    """A copy of a state dict whose tensors own their memory (none is a view of a memory-mapped checkpoint)."""
+    if isinstance(x, dict):
+        return {k: _owned(v) for k, v in x.items()}
+    if isinstance(x, (list, tuple)):
+        return type(x)(_owned(v) for v in x)
+    return x.clone() if torch.is_tensor(x) else x
+
+
+def _first_difference(a, b, name: str):
+    """The dotted name of the first tensor or value in which two state dicts differ (tensors bitwise), or None."""
+    if isinstance(a, dict) and isinstance(b, dict):
+        if list(a) != list(b):
+            return f"{name} (keys)"
+        for k in a:
+            d = _first_difference(a[k], b[k], f"{name}.{k}")
+            if d is not None:
+                return d
+        return None
+    if isinstance(a, (list, tuple)) and isinstance(b, (list, tuple)):
+        if len(a) != len(b):
+            return f"{name} (length)"
+        for i, (x, y) in enumerate(zip(a, b)):
+            d = _first_difference(x, y, f"{name}.{i}")
+            if d is not None:
+                return d
+        return None
+    if torch.is_tensor(a) and torch.is_tensor(b):
+        same = (a.dtype == b.dtype and a.shape == b.shape
+                and torch.equal(a.contiguous().reshape(-1).view(torch.uint8), b.contiguous().reshape(-1).view(torch.uint8)))
+        return None if same else name
+    return None if (type(a) is type(b) and a == b) else name

@@ -24,6 +24,15 @@ _FORK_SHAPES = {"pid": (24, torch.float32), "heading": (3, torch.float32)}     #
 _ENV_FIELDS = {"tick": torch.int32, "svd_ctr": torch.int32, "step_ctr": torch.int32}
 
 
+# the qs_config fields the rows and width of a handle's observation follow from (fill_const, csrc/quadsim.cu)
+_OBS_LAYOUT_FIELDS = ("num_agents", "env_mode", "obs_repr", "neighbor_obs_type", "neighbor_visible_num", "use_obstacles")
+
+
+def _blob_config(blob: torch.Tensor) -> QsConfigC:
+    """The qs_config of a snapshot blob: it sits at offset 16 (include/quadsim.h)."""
+    return QsConfigC.from_buffer_copy(blob[16:16 + C.sizeof(QsConfigC)].numpy().tobytes())
+
+
 class QuadSwarmSim:
     def __init__(self, cfg: QuadSimConfig, device: Optional[torch.device | int | str] = None):
         if not torch.cuda.is_available():
@@ -275,11 +284,52 @@ class QuadSwarmSim:
             rc = self._lib.qs_restore(self._h, C.c_void_p(blob.data_ptr()), blob.numel(), self._stream())
         _capi.check(self._h, rc, "qs_restore")
         self.obs.copy_(obs.reshape(self.obs.shape))
-        # the qs_config of the snapshot sits at offset 16 of the blob (include/quadsim.h)
-        c = QsConfigC.from_buffer_copy(blob[16:16 + C.sizeof(QsConfigC)].numpy().tobytes())
+        self._take_rew_coeffs(_blob_config(blob))
+        return self.obs
+
+    def restore_shards(self, snaps) -> torch.Tensor:
+        """Load this handle's envs from the `snapshot()`s of the shards of a run saved on any number of GPUs (`qs_restore_shards`,
+        include/quadsim.h): every blob whose env range meets this handle's contributes its slice, the others are ignored, so every
+        new rank may pass the full list.  The ranges must not overlap and must cover this handle's; everything else must match as for
+        `restore`.  On a rejection nothing changes.  Returns the restored observation (self.obs)."""
+        snaps = list(snaps)
+        blobs = [torch.as_tensor(s["blob"]).detach().to("cpu", torch.uint8).contiguous().reshape(-1) for s in snaps]
+        obs = [torch.as_tensor(s["obs"]) for s in snaps]
+        lo, K = self.cfg.env_id_offset, self.K
+        ranges = []
+        # Each snapshot's observation must fit its blob's env range, checked before the call so that a misfit changes nothing.  The
+        # check needs the blob's observation width, which is this handle's when the qs_config fields it follows from are; a blob that
+        # differs there, or has no readable header, is left to qs_restore_shards, which rejects it and names the field.  Every blob
+        # the call accepts has therefore been checked.
+        for i, (b, o) in enumerate(zip(blobs, obs)):
+            if b.numel() < 16 + C.sizeof(QsConfigC) or bytes(b[:4].numpy()) != b"QSSN":
+                ranges.append(None)
+                continue
+            c = _blob_config(b)
+            ranges.append((c.env_id_offset, c.env_id_offset + c.num_envs))
+            if any(getattr(c, f) != getattr(self._c, f) for f in _OBS_LAYOUT_FIELDS):
+                continue
+            if o.numel() != c.num_envs * K * self.D:
+                raise ValueError(f"restore_shards: snapshot {i} has {o.numel()} observation values, its {c.num_envs} envs "
+                                 f"x {K} x {self.D} need {c.num_envs * K * self.D}")
+        n = len(blobs)
+        ptrs = (C.c_void_p * n)(*[b.data_ptr() for b in blobs])
+        sizes = (C.c_size_t * n)(*[b.numel() for b in blobs])
+        with torch.cuda.device(self.device):
+            rc = self._lib.qs_restore_shards(self._h, ptrs, sizes, n, self._stream())
+        _capi.check(self._h, rc, "qs_restore_shards")
+        hi = lo + self.N
+        for (b0, b1), o in zip(ranges, obs):
+            a, b = max(lo, b0), min(hi, b1)
+            if a < b:
+                self.obs[(a - lo) * K:(b - lo) * K].copy_(o.reshape(-1, self.D)[(a - b0) * K:(b - b0) * K])
+        self._take_rew_coeffs(_blob_config(blobs[0]))
+        return self.obs
+
+    def _take_rew_coeffs(self, c: QsConfigC):
+        """The reward coefficients a restored snapshot brought in, as far as they differ from this handle's configuration."""
         self.rew_coeff_overrides = {k: getattr(c, "rew_" + k) for k in PARAM_KEYS if k != "capture_radius"
                                     and getattr(c, "rew_" + k) != getattr(self._c, "rew_" + k)}
-        return self.obs
 
     # parameters / stats ------------------------------------------------------------------------------
     def set_rew_coeff(self, **coeffs):
